@@ -2,7 +2,7 @@
 """bench.py - headline benchmark of the B200 path tracer (BASELINE.json metric:
 Mpaths*bounces/s = path SEGMENTS per second, one segment = one closest-hit query + its shading).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c1..c5] [--scaling weak|strong]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c1..c5] [--scaling weak|strong] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], "c2"): bundled Scene1 (67 spheres), 1920x1080, 1024 spp, depth 8,
 default camera. One step = one rt_render_spp(1024) over the whole frame (2.12 G paths).
@@ -26,6 +26,11 @@ checks that the fused surface equals the resolve of the sum of all ranks' buffer
            frame, and with glibc's locked rand() instead of MSVC's per-thread one); the c3 leg carries the same for ITS scene.
 `--impl reference`: the reference's own CPU code (oracle/_ref, else the validated C port) on the host cores, same
            metric, bounded sample per step.
+`--dump-outputs DIR`: after the timed steps, what the last timed step handed its caller, as DIR/<name>.npy in float32, so that
+           two builds can be compared output for output (the inputs are seeded: the same arguments give the same inputs):
+           `accum` (height x width x 4, rt_read_accum: the step's sample sums), or at N > 1 with the fused exchange and for c5
+           `surface_argb` (height x width x 4, the resolved ARGB8 frame, one channel per byte). Past 60 MiB in all, a fixed seeded
+           sample of pixels is kept, with their flat indices in `pixel_index` (float64).
 """
 import argparse
 import json
@@ -55,6 +60,30 @@ def workload_config(scene="Scene1", n_obj=67, w=W, h=H, depth=DEPTH):
     """The part of `config` both arms share word for word (the driver compares them)."""
     return {"workload": "%s (%d objects) %dx%d, depth %d, path mode" % (scene, n_obj, w, h, depth), "scene": scene, "width": w, "height": h,
             "depth": depth, "mode": "path", "l2": L2_NOTE}
+
+
+DUMP_BYTES = 60 << 20                 # stays under 64 MB with the .npy headers
+
+
+def argb_channels(argb):
+    """packed ARGB8 surface (h x w uint32) -> h x w x 4 float32 (A, R, G, B)."""
+    return np.stack([(argb >> s) & 255 for s in (24, 16, 8, 0)], -1).astype(np.float32)
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every h x w x c array as out_dir/<name>.npy (float32). Over DUMP_BYTES in all, the same seeded sample of
+    pixels is taken from each array and their flat indices are written as pixel_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    h, w = next(iter(arrays.values())).shape[:2]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        keep = DUMP_BYTES // (total // (h * w) + 8)          # + 8: the pixel's index
+        idx = np.sort(np.random.default_rng(0).choice(h * w, keep, replace=False))
+        arrays = {k: v.reshape(h * w, -1)[idx] for k, v in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def flops_per_segment(objs):
@@ -351,10 +380,11 @@ def run_leg(args, config, torch, stream, steps=3, warmup=3):
     return out
 
 
-def interactive_line(tr, wl, frames):
+def interactive_line(tr, wl, frames, outputs=None):
     """BASELINE.json configs[4]: progressive 1 spp frames at 1280x720, each frame = rt_render_frame(1) into a HOST surface
     (3.7 MB per frame over PCIe), what a viewer's frame loop does (Raytracer.cpp:572-595). Frame latency p50/p99 (host clock around
-    the call, which synchronises), the same frame as rt_render_spp + rt_resolve_rgba8, and the device time of the render kernel alone."""
+    the call, which synchronises), the same frame as rt_render_spp + rt_resolve_rgba8, and the device time of the render kernel alone.
+    `outputs` (a dict) receives the last timed frame as "surface_argb"."""
     import rtb200
     w, h = wl["w"], wl["h"]
     out, _owner = rtb200.host_surface(w, h)              # page-locked surface (rt_host_alloc): one DMA per frame
@@ -376,6 +406,8 @@ def interactive_line(tr, wl, frames):
         tr.render_frame(1, True, out)                    # rt_render_frame: synchronises, the frame is on the host
         lat.append((time.perf_counter() - t0) * 1e3)
     total = time.perf_counter() - t_all
+    if outputs is not None:
+        outputs["surface_argb"] = argb_channels(out)
     for _ in range(50):                                  # device time of the render kernel (rt_get_stats synchronises: outside the latency loop)
         tr.render_spp(1)
         dev.append(tr.stats().last_render_ms)
@@ -422,12 +454,15 @@ def run_b200(args):
     tr = make_tracer(args, local, stream.cuda_stream, wl, seed_hi=0 if strong else rank)
     if strong:
         tr.set_shard(rank, world)
+    outputs = {}
     if args.config == "c5":
         with torch.cuda.stream(stream):
-            line = interactive_line(tr, wl, frames=max(args.steps, 1) * 200)
+            line = interactive_line(tr, wl, frames=max(args.steps, 1) * 200, outputs=outputs)
         line.update({"n_gpus": 1, "dtype": "f32", "config": {"workload": line.pop("workload")}})
         print(json.dumps(line), flush=True)
         tr.close()
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
         return
 
     class DevBuf:                                   # wrap the library's accumulation buffer for torch / NCCL
@@ -490,6 +525,11 @@ def run_b200(args):
         barrier()
         step_ms = timed(args.steps)
         clocks = sampler.summary()
+        if args.dump_outputs and rank == 0:                  # before anything else renders into the buffers
+            if fused:
+                outputs["surface_argb"] = argb_channels(tr.read_surface())
+            else:
+                outputs["accum"] = tr.read_accum()[0]
         s1 = tr.stats()
         segs_rank = s1.total_segments - s0.total_segments
         traced_rank = s1.total_traced_segments - s0.total_traced_segments
@@ -690,6 +730,8 @@ def run_b200(args):
             if "glibc_rand_variant" in info:
                 line["cpu_baseline"]["glibc_rand_variant"] = info["glibc_rand_variant"]
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -721,7 +763,12 @@ def main():
     ap.add_argument("--wf-node-min", type=int, default=-1, help="RT_OPT_WF_NODE_MIN override")
     ap.add_argument("--wave-mpaths", type=int, default=-1, help="RT_OPT_WF_WAVE_MPATHS override")
     ap.add_argument("--scene", default="Scene1", help="bundled scene fixture (the headline config is Scene1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:
