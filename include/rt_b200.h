@@ -268,7 +268,9 @@ int rt_env_color(rt_ctx* ctx, const float* dirs, int n, float* rgb);
 int rt_philox_block(rt_ctx* ctx, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 /* Device self-tests of exact-equivalence shortcuts; *failures = number of mismatching inputs.
  * which = 0: unit_from_word, (float)((double)k * (1.0/32767.0)) == (float)k / 32767.0f for all 32768 k.
- * which = 1: normalize (Common.hpp:159-162) with one shared reciprocal == three IEEE divisions, 2^28 vectors. */
+ * which = 1: normalize (Common.hpp:159-162) with one shared reciprocal == three IEEE divisions, 2^28 vectors.
+ * which = 2: packed FP32 pairs (add / sub / mul / fma.rn.f32x2) == the scalar .rn ops on each half, 2^26 operand sets of
+ *            random and edge values (subnormals, +-0, +-inf, near overflow, mixed exponents); two NaN results count as equal. */
 int rt_selftest(rt_ctx* ctx, int which, int* failures);
 int rt_get_stats(rt_ctx* ctx, rt_stats* out);
 /* BVH traversal work actually executed by the render kernels since rt_reset_accumulation, counted on the device while

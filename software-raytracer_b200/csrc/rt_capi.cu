@@ -1116,10 +1116,11 @@ int rt_philox_block(rt_ctx* c, const uint32_t ctr[4], const uint32_t key[2], uin
 }
 
 int rt_selftest(rt_ctx* c, int which, int* failures) {
-    if (!c || !failures || which < 0 || which > 1) return RT_ERR_INVALID;
+    if (!c || !failures || which < 0 || which > 2) return RT_ERR_INVALID;
     RT_CUDA(c, cudaSetDevice(c->device));
     if (which == 0) RT_CUDA(c, launch_selftest_uniform((int*)c->d_scratch, c->stream));
-    else RT_CUDA(c, launch_selftest_normalize((int*)c->d_scratch, c->stream));
+    else if (which == 1) RT_CUDA(c, launch_selftest_normalize((int*)c->d_scratch, c->stream));
+    else RT_CUDA(c, launch_selftest_packed((int*)c->d_scratch, c->stream));
     RT_CUDA(c, cudaMemcpyAsync(failures, c->d_scratch, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     return RT_OK;

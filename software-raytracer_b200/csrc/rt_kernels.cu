@@ -152,6 +152,46 @@ __global__ void k_selftest_normalize(int* failures, uint32_t seed) {
     if (bad) atomicAdd(failures, bad);
 }
 
+// The packed pair ops (add2 / sub2 / mul2 / fma2: add / sub / mul / fma.rn.f32x2) against the scalar .rn ops, half by half, on 2^26
+// operand sets per call. Each operand draws its own kind - any bit pattern (NaN and infinities included), subnormals, +-0 / +-inf /
+// +-FLT_MAX / +-smallest normal, exponents near overflow and near underflow, ordinary magnitudes, the sampler's values, edge mantissas -
+// so mixed exponents come from mixing kinds; one set in eight makes c cancel a * b exactly. Bits must be equal; two NaNs count as equal.
+__device__ __forceinline__ float selftest_operand(uint32_t u, uint32_t kind) {
+    const uint32_t sign = u & 0x80000000u;
+    switch (kind & 7u) {
+    case 0u: return __uint_as_float(u);
+    case 1u: return __uint_as_float(u & 0x807fffffu);                                              // subnormal or zero
+    case 2u: {
+        const uint32_t special[8] = {0u, 0x7f800000u, 0x7f7fffffu, 0x00800000u, 0x00000001u, 0x3f800000u, 0x7f000000u, 0x00ffffffu};
+        return __uint_as_float(sign | special[(u >> 8) & 7u]);
+    }
+    case 3u: return __uint_as_float(sign | ((250u + (u >> 23) % 5u) << 23) | (u & 0x007fffffu));      // near overflow
+    case 4u: return __uint_as_float(sign | ((1u + (u >> 23) % 24u) << 23) | (u & 0x007fffffu));       // just above the subnormals
+    case 5u: return __uint_as_float(sign | ((97u + (u >> 23) % 61u) << 23) | (u & 0x007fffffu));      // 2^-30 .. 2^30
+    case 6u: return (unit_from_word(u) - 0.5f) * 2.f;                                                 // the sampler's own values
+    default: return __uint_as_float(sign | ((u >> 8) & 0x7f800000u) | ((u & 1u) ? 0x007fffffu : (1u << (u % 23u))));
+    }
+}
+__device__ __forceinline__ bool same_bits(float a, float b) { return __float_as_uint(a) == __float_as_uint(b) || (a != a && b != b); }
+__global__ void k_selftest_packed(int* failures, uint32_t seed) {
+    const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x;
+    int bad = 0;
+    for (uint32_t it = 0; it < 64u; ++it) {
+        const uint4 w0 = philox4x32_10(tid, it, 0u, 0u, seed, 0x9ac4ed2fu), w1 = philox4x32_10(tid, it, 1u, 0u, seed, 0x9ac4ed2fu);
+        const uint32_t k = w1.w;
+        const fpair a = fp(selftest_operand(w0.x, k), selftest_operand(w0.y, k >> 3));
+        const fpair b = fp(selftest_operand(w0.z, k >> 6), selftest_operand(w0.w, k >> 9));
+        fpair c = fp(selftest_operand(w1.x, k >> 12), selftest_operand(w1.y, k >> 15));
+        if (((k >> 18) & 7u) == 0u) c = fp(-__fmul_rn(a.x, b.x), -__fmul_rn(a.y, b.y));           // exact cancellation in the fma
+        const fpair s = add2(a, b), d = sub2(a, b), m = mul2(a, b), f = fma2(a, b, c);
+        bad += !same_bits(s.x, __fadd_rn(a.x, b.x)) + !same_bits(s.y, __fadd_rn(a.y, b.y));
+        bad += !same_bits(d.x, __fsub_rn(a.x, b.x)) + !same_bits(d.y, __fsub_rn(a.y, b.y));
+        bad += !same_bits(m.x, __fmul_rn(a.x, b.x)) + !same_bits(m.y, __fmul_rn(a.y, b.y));
+        bad += !same_bits(f.x, __fmaf_rn(a.x, b.x, c.x)) + !same_bits(f.y, __fmaf_rn(a.y, b.y, c.y));
+    }
+    if (bad) atomicAdd(failures, bad);
+}
+
 __global__ void k_philox(uint4 ctr, uint2 key, uint4* out) { *out = philox4x32_10(ctr.x, ctr.y, ctr.z, ctr.w, key.x, key.y); }
 
 // ---- the render kernel -----------------------------------------------------------------------
@@ -972,6 +1012,13 @@ cudaError_t launch_selftest_normalize(int* dev_failures, cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(dev_failures, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     k_selftest_normalize<<<16384, 256, 0, st>>>(dev_failures, 0x2b200u);            // 2^28 vectors
+    return cudaGetLastError();
+}
+
+cudaError_t launch_selftest_packed(int* dev_failures, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(dev_failures, 0, sizeof(int), st);
+    if (e != cudaSuccess) return e;
+    k_selftest_packed<<<4096, 256, 0, st>>>(dev_failures, 0xf32c2u);                 // 2^26 operand sets
     return cudaGetLastError();
 }
 

@@ -44,6 +44,7 @@ cudaError_t launch_env_color(const FrameView& fr, const float* dir, int n, float
 cudaError_t launch_philox(const uint32_t ctr[4], const uint32_t key[2], uint32_t* dev_out4, cudaStream_t st);
 cudaError_t launch_selftest_uniform(int* dev_failures, cudaStream_t st);
 cudaError_t launch_selftest_normalize(int* dev_failures, cudaStream_t st);
+cudaError_t launch_selftest_packed(int* dev_failures, cudaStream_t st);
 cudaError_t launch_pick(const SceneView& sc, const AccelSel& ac, const FrameView& fr, int px, int py, int* dev_id, cudaStream_t st);
 // A frame rendered INTO a surface (rt_render_frame): when the launch is the pixel-pool kernel's (1-2 samples), finished pixels are
 // resolved into `surface` by the render kernel itself and - with `mapped_host` - copied to the caller's page-locked surface chunk by

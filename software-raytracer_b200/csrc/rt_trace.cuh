@@ -26,7 +26,7 @@ static_assert(kThreads == kLaneThreads, "rt_bvh_lane.cuh lays the traversal stac
 //                                                                    form exists (bvh_wide.h) MODE 3 traverses that one
 // MODE 4: flat two-level accelerator (flat_build.h), everything staged in shared memory
 // Shared memory layout: [BVH stack: stack_entries x blockDim ints][spheres][cubes][nodes][refs]
-//                       MODE 4: [cluster boxes per octant: 16 x n_clusters float4][candidate queues: kFlatQueue x blockDim bytes][spheres][cubes][level-1 boxes][cull records][prim ids][cull slots]
+//                       MODE 4: [cluster boxes per octant: 16 x n_clusters float4][candidate queues: kFlatQueue x blockDim bytes][spheres][cubes][level-1 boxes][cull records, packed pairs][prim ids][cull slots]
 struct TraceCtx {
     const float4* sph; const float4* box; const float4* nodes; const int* refs;
     int* stack; float* stack_t; int stride;
@@ -45,6 +45,24 @@ constexpr int kCoopPairs = 64;                  // (owner lane, cluster) pairs p
 constexpr int kCoopCands = RTB_COOP_CANDS;      // sphere candidates per call (every pair full + every lane's level-1 queue full would be 64 * 8 + 32 * 56 = 2304:
                                                 // 4.6 KB per warp, which held the kernel at 6 CTAs per SM); a call whose upper bound is larger takes the per-lane fallback
 constexpr int kCoopBytesPerWarp = 6 * 32 * 4 + kCoopPairs * 2 + kCoopCands * 2 + 32 * 8;
+
+// Float4 i of the staged cull records (cull_pair): records j, j + 1 of a cluster (j = 0, 2, 4, 6) or of the singles become
+// [x_j x_j+1 y_j y_j+1][z_j z_j+1 R'_j R'_j+1] in place; a cluster's pad stays as it is. With an odd number of singles the last
+// pair's second half is zeros and one float4 more is staged than the host holds: it fits the slack of flat_staged_bytes(),
+// which counts one cull-slot byte per record, pads included, plus 16 bytes.
+__device__ __forceinline__ float4 flat_stage_cull(const float4* __restrict__ cull, int n_clusters, int n_singles, int i) {
+    const int nclu = kClusterStride * n_clusters;
+    int j, last;                                   // the pair's first record, the last record of its group
+    if (i < nclu) {
+        const int w = i % kClusterStride;
+        if (w == 8) return __ldg(cull + i);
+        j = i - w + (w & ~1); last = i - w + 7;
+    } else {
+        j = nclu + ((i - nclu) & ~1); last = nclu + n_singles - 1;
+    }
+    const float4 a = __ldg(cull + j), b = j + 1 <= last ? __ldg(cull + j + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
+    return ((i - j) & 1) ? make_float4(a.z, b.z, a.w, b.w) : make_float4(a.x, b.x, a.y, b.y);
+}
 
 template <int MODE>
 __device__ __forceinline__ TraceCtx setup_trace(const SceneView& sc, const BvhView& bv, const FlatView& fl, float4* smem) {
@@ -74,8 +92,9 @@ __device__ __forceinline__ TraceCtx setup_trace(const SceneView& sc, const BvhVi
         t.sph = p; t.box = p + sc.n_sph; p += ng;
         for (int i = threadIdx.x; i < nb; i += blockDim.x) p[i] = __ldg(fl.boxes + i);
         t.fl.boxes = p; p += nb;
-        for (int i = threadIdx.x; i < ncull; i += blockDim.x) p[i] = __ldg(fl.cull + i);
-        t.fl.cull = p; p += ncull;
+        const int nstaged = ncull + (fl.n_singles & 1);
+        for (int i = threadIdx.x; i < nstaged; i += blockDim.x) p[i] = flat_stage_cull(fl.cull, fl.n_clusters, fl.n_singles, i);
+        t.fl.cull = p; p += nstaged;
         int* ids = reinterpret_cast<int*>(p);
         for (int i = threadIdx.x; i < np; i += blockDim.x) ids[i] = __ldg(fl.prim_id + i);
         t.fl.prim_id = ids;
@@ -149,11 +168,13 @@ __device__ __forceinline__ unsigned int warp_incl_scan(unsigned int v, int lane)
     return v;
 }
 
-// the rare per-lane fallback, kept out of line so it does not dilute the instruction cache of the hot loop
+// the rare per-lane fallback, kept out of line so it does not dilute the instruction cache of the hot loop. It culls one record at a
+// time: with the packed culls' register pairs in this callee, the 72-register form of the caller spills its path state across the
+// whole query (172 B of spill stores instead of none); the fallback's speed does not matter.
 static __device__ __noinline__ Hit flat_levels23_outlined(const SceneView& sc, const FlatView& fv, const float4* __restrict__ sph,
                                                    const float4* __restrict__ box, unsigned char* __restrict__ q, int qstride,
                                                    float3 o, float3 d, unsigned int cm, int nq) {
-    return flat_levels23(sc, fv, sph, box, q, qstride, o, d, cm, nq);
+    return flat_levels23<false>(sc, fv, sph, box, q, qstride, o, d, cm, nq);
 }
 
 __device__ __forceinline__ Hit closest_hit_flat_coop(const SceneView& sc, const FlatView& fv, const float4* __restrict__ sph,
