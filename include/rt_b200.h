@@ -240,6 +240,27 @@ int rt_resolve_rgba8(rt_ctx* ctx, uint32_t* host_out, int pitch_bytes, int flip_
  * filled frames, preview, shards of a multi-GPU render) run the two steps back to back. Synchronises. */
 int rt_render_frame(rt_ctx* ctx, int spp, uint32_t* host_out, int pitch_bytes, int flip_y);
 
+/* Denoised resolve: an edge-avoiding a-trous filter (B3-spline taps at steps 1, 2, 4, ..) over the mean radiance, guided by the
+ * primary-hit cache (object id, normal, t per pixel; RT_OPT_PRIMARY_REUSE), in front of the plain resolve. A pixel never takes colour
+ * from another object or from the sky; within an object the normal and the relative depth stop it at creases; the colour tolerance
+ * shrinks as sigma_color * 2^-pass / sqrt(samples), so a converged image is left almost untouched. Sky pixels come out exactly as
+ * rt_resolve_rgba8 gives them. The guides describe the CURRENT camera and scene: denoise after rendering and before moving (a call
+ * after rt_set_camera / rt_set_scene filters the buffer with the new pose's guides). If the cache is not valid (also with
+ * RT_OPT_PRIMARY_REUSE 0) the call traces it first; those queries count in traced_segments. Neither call changes the accumulation
+ * buffer, the sample counter, segments or paths; last_resolve_ms reports the device time of filter + pack. Preview mode, and
+ * passes 0, give the plain resolve. Bad parameters: RT_ERR_INVALID. See DESIGN.md 5 for the filter's definition. */
+typedef struct {
+    int32_t passes;         /* 0..8; 0 = the plain resolve, bit for bit */
+    int32_t normal_power;   /* P: 1, 2, 4, .. 256 */
+    float sigma_color;      /* sigma_c: tolerance on Reinhard luminance at 1 spp */
+    float sigma_depth;      /* sigma_z: relative depth tolerance per pixel of step */
+} rt_denoise_params;        /* 16 bytes */
+void rt_default_denoise_params(rt_denoise_params* p);
+/* rt_resolve_rgba8 with the filter in front. NULL params = defaults. Synchronises. */
+int rt_denoise_rgba8(rt_ctx* ctx, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y);
+/* The filtered MEAN radiance, width*height float4 (r,g,b,0), y-up: rt_read_accum's layout. Synchronises. */
+int rt_read_denoised(rt_ctx* ctx, const rt_denoise_params* p, float* host_rgba);
+
 /* Page-locked host memory for the surface handed to rt_resolve_rgba8 / rt_read_surface: the device-to-host copy
  * then runs as one DMA instead of being staged by the driver (1280x720 frame loop: 0.30 ms instead of 0.44 ms per
  * frame). Any host pointer works; this is only faster. */

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -13,6 +14,7 @@
 #include <vector>
 
 #include "rt_ctx.h"
+#include "rt_denoise.cuh"
 #include "rt_host_pack.h"
 
 using namespace rtb;
@@ -536,6 +538,7 @@ int rt_destroy(rt_ctx* c) {
     cudaFree(c->d_accum); cudaFree(c->d_argb); cudaFree(c->d_counters); cudaFree(c->d_scratch);
     cudaFree(c->d_bvh_nodes); cudaFree(c->d_bvh_refs); cudaFree(c->d_bvh_slots); cudaFree(c->d_bvh_qnodes); cudaFree(c->d_wide_nodes); cudaFree(c->d_wide_refs); cudaFree(c->d_tune);
     cudaFree(c->d_tri); cudaFree(c->d_tri_obj); cudaFree(c->d_prim_nt); cudaFree(c->d_prim_id); cudaFree(c->d_flags);
+    cudaFree(c->d_denoise[0]); cudaFree(c->d_denoise[1]);
     wavefront_destroy(c->wf);
     cudaFree(c->d_flat_boxes); cudaFree(c->d_flat_cull); cudaFree(c->d_flat_slots); cudaFree(c->d_flat_ids);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -721,6 +724,8 @@ int rt_set_params(rt_ctx* c, const rt_params* p) {
         if (c->d_accum) { cudaFree(c->d_accum); c->d_accum = nullptr; }
         if (c->d_argb) { cudaFree(c->d_argb); c->d_argb = nullptr; }
         c->cap_pixels = 0;
+        for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }   // 32 B per pixel, sized for the old resolution
+        c->cap_denoise = 0;
         c->prim_valid = false;
         c->exch.ready = false;
         wavefront_release(c->wf);                              // sized for the old resolution (up to tens of GB)
@@ -965,6 +970,83 @@ int rt_resolve_rgba8(rt_ctx* c, uint32_t* host_out, int pitch_bytes, int flip_y)
     if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_resolve_rgba8");
     return RT_OK;
+}
+
+void rt_default_denoise_params(rt_denoise_params* p) {
+    if (!p) return;
+    p->passes = 5; p->normal_power = 128; p->sigma_color = 2.0f; p->sigma_depth = 1.0f;   // DESIGN.md 8: sigma_color tuned at 4 spp
+}
+
+// rt_denoise_rgba8 (host_out != NULL) and rt_read_denoised (host_rgba != NULL): the filter of rt_denoise.cu over the accumulation
+// buffer, guided by the primary-hit cache; read-only on the buffer, the sample counter and the path statistics.
+static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out, int pitch_bytes, int flip_y, float* host_rgba) {
+    int rc = prepare(c);
+    if (rc != RT_OK) return rc;
+    const int w = c->par.width, h = c->par.height;
+    const char* fn = host_out ? "rt_denoise_rgba8" : "rt_read_denoised";
+    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
+    rt_denoise_params p;
+    if (user) p = *user;
+    else rt_default_denoise_params(&p);
+    int pow_log2 = 0;
+    while (pow_log2 < 9 && (1 << pow_log2) != p.normal_power) ++pow_log2;
+    if (p.passes < 0 || p.passes > kDenoiseMaxPasses) return fail(c, RT_ERR_INVALID, std::string(fn) + ": passes must be 0 .. 8");
+    if (pow_log2 > 8) return fail(c, RT_ERR_INVALID, std::string(fn) + ": normal_power must be a power of two in 1 .. 256");
+    if (!(p.sigma_color > 0.f && p.sigma_color <= FLT_MAX) || !(p.sigma_depth > 0.f && p.sigma_depth <= FLT_MAX))
+        return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and positive");
+    // preview shading is deterministic: nothing to filter
+    const int passes = c->par.mode == RT_MODE_PREVIEW ? 0 : p.passes;
+    if (host_out && passes == 0) return rt_resolve_rgba8(c, host_out, pitch_bytes, flip_y);
+    const size_t px = (size_t)w * h;
+    if (passes > 0) {
+        AccelSel ac;
+        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
+        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
+    }
+    if (c->cap_denoise < px || !c->d_denoise[0]) {
+        RT_CUDA(c, cudaStreamSynchronize(c->stream));
+        for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }
+        c->cap_denoise = 0;
+        cudaError_t e = cudaMalloc((void**)&c->d_denoise[0], px * sizeof(float4));
+        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_denoise[1], px * sizeof(float4));
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }
+            return cuda_fail(c, e, "denoiser buffers");
+        }
+        c->cap_denoise = px;
+    }
+    uint32_t* mapped = host_out ? mapped_surface(host_out, pitch_bytes, w) : nullptr;
+    DenoiseLaunch d;
+    d.accum = c->d_accum; d.samples = c->samples;
+    d.nt = c->d_prim_nt; d.id = c->d_prim_id;
+    d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
+    d.sigma_color = p.sigma_color; d.sigma_depth = p.sigma_depth;
+    d.buf[0] = c->d_denoise[0]; d.buf[1] = c->d_denoise[1];
+    d.argb = host_out ? c->d_argb : nullptr; d.argb_host = mapped; d.flip_y = flip_y ? 1 : 0;
+    cudaEventRecord(c->ev2, c->stream);
+    cudaError_t e = launch_denoise(d, c->stream);
+    cudaEventRecord(c->ev3, c->stream);
+    if (e == cudaSuccess && host_rgba)
+        e = cudaMemcpyAsync(host_rgba, c->d_denoise[passes > 0 ? (passes - 1) & 1 : 0], px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
+    else if (e == cudaSuccess && !mapped) {
+        if (pitch_bytes == w * 4) e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
+        else e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
+    if (e != cudaSuccess) return cuda_fail(c, e, fn);
+    return RT_OK;
+}
+
+int rt_denoise_rgba8(rt_ctx* c, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y) {
+    if (!host_out) return fail(c, RT_ERR_INVALID, "rt_denoise_rgba8: bad output buffer");
+    return denoise(c, p, host_out, pitch_bytes, flip_y, nullptr);
+}
+
+int rt_read_denoised(rt_ctx* c, const rt_denoise_params* p, float* host_rgba) {
+    if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_read_denoised: NULL output");
+    return denoise(c, p, nullptr, 0, 0, host_rgba);
 }
 
 void* rt_host_alloc(size_t bytes) {

@@ -86,6 +86,8 @@ struct rt_ctx {
     float4* d_prim_nt = nullptr; int* d_prim_id = nullptr;
     size_t cap_prim = 0;
     bool prim_valid = false;
+    float4* d_denoise[2] = {nullptr, nullptr};    // ping-pong images of the denoiser (rt_denoise.cu), allocated on first use
+    size_t cap_denoise = 0;
     ExchFlags* d_flags = nullptr;                 // this context's exchange flags (rt_exchange_*), zeroed at creation
     ExchangeState exch;
     uint32_t* d_scratch = nullptr;                // small device scratch (philox / pick)

@@ -1,4 +1,4 @@
-// rt_kernels.h - host-visible launchers of the CUDA kernels in rt_kernels.cu and rt_wavefront.cu.
+// rt_kernels.h - host-visible launchers of the CUDA kernels in rt_kernels.cu, rt_wavefront.cu and rt_denoise.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -75,6 +75,24 @@ cudaError_t launch_resolve(const float4* accum, uint32_t samples, int width, int
 
 cudaError_t launch_resolve_fused(const PeerPtrs& peers, int world, uint32_t samples, int width, int height, int first, int n,
                                  int flip_y, uint32_t* out, cudaStream_t st);
+
+// ---- denoised resolve (rt_denoise.cu; filter in rt_denoise.cuh) ----------------------------------------------------
+// Largest a-trous step whose pass stages its tile + apron in shared memory; larger steps read through L1 (measured: DESIGN.md 8).
+constexpr int kDenoiseStageDefault = 4;
+struct DenoiseLaunch {
+    const float4* accum; uint32_t samples;     // the accumulation buffer (samples 0: it holds a mean)
+    const float4* nt; const int* id;           // guides: the primary-hit cache (unused when passes == 0)
+    int width, height;
+    int passes;                                // 0: no filtering (the plain mean / resolve)
+    int pow_log2;                              // log2 of the normal power P
+    float sigma_color, sigma_depth;
+    float4* buf[2];                            // ping-pong (r, g, b, l) images; the result of a mean output is in buf[(passes - 1) & 1]
+                                               // (buf[0] for passes == 0) as (r, g, b, 0)
+    uint32_t* argb;                            // non-NULL: the last pass packs ARGB8 into this device surface instead (whole image) ...
+    uint32_t* argb_host;                       // ... and into this device alias of a page-locked host surface, if non-NULL
+    int flip_y;
+};
+cudaError_t launch_denoise(const DenoiseLaunch& d, cudaStream_t st);
 
 // Exchange flags of one rank (rt_exchange_*): arrive[r] / done[r] are written by rank r (over NVLink when r is a peer) with
 // the epoch of the exchange; epochs only grow. 256 bytes, zeroed once when the context is created.

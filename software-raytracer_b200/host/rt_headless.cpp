@@ -1,11 +1,13 @@
 // rt_headless - headless driver over the C-ABI: the reference's main loop without SDL/ImGui.
 //   rt_headless --scene Scenes/Scene1.json [--width 1280 --height 720 --spp 64 --bounces 8]
-//               [--preview] [--scale S] [--out frame.ppm] [--interactive N] [--gpus G]
+//               [--preview] [--scale S] [--out frame.ppm] [--interactive N] [--gpus G] [--denoise K]
 // --gpus G (G > 1): the library-owned multi-GPU group (rt_create_multi): the spp are sharded over G devices of this
 // process and one fused reduce + resolve kernel per frame writes device 0's surface (path mode, full resolution).
 // --scale S: the reference's SCREEN_SCALE (render scale slider, default here 1.0 = every pixel; the reference's is 0.5).
 // --interactive N: N frames of 1 spp + resolve + download each (the viewer's per-frame work,
 // BASELINE config 5) and prints p50/p99 frame latency.
+// --denoise K: the final image, and every --interactive frame, is presented through K passes of the edge-avoiding a-trous
+// filter (rt_denoise_rgba8; single GPU only).
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -30,7 +32,7 @@ struct Pinned {
 
 int main(int argc, char** argv) {
     std::string scene_path, out_path;
-    int w = 1280, h = 720, spp = 64, bounces = 8, interactive = 0, gpus = 1;
+    int w = 1280, h = 720, spp = 64, bounces = 8, interactive = 0, gpus = 1, denoise = 0;
     bool preview = false;
     float scale = 1.0f;
     for (int i = 1; i < argc; ++i) {
@@ -44,10 +46,16 @@ int main(int argc, char** argv) {
         else if (arg("--interactive")) interactive = atoi(argv[++i]);
         else if (arg("--scale")) scale = (float)atof(argv[++i]);
         else if (arg("--gpus")) gpus = atoi(argv[++i]);
+        else if (arg("--denoise")) denoise = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--preview")) preview = true;
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
     }
     if (scene_path.empty()) { fprintf(stderr, "usage: rt_headless --scene file.json [options]\n"); return 2; }
+    if (denoise < 0 || denoise > 8) { fprintf(stderr, "rt_headless: --denoise takes 0 .. 8 passes\n"); return 2; }
+    if (gpus > 1 && denoise > 0) {
+        fprintf(stderr, "rt_headless: --denoise is not supported with --gpus > 1 (a member's buffer holds only its shard of the samples)\n");
+        return 2;
+    }
     if (gpus > 1) {
         // what the reference does with 16 worker threads, across devices: spawn (rt_create_multi), frames (rt_group_render_spp),
         // join + present (rt_group_resolve_rgba8)
@@ -87,6 +95,7 @@ int main(int argc, char** argv) {
         rtb200::Raytracer rt(w, h);
         rt.SetObjectsToRender(scene1.GetObjects());
         rt.SIMPLEDRAW = preview; rt.MAXBOUNCES = bounces; rt.TARGETFRAMES = 1 << 30; rt.SCREEN_SCALE = scale;
+        rt.DENOISE_PASSES = denoise;
         Pinned surface((size_t)w * h);                          // interactive frames are streamed into it by the render kernel itself (rt_render_frame)
         using clk = std::chrono::steady_clock;
         if (interactive > 0) {

@@ -52,6 +52,10 @@ class RtStats(C.Structure):
                 ("traced_segments", C.c_uint64), ("total_traced_segments", C.c_uint64)]
 
 
+class RtDenoiseParams(C.Structure):
+    _fields_ = [("passes", C.c_int32), ("normal_power", C.c_int32), ("sigma_color", C.c_float), ("sigma_depth", C.c_float)]
+
+
 class RtTraversalStats(C.Structure):
     _fields_ = [("queries", C.c_uint64), ("node_visits", C.c_uint64), ("prim_tests", C.c_uint64),
                 ("sphere_tests", C.c_uint64), ("cube_tests", C.c_uint64), ("tri_tests", C.c_uint64),
@@ -77,6 +81,7 @@ EXPORTS = [
     "rt_create_multi", "rt_group_destroy", "rt_group_size", "rt_group_ctx", "rt_group_last_error", "rt_group_set_scene", "rt_group_load_scene",
     "rt_group_set_mesh", "rt_group_set_camera", "rt_group_set_params", "rt_group_set_option", "rt_group_reset_accumulation",
     "rt_group_render_spp", "rt_group_resolve_rgba8", "rt_group_get_stats",
+    "rt_default_denoise_params", "rt_denoise_rgba8", "rt_read_denoised",
 ]
 
 
@@ -108,7 +113,7 @@ def load_library(path=None):
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name in ("rt_host_alloc", "rt_host_free", "rt_last_error", "rt_accum_device_ptr", "rt_argb_device_ptr", "rt_create", "rt_default_params", "rt_default_camera",
-                    "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
+                    "rt_default_denoise_params", "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
             continue
         fn.restype = C.c_int
     lib.rt_group_ctx.restype = C.c_void_p
@@ -128,6 +133,7 @@ def load_library(path=None):
     lib.rt_host_free.argtypes = [C.c_void_p]
     lib.rt_default_params.restype = None
     lib.rt_default_camera.restype = None
+    lib.rt_default_denoise_params.restype = None
     lib.rt_rotate_camera.restype = None
     if path is None:
         _lib = lib
@@ -141,6 +147,15 @@ def _p(a):
 def default_params(**kw):
     p = RtParams()
     load_library().rt_default_params(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
+
+
+def default_denoise_params(**kw):
+    """rt_default_denoise_params, with any field overridden by keyword (passes, normal_power, sigma_color, sigma_depth)."""
+    p = RtDenoiseParams()
+    load_library().rt_default_denoise_params(C.byref(p))
     for k, v in kw.items():
         setattr(p, k, v)
     return p
@@ -326,6 +341,21 @@ class PathTracer:
         if out is None:
             out = np.zeros((h, w), np.uint32)
         self._chk(self.lib.rt_render_frame(self.h, int(spp), _p(out), out.strides[0], int(flip_y)))
+        return out
+
+    def denoise_rgba8(self, params=None, flip_y=True, out=None):
+        """rt_denoise_rgba8: the resolved frame with the a-trous filter in front (params None: the library's defaults)."""
+        w, h = self.params.width, self.params.height
+        if out is None:
+            out = np.zeros((h, w), np.uint32)
+        self._chk(self.lib.rt_denoise_rgba8(self.h, C.byref(params) if params is not None else None, _p(out), out.strides[0], int(flip_y)))
+        return out
+
+    def read_denoised(self, params=None):
+        """rt_read_denoised: the filtered mean radiance, (height, width, 4) float32 (r, g, b, 0), y-up."""
+        w, h = self.params.width, self.params.height
+        out = np.zeros((h, w, 4), np.float32)
+        self._chk(self.lib.rt_read_denoised(self.h, C.byref(params) if params is not None else None, _p(out)))
         return out
 
     def pick(self, x, y_window):
