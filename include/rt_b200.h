@@ -261,6 +261,41 @@ int rt_denoise_rgba8(rt_ctx* ctx, const rt_denoise_params* p, uint32_t* host_out
 /* The filtered MEAN radiance, width*height float4 (r,g,b,0), y-up: rt_read_accum's layout. Synchronises. */
 int rt_read_denoised(rt_ctx* ctx, const rt_denoise_params* p, float* host_rgba);
 
+/* Temporal resolve: carries the presented image across camera moves. The context keeps a history after every temporal call:
+ * per pixel the presented colour H and its weight W_H, that pose's primary-hit guides (object id, normal, t), the pose, the
+ * accumulation epoch (it changes on rt_reset_accumulation, rt_write_accum, rt_set_sample_count and a resize) and the radiance key
+ * (it changes on rt_set_scene, rt_load_scene, rt_set_mesh, rt_load_mesh_obj and any rt_set_params change of mode, max_bounces, the
+ * environment colours, sun_dir, dissipation or eps; not on the seed, selected_id or the pixel step). It also keeps a prior per pixel,
+ * colour P and weight w_P. A call
+ *   1. drops the history (w_P = 0 everywhere) when there is none, after rt_reset_temporal, a resize or a radiance-key change;
+ *   2. else, when the epoch or the pose (origin and axes of the rays) changed, rebuilds the prior: an identical pose copies it
+ *      (P = H, w_P = min(W_H, max_history)); otherwise every pixel with a primary hit projects its hit point into the history's
+ *      pose and takes the bilinear 2x2 history taps of the same object id within tau_depth * distance of the point and with
+ *      normals n_p . n_q >= tau_normal (w_P = min(max_history, sum b_q W_H), 0 when none counts); sky pixels get w_P = 0;
+ *   3. else keeps the prior (more samples were added, or the call was repeated);
+ *   4. presents O = (S + w_P P) / (N + w_P) (S the sample sum, N the sample count) where w_P > 0 and the pixel has a hit and N > 0,
+ *      elsewhere the plain mean, bit for bit rt_resolve_rgba8's; and stores (O, N + w_P) as the new history.
+ * With filter parameters (dn non-NULL, passes > 0) the a-trous filter of rt_denoise_rgba8 runs over O, its colour tolerance per
+ * pixel from N_eff = N + w_P instead of N; the history keeps the unfiltered O. Without a history the calls give exactly what
+ * rt_resolve_rgba8 / rt_read_denoised / rt_denoise_rgba8 give. No colour crosses an object id. Moving objects need a scene edit,
+ * which drops the history; mirror reflections lag by up to max_history frames. Preview mode gives the plain resolve and drops the
+ * history. Neither call changes the accumulation buffer, the sample counter, segments or paths; an invalid primary-hit cache is
+ * traced first (counted in traced_segments). last_resolve_ms reports the device time of reprojection, filter and pack. A shard
+ * context (rt_set_shard world > 1) and bad parameters: RT_ERR_INVALID. Synchronise. See DESIGN.md 5. */
+typedef struct {
+    int32_t max_history;    /* cap of the prior's weight in samples: 1 .. 4096 */
+    float tau_depth;        /* relative distance tolerance of a history tap, finite and > 0 */
+    float tau_normal;       /* smallest n_p . n_q of a history tap, -1 .. 1 */
+    int32_t reserved;
+} rt_temporal_params;       /* 16 bytes */
+void rt_default_temporal_params(rt_temporal_params* p);
+/* The temporally reprojected frame as ARGB8 (NULL tp = defaults; dn NULL or passes 0: no filter). */
+int rt_temporal_rgba8(rt_ctx* ctx, const rt_temporal_params* tp, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y);
+/* The same as width*height float4 (r, g, b, N_eff), y-up: rt_read_accum's layout (rgb filtered when dn asks for it). */
+int rt_read_temporal(rt_ctx* ctx, const rt_temporal_params* tp, const rt_denoise_params* dn, float* host_rgba);
+/* Forget the history: the next temporal call presents the plain (or filtered) mean. */
+int rt_reset_temporal(rt_ctx* ctx);
+
 /* Page-locked host memory for the surface handed to rt_resolve_rgba8 / rt_read_surface: the device-to-host copy
  * then runs as one DMA instead of being staged by the driver (1280x720 frame loop: 0.30 ms instead of 0.44 ms per
  * frame). Any host pointer works; this is only faster. */

@@ -268,6 +268,17 @@ int ensure_prim_cache(rt_ctx* c, const AccelSel& ac) {
     c->prim_valid = true;
     return RT_OK;
 }
+// the temporal resolve's history, guides and prior (88 B per pixel); the history is gone with them
+void release_temporal(rt_ctx* c) {
+    for (int k = 0; k < 2; ++k) {
+        cudaFree(c->d_tp_h[k]); cudaFree(c->d_tp_nt[k]); cudaFree(c->d_tp_id[k]);
+        c->d_tp_h[k] = c->d_tp_nt[k] = nullptr; c->d_tp_id[k] = nullptr;
+    }
+    cudaFree(c->d_tp_prior); c->d_tp_prior = nullptr;
+    c->cap_temporal = 0;
+    c->tp_valid = false;
+}
+
 // what the render launchers take: the cache when reuse is on, NULL when every sample re-traces its primary ray
 const PrimCache* prim_cache_arg(rt_ctx* c, PrimCache& pc) {
     if (!c->opt_primary_reuse) return nullptr;
@@ -539,6 +550,7 @@ int rt_destroy(rt_ctx* c) {
     cudaFree(c->d_bvh_nodes); cudaFree(c->d_bvh_refs); cudaFree(c->d_bvh_slots); cudaFree(c->d_bvh_qnodes); cudaFree(c->d_wide_nodes); cudaFree(c->d_wide_refs); cudaFree(c->d_tune);
     cudaFree(c->d_tri); cudaFree(c->d_tri_obj); cudaFree(c->d_prim_nt); cudaFree(c->d_prim_id); cudaFree(c->d_flags);
     cudaFree(c->d_denoise[0]); cudaFree(c->d_denoise[1]);
+    release_temporal(c);
     wavefront_destroy(c->wf);
     cudaFree(c->d_flat_boxes); cudaFree(c->d_flat_cull); cudaFree(c->d_flat_slots); cudaFree(c->d_flat_ids);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -557,6 +569,7 @@ int rt_load_scene(rt_ctx* c, const char* json_path) {
     std::string err;
     int rc = c->scene.Load(json_path, err);
     int up = upload_scene(c);                                  // also after a partial load, like the reference
+    ++c->radiance_key;
     rt_reset_accumulation(c);
     if (rc != RT_OK) return fail(c, rc, err);
     if (up != RT_OK) return up;
@@ -590,6 +603,7 @@ int rt_set_scene(rt_ctx* c, const rt_object* objects, int n) {
     const int keep_tuned = same ? c->tuned_accel : -1, keep_pipe = same ? c->tuned_pipeline : -1;
     const bool keep_flat = same && c->flat_valid;
     int rc = upload_scene(c);
+    ++c->radiance_key;
     if (rc != RT_OK) return rc;
     if (same) { c->bvh_valid = true; c->flat_valid = keep_flat; }
     c->tuned_accel = keep_tuned; c->tuned_pipeline = keep_pipe;
@@ -656,6 +670,7 @@ const char* rt_scene_name(rt_ctx* c) { return c ? c->scene.scene_name.c_str() : 
 // ---- mesh extension ------------------------------------------------------------------------------
 static int mesh_changed(rt_ctx* c) {
     int rc = upload_scene(c);
+    ++c->radiance_key;
     if (rc != RT_OK) return rc;
     return rt_reset_accumulation(c);
 }
@@ -713,8 +728,13 @@ int rt_set_params(rt_ctx* c, const rt_params* p) {
     if (!(fabsf(p->eps) <= fabsf(c->par.eps))) { c->bvh_valid = false; c->flat_valid = false; }   // margins were derived for the old offset
     if (resized || p->max_bounces != c->par.max_bounces || p->mode != c->par.mode) c->tuned_accel = c->tuned_pipeline = -1;
     // the primary-hit cache keeps the environment colour of the pixels whose primary ray misses
-    if (memcmp(p->sun_dir, c->par.sun_dir, sizeof p->sun_dir) || memcmp(p->sky, c->par.sky, sizeof p->sky) || memcmp(p->horizon, c->par.horizon, sizeof p->horizon) ||
-        memcmp(p->ground, c->par.ground, sizeof p->ground) || memcmp(p->sun, c->par.sun, sizeof p->sun)) c->prim_valid = false;
+    const bool env_changed = memcmp(p->sun_dir, c->par.sun_dir, sizeof p->sun_dir) || memcmp(p->sky, c->par.sky, sizeof p->sky) ||
+                             memcmp(p->horizon, c->par.horizon, sizeof p->horizon) || memcmp(p->ground, c->par.ground, sizeof p->ground) ||
+                             memcmp(p->sun, c->par.sun, sizeof p->sun);
+    if (env_changed) c->prim_valid = false;
+    // what changes the expected radiance ends a temporal history (the seed, selected_id and the pixel step do not)
+    if (p->mode != c->par.mode || (p->max_bounces < 0 ? 0 : p->max_bounces) != c->par.max_bounces || env_changed ||
+        memcmp(&p->dissipation, &c->par.dissipation, sizeof p->dissipation) || memcmp(&p->eps, &c->par.eps, sizeof p->eps)) ++c->radiance_key;
     c->par = *p;
     if (c->par.max_bounces < 0) c->par.max_bounces = 0;        // MAXBOUNCES = max(MAXBOUNCES, 0) Raytracer.cpp:475
     c->frame_dirty = true;
@@ -726,6 +746,8 @@ int rt_set_params(rt_ctx* c, const rt_params* p) {
         c->cap_pixels = 0;
         for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }   // 32 B per pixel, sized for the old resolution
         c->cap_denoise = 0;
+        release_temporal(c);                                   // sized for the old resolution
+        ++c->accum_epoch;
         c->prim_valid = false;
         c->exch.ready = false;
         wavefront_release(c->wf);                              // sized for the old resolution (up to tens of GB)
@@ -818,6 +840,7 @@ int rt_reset_accumulation(rt_ctx* c) {
     RT_CUDA(c, cudaMemsetAsync(c->d_counters + 2, 0, sizeof(unsigned long long), c->stream));
     RT_CUDA(c, cudaMemsetAsync(c->d_counters + 8, 0, 8 * sizeof(unsigned long long), c->stream));
     c->samples = 0; c->next_sample = 0; c->paths = 0;
+    ++c->accum_epoch;
     return RT_OK;
 }
 
@@ -977,32 +1000,21 @@ void rt_default_denoise_params(rt_denoise_params* p) {
     p->passes = 5; p->normal_power = 128; p->sigma_color = 2.0f; p->sigma_depth = 1.0f;   // DESIGN.md 8: sigma_color tuned at 4 spp
 }
 
-// rt_denoise_rgba8 (host_out != NULL) and rt_read_denoised (host_rgba != NULL): the filter of rt_denoise.cu over the accumulation
-// buffer, guided by the primary-hit cache; read-only on the buffer, the sample counter and the path statistics.
-static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out, int pitch_bytes, int flip_y, float* host_rgba) {
-    int rc = prepare(c);
-    if (rc != RT_OK) return rc;
-    const int w = c->par.width, h = c->par.height;
-    const char* fn = host_out ? "rt_denoise_rgba8" : "rt_read_denoised";
-    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
-    rt_denoise_params p;
+// the filter parameters of rt_denoise_rgba8 / rt_read_denoised / the temporal calls (NULL: the defaults) and log2 of the normal power
+static int check_denoise_params(rt_ctx* c, const char* fn, const rt_denoise_params* user, rt_denoise_params& p, int& pow_log2) {
     if (user) p = *user;
     else rt_default_denoise_params(&p);
-    int pow_log2 = 0;
+    pow_log2 = 0;
     while (pow_log2 < 9 && (1 << pow_log2) != p.normal_power) ++pow_log2;
     if (p.passes < 0 || p.passes > kDenoiseMaxPasses) return fail(c, RT_ERR_INVALID, std::string(fn) + ": passes must be 0 .. 8");
     if (pow_log2 > 8) return fail(c, RT_ERR_INVALID, std::string(fn) + ": normal_power must be a power of two in 1 .. 256");
     if (!(p.sigma_color > 0.f && p.sigma_color <= FLT_MAX) || !(p.sigma_depth > 0.f && p.sigma_depth <= FLT_MAX))
         return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and positive");
-    // preview shading is deterministic: nothing to filter
-    const int passes = c->par.mode == RT_MODE_PREVIEW ? 0 : p.passes;
-    if (host_out && passes == 0) return rt_resolve_rgba8(c, host_out, pitch_bytes, flip_y);
-    const size_t px = (size_t)w * h;
-    if (passes > 0) {
-        AccelSel ac;
-        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
-        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
-    }
+    return RT_OK;
+}
+
+// the filter's ping-pong images, 32 B per pixel
+static int ensure_denoise_buffers(rt_ctx* c, size_t px) {
     if (c->cap_denoise < px || !c->d_denoise[0]) {
         RT_CUDA(c, cudaStreamSynchronize(c->stream));
         for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }
@@ -1016,6 +1028,30 @@ static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out,
         }
         c->cap_denoise = px;
     }
+    return RT_OK;
+}
+
+// rt_denoise_rgba8 (host_out != NULL) and rt_read_denoised (host_rgba != NULL): the filter of rt_denoise.cu over the accumulation
+// buffer, guided by the primary-hit cache; read-only on the buffer, the sample counter and the path statistics.
+static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out, int pitch_bytes, int flip_y, float* host_rgba) {
+    int rc = prepare(c);
+    if (rc != RT_OK) return rc;
+    const int w = c->par.width, h = c->par.height;
+    const char* fn = host_out ? "rt_denoise_rgba8" : "rt_read_denoised";
+    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
+    rt_denoise_params p;
+    int pow_log2;
+    if ((rc = check_denoise_params(c, fn, user, p, pow_log2)) != RT_OK) return rc;
+    // preview shading is deterministic: nothing to filter
+    const int passes = c->par.mode == RT_MODE_PREVIEW ? 0 : p.passes;
+    if (host_out && passes == 0) return rt_resolve_rgba8(c, host_out, pitch_bytes, flip_y);
+    const size_t px = (size_t)w * h;
+    if (passes > 0) {
+        AccelSel ac;
+        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
+        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
+    }
+    if ((rc = ensure_denoise_buffers(c, px)) != RT_OK) return rc;
     uint32_t* mapped = host_out ? mapped_surface(host_out, pitch_bytes, w) : nullptr;
     DenoiseLaunch d;
     d.accum = c->d_accum; d.samples = c->samples;
@@ -1024,6 +1060,7 @@ static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out,
     d.sigma_color = p.sigma_color; d.sigma_depth = p.sigma_depth;
     d.buf[0] = c->d_denoise[0]; d.buf[1] = c->d_denoise[1];
     d.argb = host_out ? c->d_argb : nullptr; d.argb_host = mapped; d.flip_y = flip_y ? 1 : 0;
+    d.neff = nullptr;
     cudaEventRecord(c->ev2, c->stream);
     cudaError_t e = launch_denoise(d, c->stream);
     cudaEventRecord(c->ev3, c->stream);
@@ -1047,6 +1084,130 @@ int rt_denoise_rgba8(rt_ctx* c, const rt_denoise_params* p, uint32_t* host_out, 
 int rt_read_denoised(rt_ctx* c, const rt_denoise_params* p, float* host_rgba) {
     if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_read_denoised: NULL output");
     return denoise(c, p, nullptr, 0, 0, host_rgba);
+}
+
+void rt_default_temporal_params(rt_temporal_params* p) {
+    if (!p) return;
+    p->max_history = 32; p->tau_depth = 0.02f; p->tau_normal = 0.9f; p->reserved = 0;   // DESIGN.md 8: chosen from a measured sweep
+}
+
+// rt_temporal_rgba8 (host_out != NULL) and rt_read_temporal (host_rgba != NULL): the prior from the history (rt_temporal.cuh), the
+// blend, optionally the filter in its per-pixel count form, then the new history; read-only on the accumulation buffer, the sample
+// counter and the path statistics.
+static int temporal(rt_ctx* c, const rt_temporal_params* user, const rt_denoise_params* dn_user, uint32_t* host_out, int pitch_bytes,
+                    int flip_y, float* host_rgba) {
+    int rc = prepare(c);
+    if (rc != RT_OK) return rc;
+    const int w = c->par.width, h = c->par.height;
+    const char* fn = host_out ? "rt_temporal_rgba8" : "rt_read_temporal";
+    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
+    if (c->world > 1) return fail(c, RT_ERR_INVALID, std::string(fn) + ": not supported on a shard (its buffer holds only part of the samples)");
+    rt_temporal_params tp;
+    if (user) tp = *user;
+    else rt_default_temporal_params(&tp);
+    if (tp.max_history < 1 || tp.max_history > 4096) return fail(c, RT_ERR_INVALID, std::string(fn) + ": max_history must be 1 .. 4096");
+    if (!(tp.tau_depth > 0.f && tp.tau_depth <= FLT_MAX)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_depth must be finite and positive");
+    if (!(tp.tau_normal >= -1.f && tp.tau_normal <= 1.f)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_normal must be in -1 .. 1");
+    rt_denoise_params dp;
+    int pow_log2 = 0;
+    if (dn_user) {
+        if ((rc = check_denoise_params(c, fn, dn_user, dp, pow_log2)) != RT_OK) return rc;
+    } else {
+        rt_default_denoise_params(&dp);
+        dp.passes = 0;
+    }
+    // preview shading is deterministic: the plain resolve, and no history
+    const bool preview = c->par.mode == RT_MODE_PREVIEW;
+    const int passes = preview ? 0 : dp.passes;
+    const size_t px = (size_t)w * h;
+    if (!preview) {
+        AccelSel ac;
+        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
+        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
+    }
+    if (c->cap_temporal < px || !c->d_tp_prior) {
+        RT_CUDA(c, cudaStreamSynchronize(c->stream));
+        release_temporal(c);
+        cudaError_t e = cudaSuccess;
+        for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
+            e = cudaMalloc((void**)&c->d_tp_h[k], px * sizeof(float4));
+            if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_nt[k], px * sizeof(float4));
+            if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_id[k], px * sizeof(int));
+        }
+        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_prior, px * sizeof(float4));
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            release_temporal(c);
+            return cuda_fail(c, e, "temporal history buffers");
+        }
+        c->cap_temporal = px;
+    }
+    if (passes > 0 && (rc = ensure_denoise_buffers(c, px)) != RT_OK) return rc;
+
+    TemporalLaunch t;
+    t.accum = c->d_accum; t.count = (float)c->samples;
+    t.nt = preview ? nullptr : c->d_prim_nt; t.id = preview ? nullptr : c->d_prim_id;
+    t.width = w; t.height = h;
+    t.cap = (float)tp.max_history; t.tau_z = tp.tau_depth; t.tau_n = tp.tau_normal;
+    t.cur.o = c->frame.cam_pos; t.cur.u = c->frame.u_axis; t.cur.v = c->frame.v_axis; t.cur.f = c->frame.fwd;
+    t.prev = c->tp_pose;
+    tp_inverse(t.prev, t.m);
+    // the prior: none without a history of the same radiance; rebuilt when the accumulation restarted or the pose moved
+    const bool same_pose = memcmp(&t.cur, &t.prev, sizeof t.cur) == 0;
+    if (preview || !c->tp_valid || c->tp_key != c->radiance_key) t.mode = kTpZero;
+    else if (c->tp_epoch != c->accum_epoch || !same_pose) t.mode = same_pose ? kTpCopy : kTpReproject;
+    else t.mode = kTpKeep;
+    const int old = c->tp_cur, cur = old ^ 1;
+    t.hist.h = c->d_tp_h[old]; t.hist.nt = c->d_tp_nt[old]; t.hist.id = c->d_tp_id[old];
+    t.prior = c->d_tp_prior;
+    t.h_out = c->d_tp_h[cur]; t.nt_out = c->d_tp_nt[cur]; t.id_out = c->d_tp_id[cur];
+    uint32_t* mapped = host_out ? mapped_surface(host_out, pitch_bytes, w) : nullptr;
+    t.next = passes > 0 ? c->d_denoise[1] : nullptr;
+    t.argb = host_out && passes == 0 ? c->d_argb : nullptr; t.argb_host = t.argb ? mapped : nullptr; t.flip_y = flip_y ? 1 : 0;
+    c->tp_valid = false;                                      // until the new history is complete
+    cudaEventRecord(c->ev2, c->stream);
+    cudaError_t e = launch_temporal(t, c->stream);
+    if (e == cudaSuccess && passes > 0) {
+        DenoiseLaunch d;
+        d.accum = nullptr; d.samples = 0;
+        d.nt = c->d_prim_nt; d.id = c->d_prim_id;
+        d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
+        d.sigma_color = dp.sigma_color; d.sigma_depth = dp.sigma_depth;
+        d.buf[0] = c->d_denoise[0]; d.buf[1] = c->d_denoise[1];
+        d.argb = host_out ? c->d_argb : nullptr; d.argb_host = mapped; d.flip_y = flip_y ? 1 : 0;
+        d.neff = t.h_out;
+        e = launch_denoise(d, c->stream);
+    }
+    cudaEventRecord(c->ev3, c->stream);
+    if (e == cudaSuccess && host_rgba)
+        e = cudaMemcpyAsync(host_rgba, passes > 0 ? c->d_denoise[(passes - 1) & 1] : t.h_out, px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
+    else if (e == cudaSuccess && !mapped) {
+        if (pitch_bytes == w * 4) e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
+        else e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
+    if (e != cudaSuccess) return cuda_fail(c, e, fn);
+    c->tp_cur = cur;
+    c->tp_valid = !preview;
+    c->tp_pose = t.cur; c->tp_epoch = c->accum_epoch; c->tp_key = c->radiance_key;
+    return RT_OK;
+}
+
+int rt_temporal_rgba8(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y) {
+    if (!host_out) return fail(c, RT_ERR_INVALID, "rt_temporal_rgba8: bad output buffer");
+    return temporal(c, p, dn, host_out, pitch_bytes, flip_y, nullptr);
+}
+
+int rt_read_temporal(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, float* host_rgba) {
+    if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_read_temporal: NULL output");
+    return temporal(c, p, dn, nullptr, 0, 0, host_rgba);
+}
+
+int rt_reset_temporal(rt_ctx* c) {
+    if (!c) return RT_ERR_INVALID;
+    c->tp_valid = false;
+    return RT_OK;
 }
 
 void* rt_host_alloc(size_t bytes) {
@@ -1074,6 +1235,7 @@ int rt_write_accum(rt_ctx* c, const float* host_rgba, uint32_t samples) {
     RT_CUDA(c, cudaMemcpyAsync(c->d_accum, host_rgba, (size_t)c->par.width * c->par.height * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     c->samples = samples; c->next_sample = samples;
+    ++c->accum_epoch;
     return RT_OK;
 }
 
@@ -1370,6 +1532,7 @@ int rt_sync(rt_ctx* c) {
 int rt_set_sample_count(rt_ctx* c, uint32_t samples) {
     if (!c) return RT_ERR_INVALID;
     c->samples = samples;
+    ++c->accum_epoch;
     return RT_OK;
 }
 

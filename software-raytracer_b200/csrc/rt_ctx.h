@@ -88,6 +88,18 @@ struct rt_ctx {
     bool prim_valid = false;
     float4* d_denoise[2] = {nullptr, nullptr};    // ping-pong images of the denoiser (rt_denoise.cu), allocated on first use
     size_t cap_denoise = 0;
+    // temporal resolve (rt_temporal.cu), allocated on first use, 88 B per pixel: history H and guides G as ping-pong pairs (half
+    // tp_cur holds the last call's), the prior P
+    float4* d_tp_h[2] = {nullptr, nullptr}; float4* d_tp_nt[2] = {nullptr, nullptr}; int* d_tp_id[2] = {nullptr, nullptr};
+    float4* d_tp_prior = nullptr;
+    size_t cap_temporal = 0;
+    int tp_cur = 0;
+    bool tp_valid = false;                        // a history exists; it belongs to tp_pose, tp_epoch and tp_key
+    TemporalPose tp_pose = {};
+    uint64_t tp_epoch = 0, tp_key = 0;
+    uint64_t accum_epoch = 0;                     // bumped whenever the accumulation restarts or is replaced (rt_reset_accumulation,
+                                                  // rt_write_accum, rt_set_sample_count, a resize)
+    uint64_t radiance_key = 0;                    // bumped whenever the expected radiance changes (scene, mesh, radiance parameters)
     ExchFlags* d_flags = nullptr;                 // this context's exchange flags (rt_exchange_*), zeroed at creation
     ExchangeState exch;
     uint32_t* d_scratch = nullptr;                // small device scratch (philox / pick)

@@ -7,12 +7,17 @@
 //
 // Small steps stage the CTA's 32 x 8 tile plus its 2s apron of colour, guide and id in shared memory (36 B per staged pixel); larger
 // steps, whose apron exceeds the tile, read the taps through L1 (__ldg). Compiled with -fmad=false like every file.
+//
+// The per-pixel count form (NEFF, behind the temporal resolve of rt_temporal.cu) filters a blend of samples and reprojected
+// history: every pass reads (r, g, b, l) images, and the colour tolerance of pixel p uses its own weight N_eff(p) instead of the
+// sample count (rt_temporal.cuh tp_kc).
 #include "rt_kernels.h"
 
 #include <cstdlib>
 
 #include "rt_denoise.cuh"
 #include "rt_resolve.cuh"
+#include "rt_temporal.cuh"
 
 namespace rtb {
 
@@ -24,8 +29,8 @@ constexpr int kDnMaxStagedStep = 4;   // (32 + 16) x (8 + 16) x 36 B = 41.5 KB: 
 enum { kDnOutNext = 0, kDnOutMean = 1, kDnOutArgb = 2 };
 
 struct DenoiseIO {
-    const float4* accum;       // pass 0 input: the accumulation buffer
-    float count;               // its sample count (0: it already holds a mean)
+    const float4* accum;       // pass 0 input: the accumulation buffer; NEFF: (r, g, b, N_eff) per pixel (rt_temporal.cu)
+    float count;               // its sample count (0: it already holds a mean); NEFF: sigma_c * sigma_c
     const float4* cin;         // later passes: (r, g, b, l) of the previous pass
     const float4* nt;          // guides: (normal, t) and object id per pixel (-1: the primary ray missed)
     const int* id;
@@ -43,11 +48,11 @@ __device__ __forceinline__ float4 dn_load(const DenoiseIO& io, size_t q) {
     return __ldg(io.cin + q);
 }
 
-template <int OUT>
+template <int OUT, bool NEFF>
 __device__ __forceinline__ void dn_store(const DenoiseIO& io, int x, int y, float4 o) {
     const size_t p = (size_t)x + (size_t)y * io.width;
     if (OUT == kDnOutNext) io.out[p] = o;
-    else if (OUT == kDnOutMean) io.out[p] = make_float4(o.x, o.y, o.z, 0.f);
+    else if (OUT == kDnOutMean) io.out[p] = make_float4(o.x, o.y, o.z, NEFF ? __ldg(io.accum + p).w : 0.f);
     else {
         const uint32_t v = resolve_pixel(o, 0.f);               // a mean already: count 0
         const size_t dst = (size_t)x + (size_t)(io.flip_y ? io.height - 1 - y : y) * io.width;
@@ -56,7 +61,7 @@ __device__ __forceinline__ void dn_store(const DenoiseIO& io, int x, int y, floa
     }
 }
 
-template <bool FIRST, bool STAGED, int OUT>
+template <bool FIRST, bool STAGED, int OUT, bool NEFF>
 __global__ void __launch_bounds__(kDnTileW * kDnTileH) k_denoise_pass(DenoiseIO io, DenoisePass ps) {
     extern __shared__ float4 dn_smem[];
     const int W = io.width, H = io.height, s = ps.step;
@@ -85,12 +90,14 @@ __global__ void __launch_bounds__(kDnTileW * kDnTileH) k_denoise_pass(DenoiseIO 
     const int kc = (threadIdx.y + apron) * sw + threadIdx.x + apron;   // centre in the staged window
     const int idp = io.copy_only ? -1 : STAGED ? s_id[kc] : __ldg(io.id + p);
     if (idp < 0) {                                             // sky (or no filtering): copied unchanged
-        dn_store<OUT>(io, x, y, dn_load<FIRST>(io, p));
+        dn_store<OUT, NEFF>(io, x, y, dn_load<FIRST>(io, p));
         return;
     }
     const float4 np = STAGED ? s_nt[kc] : __ldg(io.nt + p);
     const float4 cp = STAGED ? s_c[kc] : dn_load<FIRST>(io, p);
     const float dz = dn_depth_scale(ps, np.w);
+    DenoisePass pp = ps;
+    if (NEFF) pp.kc = tp_kc(s, __ldg(io.accum + p).w, io.count);
     DenoiseAcc acc = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll 1
     for (int dy = -2; dy <= 2; ++dy) {
@@ -111,19 +118,19 @@ __global__ void __launch_bounds__(kDnTileW * kDnTileH) k_denoise_pass(DenoiseIO 
                 if (__ldg(io.id + q) != idp) continue;
                 nq = __ldg(io.nt + q); cq = dn_load<FIRST>(io, q);
             }
-            const float w = dn_weight(dn_h(dx) * hy, np, dz, cp.w, nq, cq.w, ps);
+            const float w = dn_weight(dn_h(dx) * hy, np, dz, cp.w, nq, cq.w, pp);
             dn_add(acc, w, cq);
         }
     }
-    dn_store<OUT>(io, x, y, dn_finish(acc));
+    dn_store<OUT, NEFF>(io, x, y, dn_finish(acc));
 }
 
-template <bool FIRST, bool STAGED>
+template <bool FIRST, bool STAGED, bool NEFF = false>
 cudaError_t dn_launch(int out, dim3 grid, size_t smem, cudaStream_t st, const DenoiseIO& io, const DenoisePass& ps) {
     const dim3 block(kDnTileW, kDnTileH);
-    if (out == kDnOutNext) k_denoise_pass<FIRST, STAGED, kDnOutNext><<<grid, block, smem, st>>>(io, ps);
-    else if (out == kDnOutMean) k_denoise_pass<FIRST, STAGED, kDnOutMean><<<grid, block, smem, st>>>(io, ps);
-    else k_denoise_pass<FIRST, STAGED, kDnOutArgb><<<grid, block, smem, st>>>(io, ps);
+    if (out == kDnOutNext) k_denoise_pass<FIRST, STAGED, kDnOutNext, NEFF><<<grid, block, smem, st>>>(io, ps);
+    else if (out == kDnOutMean) k_denoise_pass<FIRST, STAGED, kDnOutMean, NEFF><<<grid, block, smem, st>>>(io, ps);
+    else k_denoise_pass<FIRST, STAGED, kDnOutArgb, NEFF><<<grid, block, smem, st>>>(io, ps);
     return cudaGetLastError();
 }
 
@@ -153,16 +160,19 @@ cudaError_t launch_denoise(const DenoiseLaunch& d, cudaStream_t st) {
         return dn_launch<true, false>(last_out, grid, 0, st, io, dn_pass(0, d.pow_log2, d.sigma_color, d.sigma_depth, d.samples));
     }
     const int stage_max = stage_max_step();
+    const bool neff = d.neff != nullptr;
+    if (neff) { io.accum = d.neff; io.count = d.sigma_color * d.sigma_color; }
     for (int i = 0; i < d.passes; ++i) {
         const DenoisePass ps = dn_pass(i, d.pow_log2, d.sigma_color, d.sigma_depth, d.samples);
         const bool staged = ps.step <= stage_max;
         const int a = 2 * ps.step;
         const size_t smem = staged ? (size_t)(kDnTileW + 2 * a) * (kDnTileH + 2 * a) * (2 * sizeof(float4) + sizeof(int)) : 0;
         const int out = i == d.passes - 1 ? last_out : kDnOutNext;
-        io.cin = i > 0 ? d.buf[(i - 1) & 1] : nullptr;
+        io.cin = i > 0 || neff ? d.buf[(i - 1) & 1] : nullptr;   // NEFF pass 0: buf[1]
         io.out = d.buf[i & 1];
         cudaError_t e;
-        if (i == 0) e = staged ? dn_launch<true, true>(out, grid, smem, st, io, ps) : dn_launch<true, false>(out, grid, smem, st, io, ps);
+        if (neff) e = staged ? dn_launch<false, true, true>(out, grid, smem, st, io, ps) : dn_launch<false, false, true>(out, grid, smem, st, io, ps);
+        else if (i == 0) e = staged ? dn_launch<true, true>(out, grid, smem, st, io, ps) : dn_launch<true, false>(out, grid, smem, st, io, ps);
         else e = staged ? dn_launch<false, true>(out, grid, smem, st, io, ps) : dn_launch<false, false>(out, grid, smem, st, io, ps);
         if (e != cudaSuccess) return e;
     }

@@ -1,9 +1,10 @@
-// rt_kernels.h - host-visible launchers of the CUDA kernels in rt_kernels.cu, rt_wavefront.cu and rt_denoise.cu.
+// rt_kernels.h - host-visible launchers of the CUDA kernels in rt_kernels.cu, rt_wavefront.cu, rt_denoise.cu and rt_temporal.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "rt_device.cuh"
+#include "rt_temporal.cuh"
 
 namespace rtb {
 
@@ -91,8 +92,30 @@ struct DenoiseLaunch {
     uint32_t* argb;                            // non-NULL: the last pass packs ARGB8 into this device surface instead (whole image) ...
     uint32_t* argb_host;                       // ... and into this device alias of a page-locked host surface, if non-NULL
     int flip_y;
+    const float4* neff;                        // non-NULL: the per-pixel count form behind the temporal resolve: pass 0 reads its (r, g, b, l)
+                                               // input from buf[1] (accum and samples are unused), each pixel's colour tolerance uses N_eff
+                                               // = neff[p].w instead of samples (rt_temporal.cuh tp_kc), and a mean output stores (r, g, b, N_eff)
 };
 cudaError_t launch_denoise(const DenoiseLaunch& d, cudaStream_t st);
+
+// ---- temporal resolve (rt_temporal.cu; per-pixel math in rt_temporal.cuh) -------------------------------------------
+struct TemporalLaunch {
+    const float4* accum; float count;          // S and N (count 0: the buffer holds a mean)
+    const float4* nt; const int* id;           // the current primary-hit cache; id NULL: no guides (preview), every pixel the plain mean
+    int width, height;
+    int mode;                                  // kTpKeep / kTpZero / kTpCopy / kTpReproject
+    float cap, tau_z, tau_n;
+    TemporalPose cur, prev;                    // the current pose and the history's
+    float m[9];                                // tp_inverse(prev)
+    TemporalHist hist;                         // the history the taps read
+    float4* prior;                             // (P.rgb, w_P) per pixel: read (kTpKeep) or rewritten
+    float4* h_out; float4* nt_out; int* id_out;   // the new history and guides
+    float4* next;                              // non-NULL: (O, l) for the filter's first pass ...
+    uint32_t* argb;                            // ... else, non-NULL: the ARGB8 pack of O into this device surface (whole image) ...
+    uint32_t* argb_host;                       // ... and into this device alias of a page-locked host surface, if non-NULL
+    int flip_y;
+};
+cudaError_t launch_temporal(const TemporalLaunch& t, cudaStream_t st);
 
 // Exchange flags of one rank (rt_exchange_*): arrive[r] / done[r] are written by rank r (over NVLink when r is a peer) with
 // the epoch of the exchange; epochs only grow. 256 bytes, zeroed once when the context is created.

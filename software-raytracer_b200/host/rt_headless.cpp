@@ -1,6 +1,6 @@
 // rt_headless - headless driver over the C-ABI: the reference's main loop without SDL/ImGui.
 //   rt_headless --scene Scenes/Scene1.json [--width 1280 --height 720 --spp 64 --bounces 8]
-//               [--preview] [--scale S] [--out frame.ppm] [--interactive N] [--gpus G] [--denoise K]
+//               [--preview] [--scale S] [--out frame.ppm] [--interactive N] [--gpus G] [--denoise K] [--temporal CAP] [--orbit DEG]
 // --gpus G (G > 1): the library-owned multi-GPU group (rt_create_multi): the spp are sharded over G devices of this
 // process and one fused reduce + resolve kernel per frame writes device 0's surface (path mode, full resolution).
 // --scale S: the reference's SCREEN_SCALE (render scale slider, default here 1.0 = every pixel; the reference's is 0.5).
@@ -8,6 +8,8 @@
 // BASELINE config 5) and prints p50/p99 frame latency.
 // --denoise K: the final image, and every --interactive frame, is presented through K passes of the edge-avoiding a-trous
 // filter (rt_denoise_rgba8; single GPU only).
+// --temporal CAP: frames are presented through the temporal resolve (rt_temporal_rgba8, history cap CAP, --denoise K as its filter;
+// single GPU only). --orbit DEG: the camera turns DEG degrees about its up axis before every --interactive frame (a fly-through).
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -32,9 +34,10 @@ struct Pinned {
 
 int main(int argc, char** argv) {
     std::string scene_path, out_path;
-    int w = 1280, h = 720, spp = 64, bounces = 8, interactive = 0, gpus = 1, denoise = 0;
+    int w = 1280, h = 720, spp = 64, bounces = 8, interactive = 0, gpus = 1, denoise = 0, temporal = 0;
     bool preview = false;
     float scale = 1.0f;
+    double orbit = 0.0;
     for (int i = 1; i < argc; ++i) {
         auto arg = [&](const char* n) { return !strcmp(argv[i], n) && i + 1 < argc; };
         if (arg("--scene")) scene_path = argv[++i];
@@ -47,6 +50,8 @@ int main(int argc, char** argv) {
         else if (arg("--scale")) scale = (float)atof(argv[++i]);
         else if (arg("--gpus")) gpus = atoi(argv[++i]);
         else if (arg("--denoise")) denoise = atoi(argv[++i]);
+        else if (arg("--temporal")) temporal = atoi(argv[++i]);
+        else if (arg("--orbit")) orbit = atof(argv[++i]);
         else if (!strcmp(argv[i], "--preview")) preview = true;
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
     }
@@ -54,6 +59,11 @@ int main(int argc, char** argv) {
     if (denoise < 0 || denoise > 8) { fprintf(stderr, "rt_headless: --denoise takes 0 .. 8 passes\n"); return 2; }
     if (gpus > 1 && denoise > 0) {
         fprintf(stderr, "rt_headless: --denoise is not supported with --gpus > 1 (a member's buffer holds only its shard of the samples)\n");
+        return 2;
+    }
+    if (temporal < 0 || temporal > 4096) { fprintf(stderr, "rt_headless: --temporal takes a history cap of 0 .. 4096\n"); return 2; }
+    if (gpus > 1 && temporal > 0) {
+        fprintf(stderr, "rt_headless: --temporal is not supported with --gpus > 1 (a member's buffer holds only its shard of the samples)\n");
         return 2;
     }
     if (gpus > 1) {
@@ -96,11 +106,14 @@ int main(int argc, char** argv) {
         rt.SetObjectsToRender(scene1.GetObjects());
         rt.SIMPLEDRAW = preview; rt.MAXBOUNCES = bounces; rt.TARGETFRAMES = 1 << 30; rt.SCREEN_SCALE = scale;
         rt.DENOISE_PASSES = denoise;
+        rt.TEMPORAL_HISTORY = temporal;
+        const float orbit_rad = (float)(orbit * M_PI / 180.0);
         Pinned surface((size_t)w * h);                          // interactive frames are streamed into it by the render kernel itself (rt_render_frame)
         using clk = std::chrono::steady_clock;
         if (interactive > 0) {
             std::vector<double> ms;
             for (int f = 0; f < interactive + 10; ++f) {
+                if (orbit != 0.0) { rt.camera.RotateAboutAxis(orbit_rad, rt.camera.up); rt.Invalidate(); }
                 auto t0 = clk::now();
                 rt.RenderFrame(surface.data(), w * 4);
                 double d = std::chrono::duration<double, std::milli>(clk::now() - t0).count();

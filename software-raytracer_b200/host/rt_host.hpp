@@ -125,6 +125,8 @@ public:
     bool SIMPLEDRAW = true;                                                         // :35
     int selectedObject = -1;                                                        // :53 (as an object index)
     int DENOISE_PASSES = 0;                         // > 0: frames are presented through the a-trous filter (rt_denoise_rgba8), 0: plain resolve
+    int TEMPORAL_HISTORY = 0;                       // > 0: frames are presented through the temporal resolve (rt_temporal_rgba8) with this
+                                                    // history cap (and DENOISE_PASSES as its filter), 0: off
     Transform camera;                                                               // :295-297
 
     Raytracer(int width = 1280, int height = 720, int device = 0) {                 // :26-27
@@ -178,10 +180,10 @@ public:
     // The same frame traced AND presented in one call (rt_render_frame): the reference's workers write the surface pixel by
     // pixel while they trace (SetScreenPixel inside renderArea, :63-76,250), and so does the render kernel for full-resolution
     // accumulation frames - with a page-locked surface the frame then costs the render alone.
-    // With DENOISE_PASSES > 0 the frame is traced (rt_render_spp) and then presented through the filter instead.
+    // With DENOISE_PASSES > 0 or TEMPORAL_HISTORY > 0 the frame is traced (rt_render_spp) and then presented through Present.
     bool RenderFrame(uint32_t* pixels, int pitch_bytes) {
         if (!BeginFrame()) return false;
-        if (DENOISE_PASSES > 0) {
+        if (DENOISE_PASSES > 0 || TEMPORAL_HISTORY > 0) {
             check(rt_render_spp(ctx, 1), ctx);
             Present(pixels, pitch_bytes);
         } else {
@@ -190,12 +192,18 @@ public:
         return true;
     }
     // SDL surface update (the resolve half of SetScreenPixel, Raytracer.cpp:73-75): ARGB8, rows y-down. With DENOISE_PASSES > 0
-    // through the edge-avoiding filter (rt_denoise_rgba8, the library's default tolerances).
+    // through the edge-avoiding filter (rt_denoise_rgba8, the library's default tolerances); with TEMPORAL_HISTORY > 0 through the
+    // temporal resolve (rt_temporal_rgba8: the library's default tolerances, TEMPORAL_HISTORY as the cap, the filter if asked for).
     void Present(uint32_t* pixels, int pitch_bytes) {
-        if (DENOISE_PASSES > 0) {
-            rt_denoise_params dp;
-            rt_default_denoise_params(&dp);
-            dp.passes = DENOISE_PASSES;
+        rt_denoise_params dp;
+        rt_default_denoise_params(&dp);
+        dp.passes = DENOISE_PASSES;
+        if (TEMPORAL_HISTORY > 0) {
+            rt_temporal_params tp;
+            rt_default_temporal_params(&tp);
+            tp.max_history = TEMPORAL_HISTORY;
+            check(rt_temporal_rgba8(ctx, &tp, DENOISE_PASSES > 0 ? &dp : nullptr, pixels, pitch_bytes, 1), ctx);
+        } else if (DENOISE_PASSES > 0) {
             check(rt_denoise_rgba8(ctx, &dp, pixels, pitch_bytes, 1), ctx);
         } else {
             check(rt_resolve_rgba8(ctx, pixels, pitch_bytes, 1), ctx);
@@ -215,7 +223,8 @@ private:
         rt_camera cam = camera.ToCamera(FOV);
         check(rt_set_camera(ctx, &cam), ctx);
         bool setFrame;
-        if (doSetFrame) { setFrame = true; ACCUMULATIONFRAMES = 1; progressiveResolutionScaler = 1.0f / 4.0f; doSetFrame = false; }   // :576-581
+        // :576-581; the 1/4-scale first frame only shows something quickly, which the reprojected history does with TEMPORAL_HISTORY > 0
+        if (doSetFrame) { setFrame = true; ACCUMULATIONFRAMES = 1; progressiveResolutionScaler = TEMPORAL_HISTORY > 0 ? 1.0f : 1.0f / 4.0f; doSetFrame = false; }
         else {
             setFrame = progressiveResolutionScaler != 1;                            // :584-587
             progressiveResolutionScaler = 1;

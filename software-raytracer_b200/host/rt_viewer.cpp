@@ -184,6 +184,7 @@ int main(int argc, char** argv) {
                 if (rt.SIMPLEDRAW) rt.SCREEN_SCALE = rt.SCREEN_SCALE < 0.25f ? 0.25f : rt.SCREEN_SCALE > 0.5f ? 0.5f : rt.SCREEN_SCALE;
                 if (rt.SCREEN_SCALE != scaleBefore) rt.Invalidate();      // block size changes: mixing would blur (the reference keeps accumulating)
                 ImGui::SliderInt("Denoise passes", &rt.DENOISE_PASSES, 0, 8);  // presentation only: the accumulation goes on
+                ImGui::SliderInt("Temporal history", &rt.TEMPORAL_HISTORY, 0, 256);   // 0: off; > 0: the image survives camera moves
             }
             ImGui::Text("Application average %.3f \nms/frame (%.1f FPS)", 1000.0f / io.Framerate, io.Framerate);
             ImGui::End();

@@ -56,6 +56,10 @@ class RtDenoiseParams(C.Structure):
     _fields_ = [("passes", C.c_int32), ("normal_power", C.c_int32), ("sigma_color", C.c_float), ("sigma_depth", C.c_float)]
 
 
+class RtTemporalParams(C.Structure):
+    _fields_ = [("max_history", C.c_int32), ("tau_depth", C.c_float), ("tau_normal", C.c_float), ("reserved", C.c_int32)]
+
+
 class RtTraversalStats(C.Structure):
     _fields_ = [("queries", C.c_uint64), ("node_visits", C.c_uint64), ("prim_tests", C.c_uint64),
                 ("sphere_tests", C.c_uint64), ("cube_tests", C.c_uint64), ("tri_tests", C.c_uint64),
@@ -82,6 +86,7 @@ EXPORTS = [
     "rt_group_set_mesh", "rt_group_set_camera", "rt_group_set_params", "rt_group_set_option", "rt_group_reset_accumulation",
     "rt_group_render_spp", "rt_group_resolve_rgba8", "rt_group_get_stats",
     "rt_default_denoise_params", "rt_denoise_rgba8", "rt_read_denoised",
+    "rt_default_temporal_params", "rt_temporal_rgba8", "rt_read_temporal", "rt_reset_temporal",
 ]
 
 
@@ -113,7 +118,7 @@ def load_library(path=None):
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name in ("rt_host_alloc", "rt_host_free", "rt_last_error", "rt_accum_device_ptr", "rt_argb_device_ptr", "rt_create", "rt_default_params", "rt_default_camera",
-                    "rt_default_denoise_params", "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
+                    "rt_default_denoise_params", "rt_default_temporal_params", "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
             continue
         fn.restype = C.c_int
     lib.rt_group_ctx.restype = C.c_void_p
@@ -134,6 +139,7 @@ def load_library(path=None):
     lib.rt_default_params.restype = None
     lib.rt_default_camera.restype = None
     lib.rt_default_denoise_params.restype = None
+    lib.rt_default_temporal_params.restype = None
     lib.rt_rotate_camera.restype = None
     if path is None:
         _lib = lib
@@ -156,6 +162,15 @@ def default_denoise_params(**kw):
     """rt_default_denoise_params, with any field overridden by keyword (passes, normal_power, sigma_color, sigma_depth)."""
     p = RtDenoiseParams()
     load_library().rt_default_denoise_params(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
+
+
+def default_temporal_params(**kw):
+    """rt_default_temporal_params, with any field overridden by keyword (max_history, tau_depth, tau_normal)."""
+    p = RtTemporalParams()
+    load_library().rt_default_temporal_params(C.byref(p))
     for k, v in kw.items():
         setattr(p, k, v)
     return p
@@ -357,6 +372,25 @@ class PathTracer:
         out = np.zeros((h, w, 4), np.float32)
         self._chk(self.lib.rt_read_denoised(self.h, C.byref(params) if params is not None else None, _p(out)))
         return out
+
+    def temporal_rgba8(self, tparams=None, dn=None, flip_y=True, out=None):
+        """rt_temporal_rgba8: the frame with the reprojected history blended in (tparams None: the library's defaults; dn None: no filter)."""
+        w, h = self.params.width, self.params.height
+        if out is None:
+            out = np.zeros((h, w), np.uint32)
+        self._chk(self.lib.rt_temporal_rgba8(self.h, C.byref(tparams) if tparams is not None else None, C.byref(dn) if dn is not None else None,
+                                             _p(out), out.strides[0], int(flip_y)))
+        return out
+
+    def read_temporal(self, tparams=None, dn=None):
+        """rt_read_temporal: (height, width, 4) float32 (r, g, b, N_eff), y-up."""
+        w, h = self.params.width, self.params.height
+        out = np.zeros((h, w, 4), np.float32)
+        self._chk(self.lib.rt_read_temporal(self.h, C.byref(tparams) if tparams is not None else None, C.byref(dn) if dn is not None else None, _p(out)))
+        return out
+
+    def reset_temporal(self):
+        self._chk(self.lib.rt_reset_temporal(self.h))
 
     def pick(self, x, y_window):
         i = C.c_int(-2)
