@@ -40,17 +40,9 @@ int cuda_fail(rt_ctx* c, cudaError_t e, const char* what) {
         if (e__ != cudaSuccess) return cuda_fail(ctx, e__, #call);      \
     } while (0)
 
+// scene and accelerator arrays: at least 16 elements, also for an empty scene
 template <typename T>
-cudaError_t ensure_capacity(T*& ptr, size_t& cap, size_t need) {
-    if (need <= cap && ptr) return cudaSuccess;
-    if (ptr) cudaFree(ptr);
-    ptr = nullptr; cap = 0;
-    size_t n = need < 16 ? 16 : need;
-    cudaError_t e = cudaMalloc((void**)&ptr, n * sizeof(T));
-    if (e == cudaSuccess) cap = n;
-    else { ptr = nullptr; cudaGetLastError(); }               // do not leave the failure for the next launch check to find
-    return e;
-}
+cudaError_t ensure_capacity(DeviceArray<T>& a, size_t need) { return a.reserve(need < 16 ? 16 : need); }
 
 void build_frame(rt_ctx* c) {
     fill_frame_view(c->cam, c->par, c->frame);
@@ -59,20 +51,11 @@ void build_frame(rt_ctx* c) {
 
 int ensure_buffers(rt_ctx* c) {
     size_t px = (size_t)c->par.width * c->par.height;
-    if (px > c->cap_pixels || !c->d_accum) {
-        if (c->d_accum) cudaFree(c->d_accum);
-        if (c->d_argb) cudaFree(c->d_argb);
-        c->d_accum = nullptr; c->d_argb = nullptr; c->cap_pixels = 0;
+    if (c->d_accum.capacity() < px) {
         c->exch.ready = false;                                 // peers hold mappings of the old buffers
-        cudaError_t e = cudaMalloc((void**)&c->d_accum, px * sizeof(float4));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_argb, px * sizeof(uint32_t));
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            cudaFree(c->d_accum); c->d_accum = nullptr;
-            return cuda_fail(c, e, "frame buffers");
-        }
-        c->cap_pixels = px;
-        RT_CUDA(c, cudaMemsetAsync(c->d_accum, 0, px * sizeof(float4), c->stream));
+        const cudaError_t e = reserve_all(px, c->d_accum, c->d_argb);
+        if (e != cudaSuccess) return cuda_fail(c, e, "frame buffers");
+        RT_CUDA(c, cudaMemsetAsync(c->d_accum.get(), 0, px * sizeof(float4), c->stream));
         c->samples = 0; c->next_sample = 0; c->paths = 0;
     }
     return RT_OK;
@@ -84,36 +67,36 @@ int upload_scene(rt_ctx* c) {
     std::vector<int> sph_id, box_id;
     pack_scene(objs, sph, sph_id, box, box_id, mat);
     RT_CUDA(c, cudaStreamSynchronize(c->stream));             // nothing in flight may still read the old arrays
-    RT_CUDA(c, ensure_capacity(c->d_sph, c->cap_sph, sph.size()));
-    RT_CUDA(c, ensure_capacity(c->d_sph_id, c->cap_sph_id, sph_id.size()));
-    RT_CUDA(c, ensure_capacity(c->d_box, c->cap_box, box.size()));
-    RT_CUDA(c, ensure_capacity(c->d_box_id, c->cap_box_id, box_id.size()));
-    RT_CUDA(c, ensure_capacity(c->d_mat, c->cap_mat, mat.size()));
+    RT_CUDA(c, ensure_capacity(c->d_sph, sph.size()));
+    RT_CUDA(c, ensure_capacity(c->d_sph_id, sph_id.size()));
+    RT_CUDA(c, ensure_capacity(c->d_box, box.size()));
+    RT_CUDA(c, ensure_capacity(c->d_box_id, box_id.size()));
+    RT_CUDA(c, ensure_capacity(c->d_mat, mat.size()));
     if (!sph.empty()) {
-        RT_CUDA(c, cudaMemcpyAsync(c->d_sph, sph.data(), sph.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-        RT_CUDA(c, cudaMemcpyAsync(c->d_sph_id, sph_id.data(), sph_id.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_sph.get(), sph.data(), sph.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_sph_id.get(), sph_id.data(), sph_id.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     }
     if (!box.empty()) {
-        RT_CUDA(c, cudaMemcpyAsync(c->d_box, box.data(), box.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-        RT_CUDA(c, cudaMemcpyAsync(c->d_box_id, box_id.data(), box_id.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_box.get(), box.data(), box.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_box_id.get(), box_id.data(), box_id.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     }
     if (!mat.empty())
-        RT_CUDA(c, cudaMemcpyAsync(c->d_mat, mat.data(), mat.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_mat.get(), mat.data(), mat.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     c->scene.meshes.resize(objs.size());
     build_tri_records(objs, c->scene.meshes, c->tris);
     const size_t nt = (size_t)c->tris.count();
-    RT_CUDA(c, ensure_capacity(c->d_tri, c->cap_tri, nt * 3));
-    RT_CUDA(c, ensure_capacity(c->d_tri_obj, c->cap_tri_obj, nt));
+    RT_CUDA(c, ensure_capacity(c->d_tri, nt * 3));
+    RT_CUDA(c, ensure_capacity(c->d_tri_obj, nt));
     if (nt) {
-        RT_CUDA(c, cudaMemcpyAsync(c->d_tri, c->tris.rec.data(), nt * 48, cudaMemcpyHostToDevice, c->stream));
-        RT_CUDA(c, cudaMemcpyAsync(c->d_tri_obj, c->tris.obj.data(), nt * 4, cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_tri.get(), c->tris.rec.data(), nt * 48, cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_tri_obj.get(), c->tris.obj.data(), nt * 4, cudaMemcpyHostToDevice, c->stream));
     }
     RT_CUDA(c, cudaStreamSynchronize(c->stream));             // host vectors die at return
-    c->view.sph = c->d_sph; c->view.sph_id = c->d_sph_id;
-    c->view.box = c->d_box; c->view.box_id = c->d_box_id;
-    c->view.mat = c->d_mat;
+    c->view.sph = c->d_sph.get(); c->view.sph_id = c->d_sph_id.get();
+    c->view.box = c->d_box.get(); c->view.box_id = c->d_box_id.get();
+    c->view.mat = c->d_mat.get();
     c->view.n_sph = (int)sph_id.size(); c->view.n_box = (int)box_id.size(); c->view.n_obj = (int)objs.size();
-    c->view.tri = c->d_tri; c->view.tri_obj = c->d_tri_obj; c->view.n_tri = (int)nt;
+    c->view.tri = c->d_tri.get(); c->view.tri_obj = c->d_tri_obj.get(); c->view.n_tri = (int)nt;
     c->bvh_valid = false; c->flat_valid = false; c->tuned_accel = c->tuned_pipeline = -1;
     c->prim_valid = false;
     return RT_OK;
@@ -134,17 +117,17 @@ int ensure_bvh(rt_ctx* c, float origin_extent) {
     c->wide = HostWideBvh();
     if (want_wide) build_wide_bvh(c->bvh, c->wide);           // not usable (huge extents, oversized leaves): the BVH2 is traversed
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
-    RT_CUDA(c, ensure_capacity(c->d_bvh_nodes, c->cap_bvh_nodes, c->bvh.nodes.size() * 4));
-    RT_CUDA(c, ensure_capacity(c->d_bvh_refs, c->cap_bvh_refs, c->bvh.refs.size()));
-    RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_nodes, c->bvh.nodes.data(), c->bvh.nodes.size() * sizeof(BvhNode), cudaMemcpyHostToDevice, c->stream));
+    RT_CUDA(c, ensure_capacity(c->d_bvh_nodes, c->bvh.nodes.size() * 4));
+    RT_CUDA(c, ensure_capacity(c->d_bvh_refs, c->bvh.refs.size()));
+    RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_nodes.get(), c->bvh.nodes.data(), c->bvh.nodes.size() * sizeof(BvhNode), cudaMemcpyHostToDevice, c->stream));
     if (!c->bvh.refs.empty())
-        RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_refs, c->bvh.refs.data(), c->bvh.refs.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_refs.get(), c->bvh.refs.data(), c->bvh.refs.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     if (c->wide.usable) {
-        RT_CUDA(c, ensure_capacity(c->d_wide_nodes, c->cap_wide_nodes, c->wide.nodes.size() * 5));
-        RT_CUDA(c, ensure_capacity(c->d_wide_refs, c->cap_wide_refs, c->wide.refs.size()));
-        RT_CUDA(c, cudaMemcpyAsync(c->d_wide_nodes, c->wide.nodes.data(), c->wide.nodes.size() * sizeof(WideNode), cudaMemcpyHostToDevice, c->stream));
+        RT_CUDA(c, ensure_capacity(c->d_wide_nodes, c->wide.nodes.size() * 5));
+        RT_CUDA(c, ensure_capacity(c->d_wide_refs, c->wide.refs.size()));
+        RT_CUDA(c, cudaMemcpyAsync(c->d_wide_nodes.get(), c->wide.nodes.data(), c->wide.nodes.size() * sizeof(WideNode), cudaMemcpyHostToDevice, c->stream));
         if (!c->wide.refs.empty())
-            RT_CUDA(c, cudaMemcpyAsync(c->d_wide_refs, c->wide.refs.data(), c->wide.refs.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+            RT_CUDA(c, cudaMemcpyAsync(c->d_wide_refs.get(), c->wide.refs.data(), c->wide.refs.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     }
     // leaf-ordered primitive slots for BVHs that are traversed from global memory (rt_trace.cuh pick_mode: MODE 3)
     c->bview.slots = nullptr;
@@ -156,10 +139,10 @@ int ensure_bvh(rt_ctx* c, float origin_extent) {
         if (staged > kMaxBvhStagedBytes && !c->wide.usable && !c->bvh.refs.empty()) {
             std::vector<float> slots;
             build_leaf_slots(c->bvh, reinterpret_cast<const float*>(sph.data()), sph_id.data(), reinterpret_cast<const float*>(box.data()), box_id.data(), &c->tris, slots);
-            RT_CUDA(c, ensure_capacity(c->d_bvh_slots, c->cap_bvh_slots, slots.size() / 4));
-            RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_slots, slots.data(), slots.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+            RT_CUDA(c, ensure_capacity(c->d_bvh_slots, slots.size() / 4));
+            RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_slots.get(), slots.data(), slots.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
             RT_CUDA(c, cudaStreamSynchronize(c->stream));     // the host vector dies here
-            c->bview.slots = c->d_bvh_slots;
+            c->bview.slots = c->d_bvh_slots.get();
         }
     }
     // ... and the 32-byte quantised form of the nodes for the persistent kernels (one 256-bit load per node visit)
@@ -168,19 +151,19 @@ int ensure_bvh(rt_ctx* c, float origin_extent) {
         HostQNodes qn;
         build_qnodes(c->bvh, qn);
         if (qn.usable) {
-            RT_CUDA(c, ensure_capacity(c->d_bvh_qnodes, c->cap_bvh_qnodes, qn.words.size() / 4));
-            RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_qnodes, qn.words.data(), qn.words.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+            RT_CUDA(c, ensure_capacity(c->d_bvh_qnodes, qn.words.size() / 4));
+            RT_CUDA(c, cudaMemcpyAsync(c->d_bvh_qnodes.get(), qn.words.data(), qn.words.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
             RT_CUDA(c, cudaStreamSynchronize(c->stream));
-            c->bview.qnodes = c->d_bvh_qnodes;
+            c->bview.qnodes = c->d_bvh_qnodes.get();
             c->bview.q_org = make_float3(qn.org[0], qn.org[1], qn.org[2]);
             c->bview.q_step = make_float3(qn.step[0], qn.step[1], qn.step[2]);
         }
     }
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->bview.nodes = c->d_bvh_nodes; c->bview.refs = c->d_bvh_refs;
+    c->bview.nodes = c->d_bvh_nodes.get(); c->bview.refs = c->d_bvh_refs.get();
     c->bview.n_nodes = (int)c->bvh.nodes.size(); c->bview.n_refs = (int)c->bvh.refs.size();
     c->bview.stack_entries = c->bvh.max_depth + 2;
-    c->bview.wnodes = c->wide.usable ? c->d_wide_nodes : nullptr; c->bview.wrefs = c->wide.usable ? c->d_wide_refs : nullptr;
+    c->bview.wnodes = c->wide.usable ? c->d_wide_nodes.get() : nullptr; c->bview.wrefs = c->wide.usable ? c->d_wide_refs.get() : nullptr;
     c->bview.n_wnodes = c->wide.usable ? (int)c->wide.nodes.size() : 0; c->bview.n_wrefs = c->wide.usable ? (int)c->wide.refs.size() : 0;
     c->bview.wstack_entries = c->wide.depth + 2;
     c->bview.q2f_hi = 0x47u;
@@ -197,16 +180,16 @@ int ensure_flat(rt_ctx* c, float origin_extent) {
     if (!c->flat.usable) return RT_OK;
     const HostFlat& f = c->flat;
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
-    RT_CUDA(c, ensure_capacity(c->d_flat_boxes, c->cap_flat_boxes, f.boxes.size() / 4));
-    RT_CUDA(c, ensure_capacity(c->d_flat_cull, c->cap_flat_cull, f.cull.size() / 4));
-    RT_CUDA(c, ensure_capacity(c->d_flat_slots, c->cap_flat_slots, f.cull_slot.size()));
-    RT_CUDA(c, ensure_capacity(c->d_flat_ids, c->cap_flat_ids, f.prim_id.size()));
-    if (!f.boxes.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_boxes, f.boxes.data(), f.boxes.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    if (!f.cull.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_cull, f.cull.data(), f.cull.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    if (!f.cull_slot.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_slots, f.cull_slot.data(), f.cull_slot.size(), cudaMemcpyHostToDevice, c->stream));
-    if (!f.prim_id.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_ids, f.prim_id.data(), f.prim_id.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    RT_CUDA(c, ensure_capacity(c->d_flat_boxes, f.boxes.size() / 4));
+    RT_CUDA(c, ensure_capacity(c->d_flat_cull, f.cull.size() / 4));
+    RT_CUDA(c, ensure_capacity(c->d_flat_slots, f.cull_slot.size()));
+    RT_CUDA(c, ensure_capacity(c->d_flat_ids, f.prim_id.size()));
+    if (!f.boxes.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_boxes.get(), f.boxes.data(), f.boxes.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    if (!f.cull.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_cull.get(), f.cull.data(), f.cull.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    if (!f.cull_slot.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_slots.get(), f.cull_slot.data(), f.cull_slot.size(), cudaMemcpyHostToDevice, c->stream));
+    if (!f.prim_id.empty()) RT_CUDA(c, cudaMemcpyAsync(c->d_flat_ids.get(), f.prim_id.data(), f.prim_id.size() * 4, cudaMemcpyHostToDevice, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->fview.boxes = c->d_flat_boxes; c->fview.cull = c->d_flat_cull; c->fview.cull_slot = c->d_flat_slots; c->fview.prim_id = c->d_flat_ids;
+    c->fview.boxes = c->d_flat_boxes.get(); c->fview.cull = c->d_flat_cull.get(); c->fview.cull_slot = c->d_flat_slots.get(); c->fview.prim_id = c->d_flat_ids.get();
     c->fview.n_clusters = f.n_clusters; c->fview.n_cubes = f.n_cubes; c->fview.n_singles = f.n_singles; c->fview.kappa = f.kappa;
     return RT_OK;
 }
@@ -253,36 +236,21 @@ int want_accel(rt_ctx* c) {
 // identical hits) and kept until the camera, the scene or the resolution changes.
 int ensure_prim_cache(rt_ctx* c, const AccelSel& ac) {
     const size_t px = (size_t)c->par.width * c->par.height;
-    if (c->prim_valid && c->cap_prim >= px) return RT_OK;
-    if (c->cap_prim < px) {
+    if (c->prim_valid && c->d_prim_nt.capacity() >= px) return RT_OK;
+    if (c->d_prim_nt.capacity() < px) {
         RT_CUDA(c, cudaStreamSynchronize(c->stream));
-        if (c->d_prim_nt) cudaFree(c->d_prim_nt);
-        if (c->d_prim_id) cudaFree(c->d_prim_id);
-        c->d_prim_nt = nullptr; c->d_prim_id = nullptr; c->cap_prim = 0;
-        cudaError_t e = cudaMalloc((void**)&c->d_prim_nt, px * sizeof(float4));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_prim_id, px * sizeof(int));
-        if (e != cudaSuccess) { cudaGetLastError(); cudaFree(c->d_prim_nt); c->d_prim_nt = nullptr; return cuda_fail(c, e, "primary-hit cache"); }
-        c->cap_prim = px;
+        const cudaError_t e = reserve_all(px, c->d_prim_nt, c->d_prim_id);
+        if (e != cudaSuccess) return cuda_fail(c, e, "primary-hit cache");
     }
-    RT_CUDA(c, launch_primary_cache(c->view, ac, c->frame, c->d_prim_nt, c->d_prim_id, c->d_counters, c->stream));
+    RT_CUDA(c, launch_primary_cache(c->view, ac, c->frame, c->d_prim_nt.get(), c->d_prim_id.get(), c->d_counters.get(), c->stream));
     c->prim_valid = true;
     return RT_OK;
-}
-// the temporal resolve's history, guides and prior (88 B per pixel); the history is gone with them
-void release_temporal(rt_ctx* c) {
-    for (int k = 0; k < 2; ++k) {
-        cudaFree(c->d_tp_h[k]); cudaFree(c->d_tp_nt[k]); cudaFree(c->d_tp_id[k]);
-        c->d_tp_h[k] = c->d_tp_nt[k] = nullptr; c->d_tp_id[k] = nullptr;
-    }
-    cudaFree(c->d_tp_prior); c->d_tp_prior = nullptr;
-    c->cap_temporal = 0;
-    c->tp_valid = false;
 }
 
 // what the render launchers take: the cache when reuse is on, NULL when every sample re-traces its primary ray
 const PrimCache* prim_cache_arg(rt_ctx* c, PrimCache& pc) {
     if (!c->opt_primary_reuse) return nullptr;
-    pc.nt = c->d_prim_nt; pc.id = c->d_prim_id;
+    pc.nt = c->d_prim_nt.get(); pc.id = c->d_prim_id.get();
     return &pc;
 }
 
@@ -309,9 +277,9 @@ int autotune_accel(rt_ctx* c, int spp) {
     int rc;
     for (int k = 0; k < n_cand; ++k) if ((rc = make_accel(c, kinds[k], camera_extent(c), sel[k])) != RT_OK) return rc;
     const size_t px = (size_t)c->par.width * c->par.height;
-    RT_CUDA(c, ensure_capacity(c->d_tune, c->cap_tune, px));
+    RT_CUDA(c, ensure_capacity(c->d_tune, px));
     cudaEvent_t* e = c->ev_tune;
-    unsigned long long* dummy = c->d_counters + 4;            // not part of the reported statistics
+    unsigned long long* dummy = c->d_counters.get() + 4;      // not part of the reported statistics
     cudaError_t err = cudaSuccess;
     PrimCache pc;
     if (c->opt_primary_reuse && (rc = ensure_prim_cache(c, sel[n_cand - 1])) != RT_OK) return rc;
@@ -319,7 +287,7 @@ int autotune_accel(rt_ctx* c, int spp) {
     for (int pass = 0; pass < 2 && err == cudaSuccess; ++pass) {   // pass 0 warms the instruction cache
         cudaEventRecord(e[0], c->stream);
         for (int k = 0; k < n_cand && err == cudaSuccess; ++k) {
-            err = launch_render_regen(c->view, sel[k], c->frame, c->d_tune, 0u, 16, prim, dummy, c->stream, 1, coop[k]);
+            err = launch_render_regen(c->view, sel[k], c->frame, c->d_tune.get(), 0u, 16, prim, dummy, c->stream, 1, coop[k]);
             cudaEventRecord(e[k + 1], c->stream);
         }
     }
@@ -349,10 +317,10 @@ int autotune_pipeline(rt_ctx* c, const AccelSel& ac, int spp) {
     // (the wavefront pipeline keeps one queue counter per bounce round: 60 rounds at most)
     if (ac.kind != kAccelBvh || prims < 2048 || c->pixel_step > 1 || c->par.max_bounces > 60) { c->tuned_pipeline = RT_PIPELINE_REGEN; return RT_OK; }
     const size_t px = (size_t)c->par.width * c->par.height;
-    RT_CUDA(c, ensure_capacity(c->d_tune, c->cap_tune, px));
+    RT_CUDA(c, ensure_capacity(c->d_tune, px));
     if (!c->wf) c->wf = wavefront_create();
     cudaEvent_t* e = c->ev_tune;
-    unsigned long long* dummy = c->d_counters + 4;
+    unsigned long long* dummy = c->d_counters.get() + 4;
     PrimCache pc;
     int rc;
     if (c->opt_primary_reuse && (rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
@@ -368,11 +336,11 @@ int autotune_pipeline(rt_ctx* c, const AccelSel& ac, int spp) {
     bool usable[3] = {true, true, true};
     for (int pass = 0; pass < 2 && err == cudaSuccess; ++pass) {   // pass 0 allocates the wavefront buffers and warms up
         cudaEventRecord(e[0], c->stream);
-        err = launch_render_regen(c->view, ac, c->frame, c->d_tune, 0u, pass ? n_regen : 1, prim, dummy, c->stream);
+        err = launch_render_regen(c->view, ac, c->frame, c->d_tune.get(), 0u, pass ? n_regen : 1, prim, dummy, c->stream);
         cudaEventRecord(e[1], c->stream);
         for (int k = 1; k <= 2 && err == cudaSuccess; ++k) {
             if (usable[k]) {
-                const cudaError_t we = launch_render_wavefront(c->wf, c->view, ac, c->frame, c->d_tune, 0u, n_tune, prim, dummy, c->stream, c->opt_bvh_sched == 0,
+                const cudaError_t we = launch_render_wavefront(c->wf, c->view, ac, c->frame, c->d_tune.get(), 0u, n_tune, prim, dummy, c->stream, c->opt_bvh_sched == 0,
                                                                c->opt_wf_refill, c->opt_wf_node_min, c->opt_wf_wave_mpaths, false, k == 2);
                 if (we == cudaErrorMemoryAllocation) usable[k] = false;      // no room for even the smallest wave: not a candidate
                 else err = we;
@@ -524,11 +492,11 @@ int rt_create(int cuda_device, rt_ctx** out) {
         (e = cudaEventCreate(&c->ev_tune[0])) != cudaSuccess || (e = cudaEventCreate(&c->ev_tune[1])) != cudaSuccess ||
         (e = cudaEventCreate(&c->ev_tune[2])) != cudaSuccess || (e = cudaEventCreate(&c->ev_tune[3])) != cudaSuccess ||
         (e = cudaEventCreate(&c->ev_tune[4])) != cudaSuccess ||
-        (e = cudaMalloc((void**)&c->d_counters, kCounters * sizeof(unsigned long long))) != cudaSuccess ||
-        (e = cudaMalloc((void**)&c->d_scratch, 4096)) != cudaSuccess ||
-        (e = cudaMalloc((void**)&c->d_flags, sizeof(ExchFlags))) != cudaSuccess ||
-        (e = cudaMemset(c->d_flags, 0, sizeof(ExchFlags))) != cudaSuccess ||
-        (e = cudaMemset(c->d_counters, 0, kCounters * sizeof(unsigned long long))) != cudaSuccess) {
+        (e = c->d_counters.reserve(kCounters)) != cudaSuccess ||
+        (e = c->d_scratch.reserve(4096 / sizeof(uint32_t))) != cudaSuccess ||
+        (e = c->d_flags.reserve(1)) != cudaSuccess ||
+        (e = cudaMemset(c->d_flags.get(), 0, sizeof(ExchFlags))) != cudaSuccess ||
+        (e = cudaMemset(c->d_counters.get(), 0, kCounters * sizeof(unsigned long long))) != cudaSuccess) {
         int rc = cuda_fail(nullptr, e, "rt_create");
         rt_destroy(c);
         return rc;
@@ -544,15 +512,8 @@ int rt_create(int cuda_device, rt_ctx** out) {
 int rt_destroy(rt_ctx* c) {
     if (!c) return RT_ERR_INVALID;
     cudaSetDevice(c->device);
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    cudaFree(c->d_sph); cudaFree(c->d_sph_id); cudaFree(c->d_box); cudaFree(c->d_box_id); cudaFree(c->d_mat);
-    cudaFree(c->d_accum); cudaFree(c->d_argb); cudaFree(c->d_counters); cudaFree(c->d_scratch);
-    cudaFree(c->d_bvh_nodes); cudaFree(c->d_bvh_refs); cudaFree(c->d_bvh_slots); cudaFree(c->d_bvh_qnodes); cudaFree(c->d_wide_nodes); cudaFree(c->d_wide_refs); cudaFree(c->d_tune);
-    cudaFree(c->d_tri); cudaFree(c->d_tri_obj); cudaFree(c->d_prim_nt); cudaFree(c->d_prim_id); cudaFree(c->d_flags);
-    cudaFree(c->d_denoise[0]); cudaFree(c->d_denoise[1]);
-    release_temporal(c);
+    if (c->stream) cudaStreamSynchronize(c->stream);           // no kernel may still use the device arrays that `delete c` frees
     wavefront_destroy(c->wf);
-    cudaFree(c->d_flat_boxes); cudaFree(c->d_flat_cull); cudaFree(c->d_flat_slots); cudaFree(c->d_flat_ids);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->ev2) cudaEventDestroy(c->ev2);
@@ -741,12 +702,12 @@ int rt_set_params(rt_ctx* c, const rt_params* p) {
     if (resized) {
         RT_CUDA(c, cudaSetDevice(c->device));
         RT_CUDA(c, cudaStreamSynchronize(c->stream));
-        if (c->d_accum) { cudaFree(c->d_accum); c->d_accum = nullptr; }
-        if (c->d_argb) { cudaFree(c->d_argb); c->d_argb = nullptr; }
-        c->cap_pixels = 0;
-        for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }   // 32 B per pixel, sized for the old resolution
-        c->cap_denoise = 0;
-        release_temporal(c);                                   // sized for the old resolution
+        // the frame buffers, the denoiser pair (32 B per pixel) and the temporal set (88 B per pixel, the history is gone with it) are
+        // sized for the old resolution
+        c->d_accum.reset(); c->d_argb.reset();
+        for (int k = 0; k < 2; ++k) { c->d_denoise[k].reset(); c->d_tp_h[k].reset(); c->d_tp_nt[k].reset(); c->d_tp_id[k].reset(); }
+        c->d_tp_prior.reset();
+        c->tp_valid = false;
         ++c->accum_epoch;
         c->prim_valid = false;
         c->exch.ready = false;
@@ -832,13 +793,13 @@ int rt_shard_range(int spp, int rank, int world, uint32_t next_sample, uint32_t*
 int rt_reset_accumulation(rt_ctx* c) {
     int rc = prepare(c);
     if (rc != RT_OK) return rc;
-    RT_CUDA(c, cudaMemsetAsync(c->d_accum, 0, (size_t)c->par.width * c->par.height * sizeof(float4), c->stream));
+    RT_CUDA(c, cudaMemsetAsync(c->d_accum.get(), 0, (size_t)c->par.width * c->par.height * sizeof(float4), c->stream));
     // counters: [0] segments since the last reset, [1] since rt_create (never cleared); [2], [3] the same for the
     // closest-hit queries actually executed (primary-hit reuse); [4..7] scratch for the autotuner; [8..12] BVH traversal
     // statistics since the last reset (RT_OPT_TRAVERSAL_STATS: queries, node visits, sphere / cube / triangle tests)
-    RT_CUDA(c, cudaMemsetAsync(c->d_counters, 0, sizeof(unsigned long long), c->stream));
-    RT_CUDA(c, cudaMemsetAsync(c->d_counters + 2, 0, sizeof(unsigned long long), c->stream));
-    RT_CUDA(c, cudaMemsetAsync(c->d_counters + 8, 0, 8 * sizeof(unsigned long long), c->stream));
+    RT_CUDA(c, cudaMemsetAsync(c->d_counters.get(), 0, sizeof(unsigned long long), c->stream));
+    RT_CUDA(c, cudaMemsetAsync(c->d_counters.get() + 2, 0, sizeof(unsigned long long), c->stream));
+    RT_CUDA(c, cudaMemsetAsync(c->d_counters.get() + 8, 0, 8 * sizeof(unsigned long long), c->stream));
     c->samples = 0; c->next_sample = 0; c->paths = 0;
     ++c->accum_epoch;
     return RT_OK;
@@ -861,7 +822,7 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
         // SCREEN_SCALE / progressive resolution: one path per block, block-filled (Raytracer.cpp:233-248)
         int mine = 1; uint32_t first = 0;
         if (c->par.mode == RT_MODE_PATH) rt_shard_range(spp, c->rank, c->world, c->next_sample, &first, &mine);
-        RT_CUDA(c, launch_render_blocks(c->view, ac, c->frame, c->d_accum, first, mine, c->pixel_step, c->strip_columns, c->d_counters, c->stream));
+        RT_CUDA(c, launch_render_blocks(c->view, ac, c->frame, c->d_accum.get(), first, mine, c->pixel_step, c->strip_columns, c->d_counters.get(), c->stream));
         const int sw = c->strip_columns > 0 && c->strip_columns < c->par.width ? c->strip_columns : c->par.width;
         uint64_t blocks = 0;
         for (int x0 = 0; x0 < c->par.width; x0 += sw) {
@@ -875,7 +836,7 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
         c->used_pipeline = RT_PIPELINE_REGEN;
     } else if (c->par.mode == RT_MODE_PREVIEW) {
         // SIMPLEDRAW: ACCUMULATIONFRAMES stays 1, every frame overwrites (Raytracer.cpp:66-67,589)
-        RT_CUDA(c, launch_render_preview(c->view, ac, c->frame, c->d_accum, c->d_counters, c->stream));
+        RT_CUDA(c, launch_render_preview(c->view, ac, c->frame, c->d_accum.get(), c->d_counters.get(), c->stream));
         c->samples = 1; c->next_sample = 0; c->paths += px; c->total_paths += px;
     } else {
         // this rank's slice of the global sample indices [next, next+spp)
@@ -892,7 +853,7 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
         const PrimCache* prim = prim_cache_arg(c, pc);
         if (wavefront) {
             if (!c->wf) c->wf = wavefront_create();
-            const cudaError_t we = launch_render_wavefront(c->wf, c->view, ac, c->frame, c->d_accum, first, mine, prim, c->d_counters, c->stream, c->opt_bvh_sched == 0,
+            const cudaError_t we = launch_render_wavefront(c->wf, c->view, ac, c->frame, c->d_accum.get(), first, mine, prim, c->d_counters.get(), c->stream, c->opt_bvh_sched == 0,
                                                            c->opt_wf_refill, c->opt_wf_node_min, c->opt_wf_wave_mpaths, c->opt_trav_stats != 0, streaming);
             if (we == cudaErrorMemoryAllocation) {
                 // not even one sample per pixel of path state fits next to what else lives on the device: the megakernel
@@ -906,10 +867,10 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
         }
         if (wavefront) {}
         else if (scheduled)
-            RT_CUDA(c, launch_render_bvh(c->view, ac, c->frame, c->d_accum, first, mine, c->d_counters, c->opt_bvh_wait_k, c->stream));
+            RT_CUDA(c, launch_render_bvh(c->view, ac, c->frame, c->d_accum.get(), first, mine, c->d_counters.get(), c->opt_bvh_wait_k, c->stream));
         else {
             if (frame) frame->samples_after = c->samples + (uint32_t)mine;
-            RT_CUDA(c, launch_render_regen(c->view, ac, c->frame, c->d_accum, first, mine, prim, c->d_counters, c->stream, c->opt_pool_tiles,
+            RT_CUDA(c, launch_render_regen(c->view, ac, c->frame, c->d_accum.get(), first, mine, prim, c->d_counters.get(), c->stream, c->opt_pool_tiles,
                                            c->opt_flat_coop == 2 ? (c->opt_accel == RT_ACCEL_AUTO ? c->tuned_flat_coop != 0 : c->view.n_box == 0) : c->opt_flat_coop != 0,
                                            c->opt_trav_stats != 0, c->world == 1 && mine > 0 ? frame : nullptr));
         }
@@ -925,7 +886,9 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
 
 int rt_render_spp(rt_ctx* c, int spp) { return render_samples(c, spp, nullptr); }
 
-// device pointer of a page-locked host surface with a tight pitch (what the kernels can store to directly), else nullptr
+// Device pointer of a page-locked host surface with a tight pitch, else nullptr. The kernels store to such a surface (rt_host_alloc)
+// themselves, over PCIe (zero-copy): an interactive frame then has no separate device-to-host copy to set up and wait for.
+// RTB200_ZEROCOPY=0 turns it off.
 static uint32_t* mapped_surface(uint32_t* host_out, int pitch_bytes, int w) {
     static const bool zero_copy = [] { const char* v = getenv("RTB200_ZEROCOPY"); return !(v && v[0] == '0'); }();
     if (!zero_copy || pitch_bytes != w * 4) return nullptr;
@@ -935,30 +898,146 @@ static uint32_t* mapped_surface(uint32_t* host_out, int pitch_bytes, int w) {
     return nullptr;
 }
 
+// the filter parameters of rt_denoise_rgba8 / rt_read_denoised / the temporal calls and log2 of the normal power
+static int check_denoise_params(rt_ctx* c, const char* fn, const rt_denoise_params& p, int& pow_log2) {
+    pow_log2 = 0;
+    while (pow_log2 < 9 && (1 << pow_log2) != p.normal_power) ++pow_log2;
+    if (p.passes < 0 || p.passes > kDenoiseMaxPasses) return fail(c, RT_ERR_INVALID, std::string(fn) + ": passes must be 0 .. 8");
+    if (pow_log2 > 8) return fail(c, RT_ERR_INVALID, std::string(fn) + ": normal_power must be a power of two in 1 .. 256");
+    if (!(p.sigma_color > 0.f && p.sigma_color <= FLT_MAX) || !(p.sigma_depth > 0.f && p.sigma_depth <= FLT_MAX))
+        return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and positive");
+    return RT_OK;
+}
+
+static int check_temporal_params(rt_ctx* c, const char* fn, const rt_temporal_params& tp) {
+    if (tp.max_history < 1 || tp.max_history > 4096) return fail(c, RT_ERR_INVALID, std::string(fn) + ": max_history must be 1 .. 4096");
+    if (!(tp.tau_depth > 0.f && tp.tau_depth <= FLT_MAX)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_depth must be finite and positive");
+    if (!(tp.tau_normal >= -1.f && tp.tau_normal <= 1.f)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_normal must be in -1 .. 1");
+    return RT_OK;
+}
+
+// Where a presented image goes: an ARGB8 host surface, or (argb NULL) the float (r, g, b, .) image of the filter or the temporal blend.
+struct PresentOut {
+    uint32_t* argb; int pitch_bytes; int flip_y;
+    float* rgba;
+};
+
+// Every call that presents an image. spp != NULL (rt_render_frame): *spp samples are rendered first, and for 1-2 samples the render
+// kernel may resolve the frame itself. Then the image: the plain resolve; with dn the filter of rt_denoise.cu, guided by the
+// primary-hit cache; with tp the prior from the temporal history (rt_temporal.cuh) and the blend, filtered when dn has passes, and the
+// new history. Apart from the render, read-only on the accumulation buffer, the sample counter and the path statistics.
+static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_temporal_params* tp, const rt_denoise_params* dn,
+                   const int* spp = nullptr) {
+    int rc = prepare(c);
+    if (rc != RT_OK) return rc;
+    const int w = c->par.width, h = c->par.height;
+    const size_t px = (size_t)w * h;
+    if (out.argb ? out.pitch_bytes < w * 4 : !out.rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
+    if (tp && c->world > 1) return fail(c, RT_ERR_INVALID, std::string(fn) + ": not supported on a shard (its buffer holds only part of the samples)");
+    if (tp && (rc = check_temporal_params(c, fn, *tp)) != RT_OK) return rc;
+    int pow_log2 = 0;
+    if (dn && (rc = check_denoise_params(c, fn, *dn, pow_log2)) != RT_OK) return rc;
+    // preview shading is deterministic: nothing to filter, and no history
+    const bool preview = c->par.mode == RT_MODE_PREVIEW;
+    const int passes = dn && !preview ? dn->passes : 0;
+    // rt_read_denoised reads the filter's output also without passes: the plain mean
+    const bool filter = passes > 0 || (dn && out.rgba && !tp);
+    const int flip_y = out.flip_y ? 1 : 0;
+    uint32_t* mapped = out.argb ? mapped_surface(out.argb, out.pitch_bytes, w) : nullptr;
+    bool fused = false;
+    if (spp) {
+        static const bool fuse_on = [] { const char* v = getenv("RTB200_FRAME_FUSE"); return !(v && v[0] == '0'); }();
+        FrameTarget ft;
+        ft.surface = c->d_argb.get(); ft.mapped_host = mapped; ft.flip_y = flip_y;
+        const bool candidate = fuse_on && c->par.mode == RT_MODE_PATH && c->pixel_step <= 1 && c->world == 1;
+        if ((rc = render_samples(c, *spp, candidate ? &ft : nullptr)) != RT_OK) return rc;
+        fused = ft.fused;
+    }
+    if (passes > 0 || (tp && !preview)) {
+        AccelSel ac;
+        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
+        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
+    }
+    if (tp && c->d_tp_prior.capacity() < px) {
+        RT_CUDA(c, cudaStreamSynchronize(c->stream));
+        c->tp_valid = false;                                   // the history is gone with its arrays
+        const cudaError_t e = reserve_all(px, c->d_tp_h[0], c->d_tp_nt[0], c->d_tp_id[0], c->d_tp_h[1], c->d_tp_nt[1], c->d_tp_id[1], c->d_tp_prior);
+        if (e != cudaSuccess) return cuda_fail(c, e, "temporal history buffers");
+    }
+    if (filter && c->d_denoise[0].capacity() < px) {
+        RT_CUDA(c, cudaStreamSynchronize(c->stream));
+        const cudaError_t e = reserve_all(px, c->d_denoise[0], c->d_denoise[1]);
+        if (e != cudaSuccess) return cuda_fail(c, e, "denoiser buffers");
+    }
+
+    TemporalLaunch t;
+    const int cur = c->tp_cur ^ 1;                             // the half the new history goes to
+    if (tp) {
+        t.accum = c->d_accum.get(); t.count = (float)c->samples;
+        t.nt = preview ? nullptr : c->d_prim_nt.get(); t.id = preview ? nullptr : c->d_prim_id.get();
+        t.width = w; t.height = h;
+        t.cap = (float)tp->max_history; t.tau_z = tp->tau_depth; t.tau_n = tp->tau_normal;
+        t.cur.o = c->frame.cam_pos; t.cur.u = c->frame.u_axis; t.cur.v = c->frame.v_axis; t.cur.f = c->frame.fwd;
+        t.prev = c->tp_pose;
+        tp_inverse(t.prev, t.m);
+        // the prior: none without a history of the same radiance; rebuilt when the accumulation restarted or the pose moved
+        const bool same_pose = memcmp(&t.cur, &t.prev, sizeof t.cur) == 0;
+        if (preview || !c->tp_valid || c->tp_key != c->radiance_key) t.mode = kTpZero;
+        else if (c->tp_epoch != c->accum_epoch || !same_pose) t.mode = same_pose ? kTpCopy : kTpReproject;
+        else t.mode = kTpKeep;
+        const int old = c->tp_cur;
+        t.hist.h = c->d_tp_h[old].get(); t.hist.nt = c->d_tp_nt[old].get(); t.hist.id = c->d_tp_id[old].get();
+        t.prior = c->d_tp_prior.get();
+        t.h_out = c->d_tp_h[cur].get(); t.nt_out = c->d_tp_nt[cur].get(); t.id_out = c->d_tp_id[cur].get();
+        t.next = passes > 0 ? c->d_denoise[1].get() : nullptr;
+        t.argb = out.argb && passes == 0 ? c->d_argb.get() : nullptr; t.argb_host = t.argb ? mapped : nullptr; t.flip_y = flip_y;
+        c->tp_valid = false;                                   // until the new history is complete
+    }
+    cudaError_t e = cudaSuccess;
+    if (!fused) {
+        cudaEventRecord(c->ev2, c->stream);
+        if (tp) e = launch_temporal(t, c->stream);
+        else if (!filter) e = launch_resolve(c->d_accum.get(), c->samples, w, h, 0, w * h, flip_y, c->d_argb.get(), 0, c->stream, mapped);
+        if (e == cudaSuccess && filter) {
+            DenoiseLaunch d;
+            d.accum = tp ? nullptr : c->d_accum.get(); d.samples = tp ? 0 : c->samples;
+            d.nt = c->d_prim_nt.get(); d.id = c->d_prim_id.get();
+            d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
+            d.sigma_color = dn->sigma_color; d.sigma_depth = dn->sigma_depth;
+            d.buf[0] = c->d_denoise[0].get(); d.buf[1] = c->d_denoise[1].get();
+            d.argb = out.argb ? c->d_argb.get() : nullptr; d.argb_host = mapped; d.flip_y = flip_y;
+            d.neff = tp ? t.h_out : nullptr;                   // the temporal form: the blend is the input, with its per-pixel count
+            e = launch_denoise(d, c->stream);
+        }
+        cudaEventRecord(c->ev3, c->stream);
+    }
+    if (e == cudaSuccess && out.rgba) {
+        const float4* img = tp && passes == 0 ? t.h_out : c->d_denoise[passes > 0 ? (passes - 1) & 1 : 0].get();
+        e = cudaMemcpyAsync(out.rgba, img, px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
+    } else if (e == cudaSuccess && !mapped) {
+        if (out.pitch_bytes == w * 4)                          // tightly packed surface: one linear copy
+            e = cudaMemcpyAsync(out.argb, c->d_argb.get(), px * 4, cudaMemcpyDeviceToHost, c->stream);
+        else
+            e = cudaMemcpy2DAsync(out.argb, (size_t)out.pitch_bytes, c->d_argb.get(), (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) return cuda_fail(c, e, fn);
+    if (fused) c->last_resolve_ms = 0.f;                       // no separate resolve ran
+    else cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
+    if (tp) {
+        c->tp_cur = cur;
+        c->tp_valid = !preview;
+        c->tp_pose = t.cur; c->tp_epoch = c->accum_epoch; c->tp_key = c->radiance_key;
+    }
+    return RT_OK;
+}
+
 // One progressive frame: rt_render_spp(spp) + rt_resolve_rgba8(host_out) with the same result, as ONE call - which is what the
 // reference's frame is (renderArea resolves every pixel as it is traced, Raytracer.cpp:63-76,223-257). For 1-2 samples per pixel the
 // render kernel resolves the pixels it finishes and streams them to a page-locked surface while it is still tracing (FrameOut,
 // rt_kernels.cu); every other case runs the two steps one after the other.
 int rt_render_frame(rt_ctx* c, int spp, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    int rc = prepare(c);
-    if (rc != RT_OK) return rc;
-    const int w = c->par.width, h = c->par.height;
-    if (!host_out || pitch_bytes < w * 4) return fail(c, RT_ERR_INVALID, "rt_render_frame: bad output buffer");
-    static const bool fuse_on = [] { const char* v = getenv("RTB200_FRAME_FUSE"); return !(v && v[0] == '0'); }();
-    FrameTarget ft;
-    ft.surface = c->d_argb; ft.mapped_host = mapped_surface(host_out, pitch_bytes, w); ft.flip_y = flip_y ? 1 : 0;
-    const bool candidate = fuse_on && c->par.mode == RT_MODE_PATH && c->pixel_step <= 1 && c->world == 1;
-    if ((rc = render_samples(c, spp, candidate ? &ft : nullptr)) != RT_OK) return rc;
-    if (!ft.fused) return rt_resolve_rgba8(c, host_out, pitch_bytes, flip_y);
-    cudaError_t e = cudaSuccess;
-    if (!ft.mapped_host) {
-        if (pitch_bytes == w * 4) e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-        else e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e != cudaSuccess) return cuda_fail(c, e, "rt_render_frame");
-    c->last_resolve_ms = 0.f;                                 // no separate resolve ran
-    return RT_OK;
+    return present(c, "rt_render_frame", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr, &spp);
 }
 
 int rt_resolve_device(rt_ctx* c, const void* dev_accum, uint32_t samples, int first_pixel, int n_pixels, void* dev_out, int flip_y) {
@@ -973,26 +1052,7 @@ int rt_resolve_device(rt_ctx* c, const void* dev_accum, uint32_t samples, int fi
 }
 
 int rt_resolve_rgba8(rt_ctx* c, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    int rc = prepare(c);
-    if (rc != RT_OK) return rc;
-    const int w = c->par.width, h = c->par.height;
-    if (!host_out || pitch_bytes < w * 4) return fail(c, RT_ERR_INVALID, "rt_resolve_rgba8: bad output buffer");
-    // A page-locked host surface (rt_host_alloc) with a tight pitch is written by the resolve kernel itself, over PCIe (zero-copy):
-    // an interactive frame then has no separate device-to-host copy to set up and wait for. RTB200_ZEROCOPY=0 turns it off.
-    uint32_t* mapped = mapped_surface(host_out, pitch_bytes, w);
-    cudaEventRecord(c->ev2, c->stream);
-    cudaError_t e = launch_resolve(c->d_accum, c->samples, w, h, 0, w * h, flip_y, c->d_argb, 0, c->stream, mapped);
-    cudaEventRecord(c->ev3, c->stream);
-    if (e == cudaSuccess && !mapped) {
-        if (pitch_bytes == w * 4)                              // tightly packed surface: one linear copy
-            e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-        else
-            e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
-    if (e != cudaSuccess) return cuda_fail(c, e, "rt_resolve_rgba8");
-    return RT_OK;
+    return present(c, "rt_resolve_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr);
 }
 
 void rt_default_denoise_params(rt_denoise_params* p) {
@@ -1000,90 +1060,16 @@ void rt_default_denoise_params(rt_denoise_params* p) {
     p->passes = 5; p->normal_power = 128; p->sigma_color = 2.0f; p->sigma_depth = 1.0f;   // DESIGN.md 8: sigma_color tuned at 4 spp
 }
 
-// the filter parameters of rt_denoise_rgba8 / rt_read_denoised / the temporal calls (NULL: the defaults) and log2 of the normal power
-static int check_denoise_params(rt_ctx* c, const char* fn, const rt_denoise_params* user, rt_denoise_params& p, int& pow_log2) {
-    if (user) p = *user;
-    else rt_default_denoise_params(&p);
-    pow_log2 = 0;
-    while (pow_log2 < 9 && (1 << pow_log2) != p.normal_power) ++pow_log2;
-    if (p.passes < 0 || p.passes > kDenoiseMaxPasses) return fail(c, RT_ERR_INVALID, std::string(fn) + ": passes must be 0 .. 8");
-    if (pow_log2 > 8) return fail(c, RT_ERR_INVALID, std::string(fn) + ": normal_power must be a power of two in 1 .. 256");
-    if (!(p.sigma_color > 0.f && p.sigma_color <= FLT_MAX) || !(p.sigma_depth > 0.f && p.sigma_depth <= FLT_MAX))
-        return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and positive");
-    return RT_OK;
-}
-
-// the filter's ping-pong images, 32 B per pixel
-static int ensure_denoise_buffers(rt_ctx* c, size_t px) {
-    if (c->cap_denoise < px || !c->d_denoise[0]) {
-        RT_CUDA(c, cudaStreamSynchronize(c->stream));
-        for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }
-        c->cap_denoise = 0;
-        cudaError_t e = cudaMalloc((void**)&c->d_denoise[0], px * sizeof(float4));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_denoise[1], px * sizeof(float4));
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            for (float4*& b : c->d_denoise) { cudaFree(b); b = nullptr; }
-            return cuda_fail(c, e, "denoiser buffers");
-        }
-        c->cap_denoise = px;
-    }
-    return RT_OK;
-}
-
-// rt_denoise_rgba8 (host_out != NULL) and rt_read_denoised (host_rgba != NULL): the filter of rt_denoise.cu over the accumulation
-// buffer, guided by the primary-hit cache; read-only on the buffer, the sample counter and the path statistics.
-static int denoise(rt_ctx* c, const rt_denoise_params* user, uint32_t* host_out, int pitch_bytes, int flip_y, float* host_rgba) {
-    int rc = prepare(c);
-    if (rc != RT_OK) return rc;
-    const int w = c->par.width, h = c->par.height;
-    const char* fn = host_out ? "rt_denoise_rgba8" : "rt_read_denoised";
-    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
-    rt_denoise_params p;
-    int pow_log2;
-    if ((rc = check_denoise_params(c, fn, user, p, pow_log2)) != RT_OK) return rc;
-    // preview shading is deterministic: nothing to filter
-    const int passes = c->par.mode == RT_MODE_PREVIEW ? 0 : p.passes;
-    if (host_out && passes == 0) return rt_resolve_rgba8(c, host_out, pitch_bytes, flip_y);
-    const size_t px = (size_t)w * h;
-    if (passes > 0) {
-        AccelSel ac;
-        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
-        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
-    }
-    if ((rc = ensure_denoise_buffers(c, px)) != RT_OK) return rc;
-    uint32_t* mapped = host_out ? mapped_surface(host_out, pitch_bytes, w) : nullptr;
-    DenoiseLaunch d;
-    d.accum = c->d_accum; d.samples = c->samples;
-    d.nt = c->d_prim_nt; d.id = c->d_prim_id;
-    d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
-    d.sigma_color = p.sigma_color; d.sigma_depth = p.sigma_depth;
-    d.buf[0] = c->d_denoise[0]; d.buf[1] = c->d_denoise[1];
-    d.argb = host_out ? c->d_argb : nullptr; d.argb_host = mapped; d.flip_y = flip_y ? 1 : 0;
-    d.neff = nullptr;
-    cudaEventRecord(c->ev2, c->stream);
-    cudaError_t e = launch_denoise(d, c->stream);
-    cudaEventRecord(c->ev3, c->stream);
-    if (e == cudaSuccess && host_rgba)
-        e = cudaMemcpyAsync(host_rgba, c->d_denoise[passes > 0 ? (passes - 1) & 1 : 0], px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
-    else if (e == cudaSuccess && !mapped) {
-        if (pitch_bytes == w * 4) e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-        else e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
-    if (e != cudaSuccess) return cuda_fail(c, e, fn);
-    return RT_OK;
-}
-
 int rt_denoise_rgba8(rt_ctx* c, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    if (!host_out) return fail(c, RT_ERR_INVALID, "rt_denoise_rgba8: bad output buffer");
-    return denoise(c, p, host_out, pitch_bytes, flip_y, nullptr);
+    rt_denoise_params d;
+    if (!p) rt_default_denoise_params(&d);
+    return present(c, "rt_denoise_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, p ? p : &d);
 }
 
 int rt_read_denoised(rt_ctx* c, const rt_denoise_params* p, float* host_rgba) {
-    if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_read_denoised: NULL output");
-    return denoise(c, p, nullptr, 0, 0, host_rgba);
+    rt_denoise_params d;
+    if (!p) rt_default_denoise_params(&d);
+    return present(c, "rt_read_denoised", {nullptr, 0, 0, host_rgba}, nullptr, p ? p : &d);
 }
 
 void rt_default_temporal_params(rt_temporal_params* p) {
@@ -1091,117 +1077,17 @@ void rt_default_temporal_params(rt_temporal_params* p) {
     p->max_history = 32; p->tau_depth = 0.02f; p->tau_normal = 0.9f; p->reserved = 0;   // DESIGN.md 8: chosen from a measured sweep
 }
 
-// rt_temporal_rgba8 (host_out != NULL) and rt_read_temporal (host_rgba != NULL): the prior from the history (rt_temporal.cuh), the
-// blend, optionally the filter in its per-pixel count form, then the new history; read-only on the accumulation buffer, the sample
-// counter and the path statistics.
-static int temporal(rt_ctx* c, const rt_temporal_params* user, const rt_denoise_params* dn_user, uint32_t* host_out, int pitch_bytes,
-                    int flip_y, float* host_rgba) {
-    int rc = prepare(c);
-    if (rc != RT_OK) return rc;
-    const int w = c->par.width, h = c->par.height;
-    const char* fn = host_out ? "rt_temporal_rgba8" : "rt_read_temporal";
-    if (host_out ? pitch_bytes < w * 4 : !host_rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
-    if (c->world > 1) return fail(c, RT_ERR_INVALID, std::string(fn) + ": not supported on a shard (its buffer holds only part of the samples)");
-    rt_temporal_params tp;
-    if (user) tp = *user;
-    else rt_default_temporal_params(&tp);
-    if (tp.max_history < 1 || tp.max_history > 4096) return fail(c, RT_ERR_INVALID, std::string(fn) + ": max_history must be 1 .. 4096");
-    if (!(tp.tau_depth > 0.f && tp.tau_depth <= FLT_MAX)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_depth must be finite and positive");
-    if (!(tp.tau_normal >= -1.f && tp.tau_normal <= 1.f)) return fail(c, RT_ERR_INVALID, std::string(fn) + ": tau_normal must be in -1 .. 1");
-    rt_denoise_params dp;
-    int pow_log2 = 0;
-    if (dn_user) {
-        if ((rc = check_denoise_params(c, fn, dn_user, dp, pow_log2)) != RT_OK) return rc;
-    } else {
-        rt_default_denoise_params(&dp);
-        dp.passes = 0;
-    }
-    // preview shading is deterministic: the plain resolve, and no history
-    const bool preview = c->par.mode == RT_MODE_PREVIEW;
-    const int passes = preview ? 0 : dp.passes;
-    const size_t px = (size_t)w * h;
-    if (!preview) {
-        AccelSel ac;
-        if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
-        if ((rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
-    }
-    if (c->cap_temporal < px || !c->d_tp_prior) {
-        RT_CUDA(c, cudaStreamSynchronize(c->stream));
-        release_temporal(c);
-        cudaError_t e = cudaSuccess;
-        for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
-            e = cudaMalloc((void**)&c->d_tp_h[k], px * sizeof(float4));
-            if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_nt[k], px * sizeof(float4));
-            if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_id[k], px * sizeof(int));
-        }
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_tp_prior, px * sizeof(float4));
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            release_temporal(c);
-            return cuda_fail(c, e, "temporal history buffers");
-        }
-        c->cap_temporal = px;
-    }
-    if (passes > 0 && (rc = ensure_denoise_buffers(c, px)) != RT_OK) return rc;
-
-    TemporalLaunch t;
-    t.accum = c->d_accum; t.count = (float)c->samples;
-    t.nt = preview ? nullptr : c->d_prim_nt; t.id = preview ? nullptr : c->d_prim_id;
-    t.width = w; t.height = h;
-    t.cap = (float)tp.max_history; t.tau_z = tp.tau_depth; t.tau_n = tp.tau_normal;
-    t.cur.o = c->frame.cam_pos; t.cur.u = c->frame.u_axis; t.cur.v = c->frame.v_axis; t.cur.f = c->frame.fwd;
-    t.prev = c->tp_pose;
-    tp_inverse(t.prev, t.m);
-    // the prior: none without a history of the same radiance; rebuilt when the accumulation restarted or the pose moved
-    const bool same_pose = memcmp(&t.cur, &t.prev, sizeof t.cur) == 0;
-    if (preview || !c->tp_valid || c->tp_key != c->radiance_key) t.mode = kTpZero;
-    else if (c->tp_epoch != c->accum_epoch || !same_pose) t.mode = same_pose ? kTpCopy : kTpReproject;
-    else t.mode = kTpKeep;
-    const int old = c->tp_cur, cur = old ^ 1;
-    t.hist.h = c->d_tp_h[old]; t.hist.nt = c->d_tp_nt[old]; t.hist.id = c->d_tp_id[old];
-    t.prior = c->d_tp_prior;
-    t.h_out = c->d_tp_h[cur]; t.nt_out = c->d_tp_nt[cur]; t.id_out = c->d_tp_id[cur];
-    uint32_t* mapped = host_out ? mapped_surface(host_out, pitch_bytes, w) : nullptr;
-    t.next = passes > 0 ? c->d_denoise[1] : nullptr;
-    t.argb = host_out && passes == 0 ? c->d_argb : nullptr; t.argb_host = t.argb ? mapped : nullptr; t.flip_y = flip_y ? 1 : 0;
-    c->tp_valid = false;                                      // until the new history is complete
-    cudaEventRecord(c->ev2, c->stream);
-    cudaError_t e = launch_temporal(t, c->stream);
-    if (e == cudaSuccess && passes > 0) {
-        DenoiseLaunch d;
-        d.accum = nullptr; d.samples = 0;
-        d.nt = c->d_prim_nt; d.id = c->d_prim_id;
-        d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
-        d.sigma_color = dp.sigma_color; d.sigma_depth = dp.sigma_depth;
-        d.buf[0] = c->d_denoise[0]; d.buf[1] = c->d_denoise[1];
-        d.argb = host_out ? c->d_argb : nullptr; d.argb_host = mapped; d.flip_y = flip_y ? 1 : 0;
-        d.neff = t.h_out;
-        e = launch_denoise(d, c->stream);
-    }
-    cudaEventRecord(c->ev3, c->stream);
-    if (e == cudaSuccess && host_rgba)
-        e = cudaMemcpyAsync(host_rgba, passes > 0 ? c->d_denoise[(passes - 1) & 1] : t.h_out, px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
-    else if (e == cudaSuccess && !mapped) {
-        if (pitch_bytes == w * 4) e = cudaMemcpyAsync(host_out, c->d_argb, (size_t)w * 4 * (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-        else e = cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess) cudaEventElapsedTime(&c->last_resolve_ms, c->ev2, c->ev3);
-    if (e != cudaSuccess) return cuda_fail(c, e, fn);
-    c->tp_cur = cur;
-    c->tp_valid = !preview;
-    c->tp_pose = t.cur; c->tp_epoch = c->accum_epoch; c->tp_key = c->radiance_key;
-    return RT_OK;
-}
-
+// dn NULL: no filter
 int rt_temporal_rgba8(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    if (!host_out) return fail(c, RT_ERR_INVALID, "rt_temporal_rgba8: bad output buffer");
-    return temporal(c, p, dn, host_out, pitch_bytes, flip_y, nullptr);
+    rt_temporal_params d;
+    if (!p) rt_default_temporal_params(&d);
+    return present(c, "rt_temporal_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, p ? p : &d, dn);
 }
 
 int rt_read_temporal(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, float* host_rgba) {
-    if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_read_temporal: NULL output");
-    return temporal(c, p, dn, nullptr, 0, 0, host_rgba);
+    rt_temporal_params d;
+    if (!p) rt_default_temporal_params(&d);
+    return present(c, "rt_read_temporal", {nullptr, 0, 0, host_rgba}, p ? p : &d, dn);
 }
 
 int rt_reset_temporal(rt_ctx* c) {
@@ -1222,7 +1108,7 @@ int rt_read_accum(rt_ctx* c, float* host_rgba, uint32_t* samples) {
     int rc = prepare(c);
     if (rc != RT_OK) return rc;
     if (host_rgba)
-        RT_CUDA(c, cudaMemcpyAsync(host_rgba, c->d_accum, (size_t)c->par.width * c->par.height * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+        RT_CUDA(c, cudaMemcpyAsync(host_rgba, c->d_accum.get(), (size_t)c->par.width * c->par.height * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     if (samples) *samples = c->samples;
     return RT_OK;
@@ -1232,7 +1118,7 @@ int rt_write_accum(rt_ctx* c, const float* host_rgba, uint32_t samples) {
     int rc = prepare(c);
     if (rc != RT_OK) return rc;
     if (!host_rgba) return fail(c, RT_ERR_INVALID, "rt_write_accum: NULL input");
-    RT_CUDA(c, cudaMemcpyAsync(c->d_accum, host_rgba, (size_t)c->par.width * c->par.height * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+    RT_CUDA(c, cudaMemcpyAsync(c->d_accum.get(), host_rgba, (size_t)c->par.width * c->par.height * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     c->samples = samples; c->next_sample = samples;
     ++c->accum_epoch;
@@ -1245,19 +1131,18 @@ int rt_read_aov(rt_ctx* c, int32_t* id, float* t, float* normal, float* point) {
     const size_t px = (size_t)c->par.width * c->par.height;
     AccelSel ac;
     if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
-    int* d_id = nullptr; float *d_t = nullptr, *d_n = nullptr, *d_p = nullptr;
+    DeviceArray<int> d_id; DeviceArray<float> d_t, d_n, d_p;
     cudaError_t e = cudaSuccess;
-    if (id) e = cudaMalloc((void**)&d_id, px * 4);
-    if (e == cudaSuccess && t) e = cudaMalloc((void**)&d_t, px * 4);
-    if (e == cudaSuccess && normal) e = cudaMalloc((void**)&d_n, px * 12);
-    if (e == cudaSuccess && point) e = cudaMalloc((void**)&d_p, px * 12);
-    if (e == cudaSuccess) e = launch_primary_aov(c->view, ac, c->frame, d_id, d_t, d_n, d_p, c->stream);
-    if (e == cudaSuccess && id) e = cudaMemcpyAsync(id, d_id, px * 4, cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess && t) e = cudaMemcpyAsync(t, d_t, px * 4, cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess && normal) e = cudaMemcpyAsync(normal, d_n, px * 12, cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess && point) e = cudaMemcpyAsync(point, d_p, px * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (id) e = d_id.reserve(px);
+    if (e == cudaSuccess && t) e = d_t.reserve(px);
+    if (e == cudaSuccess && normal) e = d_n.reserve(px * 3);
+    if (e == cudaSuccess && point) e = d_p.reserve(px * 3);
+    if (e == cudaSuccess) e = launch_primary_aov(c->view, ac, c->frame, d_id.get(), d_t.get(), d_n.get(), d_p.get(), c->stream);
+    if (e == cudaSuccess && id) e = cudaMemcpyAsync(id, d_id.get(), px * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess && t) e = cudaMemcpyAsync(t, d_t.get(), px * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess && normal) e = cudaMemcpyAsync(normal, d_n.get(), px * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess && point) e = cudaMemcpyAsync(point, d_p.get(), px * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d_id); cudaFree(d_t); cudaFree(d_n); cudaFree(d_p);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_read_aov");
     return RT_OK;
 }
@@ -1267,12 +1152,11 @@ int rt_read_ray_dirs(rt_ctx* c, float* dirs) {
     if (rc != RT_OK) return rc;
     if (!dirs) return fail(c, RT_ERR_INVALID, "rt_read_ray_dirs: NULL output");
     const size_t px = (size_t)c->par.width * c->par.height;
-    float* d = nullptr;
-    cudaError_t e = cudaMalloc((void**)&d, px * 12);
-    if (e == cudaSuccess) e = launch_ray_dirs(c->frame, d, c->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dirs, d, px * 12, cudaMemcpyDeviceToHost, c->stream);
+    DeviceArray<float> d;
+    cudaError_t e = d.reserve(px * 3);
+    if (e == cudaSuccess) e = launch_ray_dirs(c->frame, d.get(), c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dirs, d.get(), px * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_read_ray_dirs");
     return RT_OK;
 }
@@ -1299,19 +1183,19 @@ int rt_trace_rays(rt_ctx* c, const float* origins, const float* dirs, int n, int
     }
     AccelSel ac;
     if ((rc = make_accel(c, kind, ext, ac)) != RT_OK) return rc;
-    float* buf = nullptr;                                      // org3 dir3 n3 p3 t1 id1 = 14 words per ray
-    cudaError_t e = cudaMalloc((void**)&buf, N * 14 * 4);
+    DeviceArray<float> arr;                                    // org3 dir3 n3 p3 t1 id1 = 14 words per ray
+    cudaError_t e = arr.reserve(N * 14);
+    float* buf = arr.get();
     float *d_o = buf, *d_d = buf + 3 * N, *d_n = buf + 6 * N, *d_p = buf + 9 * N, *d_t = buf + 12 * N;
     int* d_id = (int*)(buf + 13 * N);
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_o, origins, N * 12, cudaMemcpyHostToDevice, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_d, dirs, N * 12, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) e = launch_trace_rays(c->view, ac, d_o, d_d, n, d_id, d_t, d_n, d_p, c->stream, c->opt_trav_stats ? c->d_counters : nullptr);
+    if (e == cudaSuccess) e = launch_trace_rays(c->view, ac, d_o, d_d, n, d_id, d_t, d_n, d_p, c->stream, c->opt_trav_stats ? c->d_counters.get() : nullptr);
     if (e == cudaSuccess) e = cudaMemcpyAsync(id, d_id, N * 4, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(t, d_t, N * 4, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(normal, d_n, N * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(point, d_p, N * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(buf);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_trace_rays");
     return RT_OK;
 }
@@ -1324,7 +1208,7 @@ int rt_pick(rt_ctx* c, int x, int y_window, int* id) {
     // through any (x, y) is well defined. One-thread launch through the same device raygen
     // and closest-hit code as the render path.
     const int y = c->par.height - y_window;
-    int* d_id = (int*)c->d_scratch;
+    int* d_id = (int*)c->d_scratch.get();
     AccelSel ac;
     if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
     RT_CUDA(c, launch_pick(c->view, ac, c->frame, x, y, d_id, c->stream));
@@ -1338,14 +1222,14 @@ int rt_env_color(rt_ctx* c, const float* dirs, int n, float* rgb) {
     if (rc != RT_OK) return rc;
     if (n < 0 || (n > 0 && (!dirs || !rgb))) return fail(c, RT_ERR_INVALID, "rt_env_color: bad arguments");
     if (n == 0) return RT_OK;
-    float* buf = nullptr;
     const size_t N = (size_t)n;
-    cudaError_t e = cudaMalloc((void**)&buf, N * 24);
+    DeviceArray<float> arr;                                    // dir3 rgb3 per direction
+    cudaError_t e = arr.reserve(N * 6);
+    float* buf = arr.get();
     if (e == cudaSuccess) e = cudaMemcpyAsync(buf, dirs, N * 12, cudaMemcpyHostToDevice, c->stream);
     if (e == cudaSuccess) e = launch_env_color(c->frame, buf, n, buf + 3 * N, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(rgb, buf + 3 * N, N * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(buf);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_env_color");
     return RT_OK;
 }
@@ -1353,8 +1237,8 @@ int rt_env_color(rt_ctx* c, const float* dirs, int n, float* rgb) {
 int rt_philox_block(rt_ctx* c, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
     if (!c || !ctr || !key || !out) return RT_ERR_INVALID;
     RT_CUDA(c, cudaSetDevice(c->device));
-    RT_CUDA(c, launch_philox(ctr, key, c->d_scratch, c->stream));
-    RT_CUDA(c, cudaMemcpyAsync(out, c->d_scratch, 16, cudaMemcpyDeviceToHost, c->stream));
+    RT_CUDA(c, launch_philox(ctr, key, c->d_scratch.get(), c->stream));
+    RT_CUDA(c, cudaMemcpyAsync(out, c->d_scratch.get(), 16, cudaMemcpyDeviceToHost, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     return RT_OK;
 }
@@ -1362,10 +1246,10 @@ int rt_philox_block(rt_ctx* c, const uint32_t ctr[4], const uint32_t key[2], uin
 int rt_selftest(rt_ctx* c, int which, int* failures) {
     if (!c || !failures || which < 0 || which > 2) return RT_ERR_INVALID;
     RT_CUDA(c, cudaSetDevice(c->device));
-    if (which == 0) RT_CUDA(c, launch_selftest_uniform((int*)c->d_scratch, c->stream));
-    else if (which == 1) RT_CUDA(c, launch_selftest_normalize((int*)c->d_scratch, c->stream));
-    else RT_CUDA(c, launch_selftest_packed((int*)c->d_scratch, c->stream));
-    RT_CUDA(c, cudaMemcpyAsync(failures, c->d_scratch, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    if (which == 0) RT_CUDA(c, launch_selftest_uniform((int*)c->d_scratch.get(), c->stream));
+    else if (which == 1) RT_CUDA(c, launch_selftest_normalize((int*)c->d_scratch.get(), c->stream));
+    else RT_CUDA(c, launch_selftest_packed((int*)c->d_scratch.get(), c->stream));
+    RT_CUDA(c, cudaMemcpyAsync(failures, c->d_scratch.get(), sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     return RT_OK;
 }
@@ -1375,7 +1259,7 @@ int rt_get_stats(rt_ctx* c, rt_stats* out) {
     RT_CUDA(c, cudaSetDevice(c->device));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     unsigned long long counters[kCounters] = {};
-    RT_CUDA(c, cudaMemcpy(counters, c->d_counters, sizeof counters, cudaMemcpyDeviceToHost));
+    RT_CUDA(c, cudaMemcpy(counters, c->d_counters.get(), sizeof counters, cudaMemcpyDeviceToHost));
     if (c->render_timed) { cudaEventElapsedTime(&c->last_render_ms, c->ev0, c->ev1); }
     memset(out, 0, sizeof *out);
     out->paths = c->paths; out->segments = counters[0];
@@ -1392,7 +1276,7 @@ int rt_get_traversal_stats(rt_ctx* c, rt_traversal_stats* out) {
     RT_CUDA(c, cudaSetDevice(c->device));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     unsigned long long counters[kCounters] = {};
-    RT_CUDA(c, cudaMemcpy(counters, c->d_counters, sizeof counters, cudaMemcpyDeviceToHost));
+    RT_CUDA(c, cudaMemcpy(counters, c->d_counters.get(), sizeof counters, cudaMemcpyDeviceToHost));
     memset(out, 0, sizeof *out);
     out->queries = counters[8]; out->node_visits = counters[9];
     out->sphere_tests = counters[10]; out->cube_tests = counters[11]; out->tri_tests = counters[12];
@@ -1403,12 +1287,12 @@ int rt_get_traversal_stats(rt_ctx* c, rt_traversal_stats* out) {
 
 void* rt_accum_device_ptr(rt_ctx* c) {
     if (!c || prepare(c) != RT_OK) return nullptr;
-    return c->d_accum;
+    return c->d_accum.get();
 }
 
 void* rt_argb_device_ptr(rt_ctx* c) {
     if (!c || prepare(c) != RT_OK) return nullptr;
-    return c->d_argb;
+    return c->d_argb.get();
 }
 
 int rt_ipc_export(rt_ctx* c, int which, unsigned char handle[RT_IPC_HANDLE_BYTES]) {
@@ -1417,7 +1301,7 @@ int rt_ipc_export(rt_ctx* c, int which, unsigned char handle[RT_IPC_HANDLE_BYTES
     if (!handle || which < 0 || which > 2) return fail(c, RT_ERR_INVALID, "rt_ipc_export: bad arguments");
     static_assert(sizeof(cudaIpcMemHandle_t) == RT_IPC_HANDLE_BYTES, "IPC handle size");
     cudaIpcMemHandle_t h;
-    RT_CUDA(c, cudaIpcGetMemHandle(&h, which == 0 ? (void*)c->d_accum : which == 1 ? (void*)c->d_argb : (void*)c->d_flags));
+    RT_CUDA(c, cudaIpcGetMemHandle(&h, which == 0 ? (void*)c->d_accum.get() : which == 1 ? (void*)c->d_argb.get() : (void*)c->d_flags.get()));
     memcpy(handle, &h, sizeof h);
     return RT_OK;
 }
@@ -1464,15 +1348,15 @@ int rt_exchange_setup(rt_ctx* c, int rank, int world, void* const* accum_ptrs, v
     // GPU are not guaranteed to run concurrently. This cannot be checked here: for a CUDA-IPC mapping cudaPointerGetAttributes
     // reports the importing context's device, not the exporter's. (Ranks sharing a device: rt_resolve_fused + host-side ordering.)
     for (int r = 0; r < world; ++r) {
-        const void* a = r == rank && !accum_ptrs[r] ? (const void*)c->d_accum : accum_ptrs[r];
-        void* f = r == rank && !flag_ptrs[r] ? (void*)c->d_flags : flag_ptrs[r];
+        const void* a = r == rank && !accum_ptrs[r] ? (const void*)c->d_accum.get() : accum_ptrs[r];
+        void* f = r == rank && !flag_ptrs[r] ? (void*)c->d_flags.get() : flag_ptrs[r];
         if (!a || !f) return fail(c, RT_ERR_INVALID, "rt_exchange_setup: NULL peer pointer");
         if ((rc = enable_peer_access_to(c, a, "rt_exchange_setup: accumulation buffer")) != RT_OK) return rc;
         if ((rc = enable_peer_access_to(c, f, "rt_exchange_setup: exchange flags")) != RT_OK) return rc;
         x.accum[r] = (const float4*)a; x.flags[r] = (ExchFlags*)f;
     }
-    if (x.accum[rank] != c->d_accum || x.flags[rank] != c->d_flags) return fail(c, RT_ERR_INVALID, "rt_exchange_setup: entry `rank` is not this context's own buffer");
-    if (!dst) dst = rank == 0 ? (void*)c->d_argb : nullptr;
+    if (x.accum[rank] != c->d_accum.get() || x.flags[rank] != c->d_flags.get()) return fail(c, RT_ERR_INVALID, "rt_exchange_setup: entry `rank` is not this context's own buffer");
+    if (!dst) dst = rank == 0 ? (void*)c->d_argb.get() : nullptr;
     if (!dst) return fail(c, RT_ERR_INVALID, "rt_exchange_setup: NULL destination surface");
     if ((rc = enable_peer_access_to(c, dst, "rt_exchange_setup: destination surface")) != RT_OK) return rc;
     x.dst = (uint32_t*)dst; x.rank = rank; x.world = world;
@@ -1499,7 +1383,7 @@ int rt_exchange_resolve(rt_ctx* c, uint32_t total_samples, int flip_y) {
 static int check_exchange_error(rt_ctx* c) {
     if (!c->exch.ready) return RT_OK;
     uint32_t err = 0;
-    RT_CUDA(c, cudaMemcpy(&err, &c->d_flags->error, sizeof err, cudaMemcpyDeviceToHost));
+    RT_CUDA(c, cudaMemcpy(&err, &c->d_flags.get()->error, sizeof err, cudaMemcpyDeviceToHost));
     if (err) return fail(c, RT_ERR_CUDA, "exchange timed out: a peer rank did not signal within 4 s");
     return RT_OK;
 }
@@ -1509,7 +1393,7 @@ int rt_read_surface(rt_ctx* c, uint32_t* host_out, int pitch_bytes) {
     if (rc != RT_OK) return rc;
     const int w = c->par.width, h = c->par.height;
     if (!host_out || pitch_bytes < w * 4) return fail(c, RT_ERR_INVALID, "rt_read_surface: bad output buffer");
-    RT_CUDA(c, cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb, (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream));
+    RT_CUDA(c, cudaMemcpy2DAsync(host_out, (size_t)pitch_bytes, c->d_argb.get(), (size_t)w * 4, (size_t)w * 4, (size_t)h, cudaMemcpyDeviceToHost, c->stream));
     RT_CUDA(c, cudaStreamSynchronize(c->stream));
     return check_exchange_error(c);
 }

@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "../../include/rt_b200.h"
+#include "rt_devbuf.h"
 #include "rt_device.cuh"
 #include "rt_kernels.h"
 #include "bvh_build.h"
@@ -45,54 +46,45 @@ struct rt_ctx {
     bool frame_dirty = true;
 
     // device scene
-    float4* d_sph = nullptr; int* d_sph_id = nullptr;
-    float4* d_box = nullptr; int* d_box_id = nullptr;
-    float4* d_mat = nullptr;
-    size_t cap_sph = 0, cap_sph_id = 0, cap_box = 0, cap_box_id = 0, cap_mat = 0;
+    DeviceArray<float4> d_sph; DeviceArray<int> d_sph_id;
+    DeviceArray<float4> d_box; DeviceArray<int> d_box_id;
+    DeviceArray<float4> d_mat;
     // mesh extension: triangle records (mesh.h)
     TriRecords tris;
-    float4* d_tri = nullptr; int* d_tri_obj = nullptr;
-    size_t cap_tri = 0, cap_tri_obj = 0;
+    DeviceArray<float4> d_tri; DeviceArray<int> d_tri_obj;
 
     // BVH (built lazily; see bvh_build.h)
     HostBvh bvh;
     BvhView bview;
-    float4* d_bvh_nodes = nullptr; int* d_bvh_refs = nullptr;
-    float4* d_bvh_slots = nullptr;     // leaf-ordered primitive slots (BVHs too large to stage in shared memory)
-    uint4* d_bvh_qnodes = nullptr;     // 32-byte quantised nodes of the same tree (bvh_build.h HostQNodes)
-    size_t cap_bvh_nodes = 0, cap_bvh_refs = 0, cap_bvh_slots = 0, cap_bvh_qnodes = 0;
+    DeviceArray<float4> d_bvh_nodes; DeviceArray<int> d_bvh_refs;
+    DeviceArray<float4> d_bvh_slots;   // leaf-ordered primitive slots (BVHs too large to stage in shared memory)
+    DeviceArray<uint4> d_bvh_qnodes;   // 32-byte quantised nodes of the same tree (bvh_build.h HostQNodes)
     int opt_bvh_quant = 1;             // RT_OPT_BVH_QUANT
     HostWideBvh wide;                  // 8-wide quantised form for BVHs read from global memory (bvh_wide.h)
-    uint4* d_wide_nodes = nullptr; int* d_wide_refs = nullptr;
-    size_t cap_wide_nodes = 0, cap_wide_refs = 0;
+    DeviceArray<uint4> d_wide_nodes; DeviceArray<int> d_wide_refs;
     bool bvh_valid = false;
 
     // flat two-level accelerator for small scenes (built lazily; see flat_build.h)
     HostFlat flat;
     FlatView fview;
-    float4* d_flat_boxes = nullptr; float4* d_flat_cull = nullptr; unsigned char* d_flat_slots = nullptr; int* d_flat_ids = nullptr;
-    size_t cap_flat_boxes = 0, cap_flat_cull = 0, cap_flat_slots = 0, cap_flat_ids = 0;
+    DeviceArray<float4> d_flat_boxes, d_flat_cull; DeviceArray<unsigned char> d_flat_slots; DeviceArray<int> d_flat_ids;
     bool flat_valid = false;
 
     WavefrontBuffers* wf = nullptr;    // RT_PIPELINE_WAVEFRONT state (rt_wavefront.cu), allocated on first use
 
-    // frame buffers
-    float4* d_accum = nullptr;
-    uint32_t* d_argb = nullptr;
-    size_t cap_pixels = 0;
-    unsigned long long* d_counters = nullptr;     // kCounters words, see rt_reset_accumulation
+    // frame buffers, width x height each
+    DeviceArray<float4> d_accum;
+    DeviceArray<uint32_t> d_argb;
+    DeviceArray<unsigned long long> d_counters;   // kCounters words, see rt_reset_accumulation
     // per-pixel primary-hit cache (RT_OPT_PRIMARY_REUSE; rt_kernels.cu k_primary_cache): valid until the camera, the scene or
     // the resolution changes
-    float4* d_prim_nt = nullptr; int* d_prim_id = nullptr;
-    size_t cap_prim = 0;
+    DeviceArray<float4> d_prim_nt; DeviceArray<int> d_prim_id;
     bool prim_valid = false;
-    float4* d_denoise[2] = {nullptr, nullptr};    // ping-pong images of the denoiser (rt_denoise.cu), allocated on first use
-    size_t cap_denoise = 0;
+    DeviceArray<float4> d_denoise[2];             // ping-pong images of the denoiser (rt_denoise.cu), allocated on first use
     // temporal resolve (rt_temporal.cu), allocated on first use, 88 B per pixel: history H and guides G as ping-pong pairs (half
     // tp_cur holds the last call's), the prior P
-    float4* d_tp_h[2] = {nullptr, nullptr}; float4* d_tp_nt[2] = {nullptr, nullptr}; int* d_tp_id[2] = {nullptr, nullptr};
-    float4* d_tp_prior = nullptr;
-    size_t cap_temporal = 0;
+    DeviceArray<float4> d_tp_h[2], d_tp_nt[2]; DeviceArray<int> d_tp_id[2];
+    DeviceArray<float4> d_tp_prior;
     int tp_cur = 0;
     bool tp_valid = false;                        // a history exists; it belongs to tp_pose, tp_epoch and tp_key
     TemporalPose tp_pose = {};
@@ -100,9 +92,9 @@ struct rt_ctx {
     uint64_t accum_epoch = 0;                     // bumped whenever the accumulation restarts or is replaced (rt_reset_accumulation,
                                                   // rt_write_accum, rt_set_sample_count, a resize)
     uint64_t radiance_key = 0;                    // bumped whenever the expected radiance changes (scene, mesh, radiance parameters)
-    ExchFlags* d_flags = nullptr;                 // this context's exchange flags (rt_exchange_*), zeroed at creation
+    DeviceArray<ExchFlags> d_flags;               // this context's exchange flags (rt_exchange_*), zeroed at creation
     ExchangeState exch;
-    uint32_t* d_scratch = nullptr;                // small device scratch (philox / pick)
+    DeviceArray<uint32_t> d_scratch;              // small device scratch (philox / pick)
 
     // accumulation state
     uint32_t samples = 0;          // samples per pixel in the buffer (global, after any external reduce)
@@ -119,7 +111,7 @@ struct rt_ctx {
     int tuned_accel = -1;          // RT_ACCEL_AUTO decision for the current scene/camera/params (-1: not measured yet)
     int tuned_pipeline = -1;       // RT_PIPELINE_AUTO decision for large BVH scenes (-1: not measured yet)
     float tune_pipe_ms[3] = {0.f, 0.f, 0.f};
-    float4* d_tune = nullptr; size_t cap_tune = 0;
+    DeviceArray<float4> d_tune;
     float tune_ms[4] = {0.f, 0.f, 0.f, 0.f};
     int used_pipeline = RT_PIPELINE_REGEN, used_accel = RT_ACCEL_BRUTE;
     float last_render_ms = 0.f, last_resolve_ms = 0.f;

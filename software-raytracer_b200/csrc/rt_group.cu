@@ -191,7 +191,7 @@ int rt_group_resolve_rgba8(rt_group* g, uint32_t* host_out, int pitch_bytes, int
         if (rc != RT_OK) return member_fail(g, i, rc);
         if (c->par.width != w || c->par.height != h) return gfail(g, RT_ERR_INVALID, "rt_group_resolve_rgba8: members differ in resolution");
         total += c->samples;
-        accum[i] = c->d_accum;
+        accum[i] = c->d_accum.get();
         RTG_CUDA(g, cudaEventRecord(g->ev_rendered[(size_t)i], c->stream));          // "my samples are in my buffer"
     }
     const long long n_px = (long long)w * h;
@@ -200,7 +200,7 @@ int rt_group_resolve_rgba8(rt_group* g, uint32_t* host_out, int pitch_bytes, int
         RTG_CUDA(g, cudaSetDevice(c->device));
         for (int j = 0; j < n; ++j) if (j != i) RTG_CUDA(g, cudaStreamWaitEvent(c->stream, g->ev_rendered[(size_t)j], 0));
         const int first = (int)(n_px * i / n), count = (int)(n_px * (i + 1) / n) - first;
-        const int rc = rtb_capi::resolve_fused_unchecked(c, accum, n, total, first, count, c0->d_argb, flip_y);   // peer access was enabled at creation
+        const int rc = rtb_capi::resolve_fused_unchecked(c, accum, n, total, first, count, c0->d_argb.get(), flip_y);   // peer access was enabled at creation
         if (rc != RT_OK) return member_fail(g, i, rc);
         RTG_CUDA(g, cudaSetDevice(c->device));
         RTG_CUDA(g, cudaEventRecord(g->ev_resolved[(size_t)i], c->stream));          // "my slice is written, I have read your buffers"

@@ -1,5 +1,5 @@
 // rt_temporal.cu - the temporal resolve behind rt_temporal_rgba8 / rt_read_temporal: one launch per call, one thread per pixel.
-// Per-pixel math (projection, tap validity, bilinear gather, blend): rt_temporal.cuh. Prior bookkeeping: rt_capi.cu temporal().
+// Per-pixel math (projection, tap validity, bilinear gather, blend): rt_temporal.cuh. Prior bookkeeping: rt_capi.cu present().
 //
 // Each thread reads its sample sum S, its primary-hit cache entry and - when the prior is rebuilt - up to four taps of the
 // previous history H and guides G; it writes the prior (when rebuilt), the new H and G into the other half of their ping-pong

@@ -21,7 +21,7 @@
 
 namespace rtb {
 
-enum { kTpKeep = 0, kTpZero = 1, kTpCopy = 2, kTpReproject = 3 };   // how a call obtains the prior (rt_capi.cu temporal())
+enum { kTpKeep = 0, kTpZero = 1, kTpCopy = 2, kTpReproject = 3 };   // how a call obtains the prior (rt_capi.cu present())
 
 // The part of a FrameView that places rays: origin and axes (a camera pose at a resolution).
 struct TemporalPose { float3 o, u, v, f; };

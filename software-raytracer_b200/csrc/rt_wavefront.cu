@@ -23,23 +23,24 @@
 #include <cstdio>
 #include <mutex>
 
+#include "rt_devbuf.h"
 #include "rt_device.cuh"
 #include "rt_trace.cuh"
 
 namespace rtb {
 
 struct WavefrontBuffers {
-    size_t cap_paths = 0, cap_px = 0, cap_rad = 0;      // per-path state arrays | launch_acc | wave_rad
     // Path state lives in DENSE ping-pong sets: slot i of round r's set is the i-th surviving path, so every kernel reads and
     // writes consecutive records (with one fixed slot per path and a queue of path ids the survivors of the later rounds are
     // scattered and a 32-byte sector carries one useful record: the shade kernel moved 3.8x its useful bytes).
-    float4 *ray_o[2] = {nullptr, nullptr}, *ray_d[2] = {nullptr, nullptr};         // per slot: o, (d, depth)
-    float4 *thr[2] = {nullptr, nullptr}, *rad[2] = {nullptr, nullptr};             // per slot: T, L
-    uint32_t* q[2] = {nullptr, nullptr};                                          // per slot: path id (tile-major pixel + npad * sample)
-    float4 *hit_nt = nullptr; int* hit_id = nullptr;                              // per slot of the current round: (normal, t), object id
-    float4* wave_rad = nullptr;                                                   // per PATH id: radiance of the finished path
-    unsigned int* counters = nullptr;                                             // [0..63] queue lengths per round, [64..127] cursors
-    float4* launch_acc = nullptr;                                                 // per pixel: this launch's sum
+    DeviceArray<float4> ray_o[2], ray_d[2];           // per slot: o, (d, depth)
+    DeviceArray<float4> thr[2], rad[2];               // per slot: T, L
+    DeviceArray<uint32_t> q[2];                       // per slot: path id (tile-major pixel + npad * sample)
+    DeviceArray<float4> hit_nt; DeviceArray<int> hit_id;   // per slot of the current round: (normal, t), object id
+    DeviceArray<float4> wave_rad;                     // per PATH id: radiance of the finished path
+    DeviceArray<unsigned int> counters;               // [0..63] queue lengths per round, [64..127] cursors
+    DeviceArray<float4> launch_acc;                   // per pixel: this launch's sum
+    size_t paths() const { return q[1].capacity(); }  // paths the per-path arrays hold (alloc_paths: all of them or none)
 };
 
 namespace {
@@ -595,15 +596,6 @@ __global__ void k_wf_commit(int n, const float4* __restrict__ launch_acc, float4
     accum[p] = a;
 }
 
-template <typename T>
-cudaError_t grow(T*& p, size_t n) {
-    if (p) cudaFree(p);
-    p = nullptr;
-    const cudaError_t e = cudaMalloc((void**)&p, n * sizeof(T));
-    if (e != cudaSuccess) p = nullptr;
-    return e;
-}
-
 template <typename K>
 cudaError_t optin(K kernel) { return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxStagedBytes); }
 
@@ -644,54 +636,21 @@ cudaError_t ensure_optin() {
 
 WavefrontBuffers* wavefront_create() { return new WavefrontBuffers(); }
 
-// frees the path-state arrays (everything that scales with the wave); the small counter block stays
+// frees the path state (everything that scales with the wave); the small counter block stays
 void wavefront_release(WavefrontBuffers* wb) {
     if (!wb) return;
-    for (int k = 0; k < 2; ++k) {
-        cudaFree(wb->ray_o[k]); cudaFree(wb->ray_d[k]); cudaFree(wb->thr[k]); cudaFree(wb->rad[k]); cudaFree(wb->q[k]);
-        wb->ray_o[k] = wb->ray_d[k] = wb->thr[k] = wb->rad[k] = nullptr; wb->q[k] = nullptr;
-    }
-    cudaFree(wb->hit_nt); cudaFree(wb->hit_id); cudaFree(wb->wave_rad); cudaFree(wb->launch_acc);
-    wb->hit_nt = nullptr; wb->hit_id = nullptr; wb->wave_rad = nullptr; wb->launch_acc = nullptr;
-    wb->cap_paths = wb->cap_px = wb->cap_rad = 0;
+    DeviceArray<unsigned int> counters = std::move(wb->counters);
+    *wb = WavefrontBuffers();
+    wb->counters = std::move(counters);
 }
 
-void wavefront_destroy(WavefrontBuffers* wb) {
-    if (!wb) return;
-    wavefront_release(wb);
-    cudaFree(wb->counters);
-    delete wb;
-}
+void wavefront_destroy(WavefrontBuffers* wb) { delete wb; }
 
 namespace {
-// all per-path arrays for `n` paths; on failure everything is freed again and the thread's last error is cleared
+// every per-path array for `n` paths, or none of them on failure (launch_acc, the per-pixel sum, stays)
 cudaError_t alloc_paths(WavefrontBuffers* wb, size_t n) {
-    cudaError_t e;
-    if ((e = grow(wb->ray_o[0], n)) != cudaSuccess || (e = grow(wb->ray_d[0], n)) != cudaSuccess ||
-        (e = grow(wb->thr[0], n)) != cudaSuccess || (e = grow(wb->rad[0], n)) != cudaSuccess ||
-        (e = grow(wb->ray_o[1], n)) != cudaSuccess || (e = grow(wb->ray_d[1], n)) != cudaSuccess ||
-        (e = grow(wb->thr[1], n)) != cudaSuccess || (e = grow(wb->rad[1], n)) != cudaSuccess ||
-        (e = grow(wb->hit_nt, n)) != cudaSuccess || (e = grow(wb->hit_id, n)) != cudaSuccess ||
-        (wb->cap_rad < n && (e = grow(wb->wave_rad, n)) != cudaSuccess) || (e = grow(wb->q[0], n)) != cudaSuccess ||
-        (e = grow(wb->q[1], n)) != cudaSuccess) {
-        float4* keep = wb->launch_acc; const size_t keep_px = wb->cap_px;
-        wb->launch_acc = nullptr;
-        wavefront_release(wb);
-        wb->launch_acc = keep; wb->cap_px = keep_px;
-        cudaGetLastError();                                  // a failed cudaMalloc leaves the error set: the next launch check must not see it
-        return e;
-    }
-    wb->cap_paths = n;
-    if (wb->cap_rad < n) wb->cap_rad = n;
-    return cudaSuccess;
-}
-// the streaming kernel needs only the finished radiance per path
-cudaError_t alloc_radiance(WavefrontBuffers* wb, size_t n) {
-    if (wb->cap_rad >= n) return cudaSuccess;
-    const cudaError_t e = grow(wb->wave_rad, n);
-    if (e != cudaSuccess) { wb->cap_rad = 0; cudaGetLastError(); return e; }
-    wb->cap_rad = n;
-    return cudaSuccess;
+    return reserve_all(n, wb->ray_o[0], wb->ray_d[0], wb->thr[0], wb->rad[0], wb->ray_o[1], wb->ray_d[1], wb->thr[1], wb->rad[1],
+                       wb->hit_nt, wb->hit_id, wb->wave_rad, wb->q[0], wb->q[1]);
 }
 }  // namespace
 
@@ -722,7 +681,7 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
     {
         size_t free_b = 0, total_b = 0;
         if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-            const size_t have = streaming ? wb->cap_rad * sizeof(float4) : wb->cap_paths * kBytesPerPath;
+            const size_t have = streaming ? wb->wave_rad.capacity() * sizeof(float4) : wb->paths() * kBytesPerPath;
             const size_t budget = (free_b + have) / 3 / bytes_per_path;
             if (wave_paths > budget) wave_paths = budget;
         }
@@ -734,15 +693,15 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
     // equal waves: 16 samples with room for 15 are two waves of 8, not 15 + a single-sample wave that runs mostly in its tail
     { const int n_waves = (n_samples + s_cap - 1) / s_cap; s_cap = (n_samples + n_waves - 1) / n_waves; }
     if ((size_t)g.npad * s_cap >= (size_t)1 << 32) return cudaErrorInvalidValue;
-    if (wb->cap_px < npix) {
+    if (wb->launch_acc.capacity() < npix) {
         cudaStreamSynchronize(st);
-        if ((e = grow(wb->launch_acc, npix)) != cudaSuccess) { wb->cap_px = 0; cudaGetLastError(); return e; }
-        wb->cap_px = npix;
+        if ((e = wb->launch_acc.reserve(npix)) != cudaSuccess) return e;
     }
-    if (streaming ? wb->cap_rad < (size_t)g.npad * s_cap : wb->cap_paths < (size_t)g.npad * s_cap) {
+    if ((streaming ? wb->wave_rad.capacity() : wb->paths()) < (size_t)g.npad * s_cap) {
         cudaStreamSynchronize(st);
         for (;;) {
-            e = streaming ? alloc_radiance(wb, (size_t)g.npad * s_cap) : alloc_paths(wb, (size_t)g.npad * s_cap);
+            // the streaming kernel needs only the finished radiance per path
+            e = streaming ? wb->wave_rad.reserve((size_t)g.npad * s_cap) : alloc_paths(wb, (size_t)g.npad * s_cap);
             if (e == cudaSuccess) break;
             if (e != cudaErrorMemoryAllocation || s_cap == 1) return e;      // s_cap == 1: not even one sample per pixel fits
             s_cap = (s_cap + 1) / 2;
@@ -754,7 +713,7 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
         fprintf(stderr, "[rtb200] wavefront launch: %d samples, %d per wave (%zu M paths, %s), free %.1f of %.1f GB\n", n_samples, s_cap, ((size_t)g.npad * s_cap) >> 20,
                 streaming ? "streaming" : "bounce rounds", free_b / 1e9, total_b / 1e9);
     }
-    if (!wb->counters && (e = cudaMalloc((void**)&wb->counters, 2 * kMaxRounds * sizeof(unsigned int))) != cudaSuccess) { cudaGetLastError(); return e; }
+    if ((e = wb->counters.reserve(2 * kMaxRounds)) != cudaSuccess) return e;
     const int rounds = reuse ? fr.max_bounces : fr.max_bounces + 1;
     if (!streaming && rounds > kMaxRounds - 1) return cudaErrorInvalidValue;      // one queue counter per bounce round; the streaming kernel has no rounds
 
@@ -764,17 +723,17 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
     const int persistent_blocks = sms * 8;
     const bool count = count_traversal && (mode == 2 || mode == 3) && bvh_refill && !ac.bvh.wnodes;
 
-    if ((e = cudaMemsetAsync(wb->launch_acc, 0, npix * sizeof(float4), st)) != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(wb->launch_acc.get(), 0, npix * sizeof(float4), st)) != cudaSuccess) return e;
     for (int s0 = 0; s0 < n_samples; s0 += s_cap) {
         const int sw = n_samples - s0 < s_cap ? n_samples - s0 : s_cap;
         const uint32_t s_first = s_begin + (uint32_t)s0;
         const size_t np = (size_t)g.npad * sw;
-        if ((e = cudaMemsetAsync(wb->counters, 0, 2 * kMaxRounds * sizeof(unsigned int), st)) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(wb->counters.get(), 0, 2 * kMaxRounds * sizeof(unsigned int), st)) != cudaSuccess) return e;
         if (streaming) {
             // one persistent launch per wave: paths are claimed from counters[0], traced and shaded to the end in the kernel
             const size_t ssb = sb + (size_t)((kStreamStateWords * kThreads + 3) / 4) * sizeof(float4);
             const int blocks = sms * RTB_WF_STREAM_MIN_BLOCKS;
-#define RTB_STREAM_ARGS sc, ac.bvh, ac.flat, fr, g.tiles_x, g.npad, s_first, (unsigned int)np, prim_nt, prim_id, wb->wave_rad, wb->counters, k_refill, k_node_min, seg_counter
+#define RTB_STREAM_ARGS sc, ac.bvh, ac.flat, fr, g.tiles_x, g.npad, s_first, (unsigned int)np, prim_nt, prim_id, wb->wave_rad.get(), wb->counters.get(), k_refill, k_node_min, seg_counter
 #define RTB_STREAM_LAUNCH(M, Q)                                                                                                     \
             if (reuse) { if (count) k_wf_stream<M, true, true, Q><<<blocks, kThreads, ssb, st>>>(RTB_STREAM_ARGS);                  \
                          else k_wf_stream<M, true, false, Q><<<blocks, kThreads, ssb, st>>>(RTB_STREAM_ARGS); }                    \
@@ -783,21 +742,21 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
             if (mode == 2) { RTB_STREAM_LAUNCH(2, false) } else if (ac.bvh.qnodes) { RTB_STREAM_LAUNCH(3, true) } else { RTB_STREAM_LAUNCH(3, false) }
 #undef RTB_STREAM_LAUNCH
 #undef RTB_STREAM_ARGS
-            k_wf_accumulate<<<(g.npad + 255) / 256, 256, 0, st>>>(fr, g.tiles_x, g.npad, sw, wb->wave_rad, wb->launch_acc);
+            k_wf_accumulate<<<(g.npad + 255) / 256, 256, 0, st>>>(fr, g.tiles_x, g.npad, sw, wb->wave_rad.get(), wb->launch_acc.get());
             continue;
         }
         const int gen_blocks = (int)((np + 255) / 256);
-        if (reuse) k_wf_generate<true><<<gen_blocks, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, sw, prim_nt, prim_id, wb->ray_o[0], wb->ray_d[0],
-                                                                    wb->thr[0], wb->rad[0], wb->wave_rad, wb->q[0], wb->counters, seg_counter);
-        else k_wf_generate<false><<<gen_blocks, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, sw, prim_nt, prim_id, wb->ray_o[0], wb->ray_d[0],
-                                                               wb->thr[0], wb->rad[0], wb->wave_rad, wb->q[0], wb->counters, seg_counter);
+        if (reuse) k_wf_generate<true><<<gen_blocks, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, sw, prim_nt, prim_id, wb->ray_o[0].get(), wb->ray_d[0].get(),
+                                                                    wb->thr[0].get(), wb->rad[0].get(), wb->wave_rad.get(), wb->q[0].get(), wb->counters.get(), seg_counter);
+        else k_wf_generate<false><<<gen_blocks, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, sw, prim_nt, prim_id, wb->ray_o[0].get(), wb->ray_d[0].get(),
+                                                               wb->thr[0].get(), wb->rad[0].get(), wb->wave_rad.get(), wb->q[0].get(), wb->counters.get(), seg_counter);
         for (int r = 0; r < rounds; ++r) {
             const int a = r & 1, b = a ^ 1;                  // this round's dense state set, the next round's
-            const uint32_t* qin = wb->q[a];
-            uint32_t* qout = wb->q[b];
-            unsigned int* cnt = wb->counters + r;
-            unsigned int* cur = wb->counters + kMaxRounds + r;
-#define RTB_WF_ARGS sc, ac.bvh, ac.flat, qin, cnt, cur, wb->ray_o[a], wb->ray_d[a], wb->hit_nt, wb->hit_id
+            const uint32_t* qin = wb->q[a].get();
+            uint32_t* qout = wb->q[b].get();
+            unsigned int* cnt = wb->counters.get() + r;
+            unsigned int* cur = wb->counters.get() + kMaxRounds + r;
+#define RTB_WF_ARGS sc, ac.bvh, ac.flat, qin, cnt, cur, wb->ray_o[a].get(), wb->ray_d[a].get(), wb->hit_nt.get(), wb->hit_id.get()
             switch (mode) {
                 case 0: k_wf_intersect<0><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS); break;
                 case 1: k_wf_intersect<1><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS); break;
@@ -805,7 +764,7 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
                         else if (bvh_refill) k_wf_intersect_bvh<2><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS, k_refill, k_node_min, seg_counter);
                         else k_wf_intersect<2><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS);
                         break;
-                case 3: if (bvh_refill && ac.bvh.wnodes) k_wf_intersect_bvh8<<<sms * RTB_WF_BVH8_MIN_BLOCKS, kThreads, sb, st>>>(sc, ac.bvh, qin, cnt, cur, wb->ray_o[a], wb->ray_d[a], wb->hit_nt, wb->hit_id, k_refill, k_node_min);
+                case 3: if (bvh_refill && ac.bvh.wnodes) k_wf_intersect_bvh8<<<sms * RTB_WF_BVH8_MIN_BLOCKS, kThreads, sb, st>>>(sc, ac.bvh, qin, cnt, cur, wb->ray_o[a].get(), wb->ray_d[a].get(), wb->hit_nt.get(), wb->hit_id.get(), k_refill, k_node_min);
                         else if (count && ac.bvh.qnodes) k_wf_intersect_bvh<3, true, true><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS, k_refill, k_node_min, seg_counter);
                         else if (count) k_wf_intersect_bvh<3, true><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS, k_refill, k_node_min, seg_counter);
                         else if (bvh_refill && ac.bvh.qnodes) k_wf_intersect_bvh<3, false, true><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS, k_refill, k_node_min, seg_counter);
@@ -815,12 +774,12 @@ cudaError_t launch_render_wavefront(WavefrontBuffers* wb, const SceneView& sc, c
                 default: k_wf_intersect<4><<<persistent_blocks, kThreads, sb, st>>>(RTB_WF_ARGS); break;
             }
 #undef RTB_WF_ARGS
-            k_wf_shade<<<sms * 8, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, qin, cnt, qout, cnt + 1, wb->ray_o[a], wb->ray_d[a], wb->thr[a], wb->rad[a], wb->ray_o[b], wb->ray_d[b], wb->thr[b], wb->rad[b],
-                                                 wb->hit_nt, wb->hit_id, wb->wave_rad, seg_counter);
+            k_wf_shade<<<sms * 8, 256, 0, st>>>(sc, fr, g.tiles_x, g.npad, s_first, qin, cnt, qout, cnt + 1, wb->ray_o[a].get(), wb->ray_d[a].get(), wb->thr[a].get(), wb->rad[a].get(), wb->ray_o[b].get(), wb->ray_d[b].get(), wb->thr[b].get(), wb->rad[b].get(),
+                                                 wb->hit_nt.get(), wb->hit_id.get(), wb->wave_rad.get(), seg_counter);
         }
-        k_wf_accumulate<<<(g.npad + 255) / 256, 256, 0, st>>>(fr, g.tiles_x, g.npad, sw, wb->wave_rad, wb->launch_acc);
+        k_wf_accumulate<<<(g.npad + 255) / 256, 256, 0, st>>>(fr, g.tiles_x, g.npad, sw, wb->wave_rad.get(), wb->launch_acc.get());
     }
-    k_wf_commit<<<(int)((npix + 255) / 256), 256, 0, st>>>((int)npix, wb->launch_acc, accum);
+    k_wf_commit<<<(int)((npix + 255) / 256), 256, 0, st>>>((int)npix, wb->launch_acc.get(), accum);
     return cudaGetLastError();
 }
 
