@@ -415,6 +415,21 @@ int rt_group_set_option(rt_group* g, int option, int value);
 int rt_group_reset_accumulation(rt_group* g);
 int rt_group_render_spp(rt_group* g, int spp);               /* spp = GLOBAL samples per pixel, split over the devices */
 int rt_group_resolve_rgba8(rt_group* g, uint32_t* host_out, int pitch_bytes, int flip_y);
+/* The denoised and temporal resolves of the group's image: rt_denoise_rgba8 / rt_read_denoised / rt_temporal_rgba8 / rt_read_temporal /
+ * rt_reset_temporal with the same parameters and NULL defaults, over the sum that rt_group_resolve_rgba8 presents - every member's
+ * accumulation buffer added in member order - and the total of the members' sample counts. The sum is gathered into a buffer on device
+ * 0 (16 B per pixel, allocated on the first call, freed on a resize) by one kernel per member over its slice of the pixels, in
+ * the same arithmetic as the fused resolve; device 0 then filters / blends and packs it. So preview mode and passes 0 give
+ * rt_group_resolve_rgba8's bits. Read-only on every member's accumulation buffer, sample counter and path statistics. The guides and
+ * the temporal history (pose, accumulation epoch, radiance key) are member 0's: every setter is broadcast and
+ * rt_group_reset_accumulation restarts member 0 too, so they describe the group. Bad parameters or output buffer: RT_ERR_INVALID,
+ * checked before anything is launched (the history stays as it was). last_resolve_ms of member 0 (rt_group_get_stats) reports
+ * filter + pack, not the reduce. Synchronise. */
+int rt_group_denoise_rgba8(rt_group* g, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y);
+int rt_group_read_denoised(rt_group* g, const rt_denoise_params* p, float* host_rgba);
+int rt_group_temporal_rgba8(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y);
+int rt_group_read_temporal(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, float* host_rgba);
+int rt_group_reset_temporal(rt_group* g);
 int rt_group_get_stats(rt_group* g, rt_stats* out);           /* sums over the members; last_render_ms = the slowest */
 
 #ifdef __cplusplus

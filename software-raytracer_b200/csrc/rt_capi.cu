@@ -702,9 +702,9 @@ int rt_set_params(rt_ctx* c, const rt_params* p) {
     if (resized) {
         RT_CUDA(c, cudaSetDevice(c->device));
         RT_CUDA(c, cudaStreamSynchronize(c->stream));
-        // the frame buffers, the denoiser pair (32 B per pixel) and the temporal set (88 B per pixel, the history is gone with it) are
-        // sized for the old resolution
-        c->d_accum.reset(); c->d_argb.reset();
+        // the frame buffers, the denoiser pair (32 B per pixel), a group's gather buffer (16 B per pixel) and the temporal set (88 B per
+        // pixel, the history is gone with it) are sized for the old resolution
+        c->d_accum.reset(); c->d_argb.reset(); c->d_gather.reset();
         for (int k = 0; k < 2; ++k) { c->d_denoise[k].reset(); c->d_tp_h[k].reset(); c->d_tp_nt[k].reset(); c->d_tp_id[k].reset(); }
         c->d_tp_prior.reset();
         c->tp_valid = false;
@@ -916,27 +916,32 @@ static int check_temporal_params(rt_ctx* c, const char* fn, const rt_temporal_pa
     return RT_OK;
 }
 
-// Where a presented image goes: an ARGB8 host surface, or (argb NULL) the float (r, g, b, .) image of the filter or the temporal blend.
-struct PresentOut {
-    uint32_t* argb; int pitch_bytes; int flip_y;
-    float* rgba;
-};
+}  // extern "C"
+
+namespace rtb_capi {
+int check_present(rt_ctx* c, const char* fn, const PresentOut& out, bool full, const rt_temporal_params* tp, const rt_denoise_params* dn,
+                  int* pow_log2) {
+    int rc, pw = 0;
+    if (out.argb ? out.pitch_bytes < c->par.width * 4 : !out.rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
+    if (tp && !full) return fail(c, RT_ERR_INVALID, std::string(fn) + ": not supported on a shard (its buffer holds only part of the samples)");
+    if (tp && (rc = check_temporal_params(c, fn, *tp)) != RT_OK) return rc;
+    if (dn && (rc = check_denoise_params(c, fn, *dn, pw)) != RT_OK) return rc;
+    if (pow_log2) *pow_log2 = pw;
+    return RT_OK;
+}
 
 // Every call that presents an image. spp != NULL (rt_render_frame): *spp samples are rendered first, and for 1-2 samples the render
-// kernel may resolve the frame itself. Then the image: the plain resolve; with dn the filter of rt_denoise.cu, guided by the
-// primary-hit cache; with tp the prior from the temporal history (rt_temporal.cuh) and the blend, filtered when dn has passes, and the
-// new history. Apart from the render, read-only on the accumulation buffer, the sample counter and the path statistics.
-static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_temporal_params* tp, const rt_denoise_params* dn,
-                   const int* spp = nullptr) {
+// kernel may resolve the frame itself. Then the image of the source: the plain resolve; with dn the filter of rt_denoise.cu, guided by
+// the primary-hit cache; with tp the prior from the temporal history (rt_temporal.cuh) and the blend, filtered when dn has passes, and
+// the new history. Apart from the render, read-only on the source, the accumulation buffer, the sample counter and the path statistics.
+int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_temporal_params* tp, const rt_denoise_params* dn,
+            const PresentSrc* src, const int* spp) {
     int rc = prepare(c);
     if (rc != RT_OK) return rc;
     const int w = c->par.width, h = c->par.height;
     const size_t px = (size_t)w * h;
-    if (out.argb ? out.pitch_bytes < w * 4 : !out.rgba) return fail(c, RT_ERR_INVALID, std::string(fn) + ": bad output buffer");
-    if (tp && c->world > 1) return fail(c, RT_ERR_INVALID, std::string(fn) + ": not supported on a shard (its buffer holds only part of the samples)");
-    if (tp && (rc = check_temporal_params(c, fn, *tp)) != RT_OK) return rc;
     int pow_log2 = 0;
-    if (dn && (rc = check_denoise_params(c, fn, *dn, pow_log2)) != RT_OK) return rc;
+    if ((rc = check_present(c, fn, out, src ? src->full : c->world == 1, tp, dn, &pow_log2)) != RT_OK) return rc;
     // preview shading is deterministic: nothing to filter, and no history
     const bool preview = c->par.mode == RT_MODE_PREVIEW;
     const int passes = dn && !preview ? dn->passes : 0;
@@ -953,6 +958,7 @@ static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_te
         if ((rc = render_samples(c, *spp, candidate ? &ft : nullptr)) != RT_OK) return rc;
         fused = ft.fused;
     }
+    const PresentSrc s = src ? *src : PresentSrc{c->d_accum.get(), c->samples, c->world == 1};
     if (passes > 0 || (tp && !preview)) {
         AccelSel ac;
         if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
@@ -973,7 +979,7 @@ static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_te
     TemporalLaunch t;
     const int cur = c->tp_cur ^ 1;                             // the half the new history goes to
     if (tp) {
-        t.accum = c->d_accum.get(); t.count = (float)c->samples;
+        t.accum = s.sum; t.count = (float)s.samples;
         t.nt = preview ? nullptr : c->d_prim_nt.get(); t.id = preview ? nullptr : c->d_prim_id.get();
         t.width = w; t.height = h;
         t.cap = (float)tp->max_history; t.tau_z = tp->tau_depth; t.tau_n = tp->tau_normal;
@@ -997,10 +1003,10 @@ static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_te
     if (!fused) {
         cudaEventRecord(c->ev2, c->stream);
         if (tp) e = launch_temporal(t, c->stream);
-        else if (!filter) e = launch_resolve(c->d_accum.get(), c->samples, w, h, 0, w * h, flip_y, c->d_argb.get(), 0, c->stream, mapped);
+        else if (!filter) e = launch_resolve(s.sum, s.samples, w, h, 0, w * h, flip_y, c->d_argb.get(), 0, c->stream, mapped);
         if (e == cudaSuccess && filter) {
             DenoiseLaunch d;
-            d.accum = tp ? nullptr : c->d_accum.get(); d.samples = tp ? 0 : c->samples;
+            d.accum = tp ? nullptr : s.sum; d.samples = tp ? 0 : s.samples;
             d.nt = c->d_prim_nt.get(); d.id = c->d_prim_id.get();
             d.width = w; d.height = h; d.passes = passes; d.pow_log2 = pow_log2;
             d.sigma_color = dn->sigma_color; d.sigma_depth = dn->sigma_depth;
@@ -1031,13 +1037,17 @@ static int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_te
     }
     return RT_OK;
 }
+}  // namespace rtb_capi
+using rtb_capi::present;
+
+extern "C" {
 
 // One progressive frame: rt_render_spp(spp) + rt_resolve_rgba8(host_out) with the same result, as ONE call - which is what the
 // reference's frame is (renderArea resolves every pixel as it is traced, Raytracer.cpp:63-76,223-257). For 1-2 samples per pixel the
 // render kernel resolves the pixels it finishes and streams them to a page-locked surface while it is still tracing (FrameOut,
 // rt_kernels.cu); every other case runs the two steps one after the other.
 int rt_render_frame(rt_ctx* c, int spp, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    return present(c, "rt_render_frame", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr, &spp);
+    return present(c, "rt_render_frame", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr, nullptr, &spp);
 }
 
 int rt_resolve_device(rt_ctx* c, const void* dev_accum, uint32_t samples, int first_pixel, int n_pixels, void* dev_out, int flip_y) {
@@ -1052,7 +1062,7 @@ int rt_resolve_device(rt_ctx* c, const void* dev_accum, uint32_t samples, int fi
 }
 
 int rt_resolve_rgba8(rt_ctx* c, uint32_t* host_out, int pitch_bytes, int flip_y) {
-    return present(c, "rt_resolve_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr);
+    return present(c, "rt_resolve_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, nullptr, nullptr);
 }
 
 void rt_default_denoise_params(rt_denoise_params* p) {
@@ -1063,13 +1073,13 @@ void rt_default_denoise_params(rt_denoise_params* p) {
 int rt_denoise_rgba8(rt_ctx* c, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y) {
     rt_denoise_params d;
     if (!p) rt_default_denoise_params(&d);
-    return present(c, "rt_denoise_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, p ? p : &d);
+    return present(c, "rt_denoise_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, p ? p : &d, nullptr);
 }
 
 int rt_read_denoised(rt_ctx* c, const rt_denoise_params* p, float* host_rgba) {
     rt_denoise_params d;
     if (!p) rt_default_denoise_params(&d);
-    return present(c, "rt_read_denoised", {nullptr, 0, 0, host_rgba}, nullptr, p ? p : &d);
+    return present(c, "rt_read_denoised", {nullptr, 0, 0, host_rgba}, nullptr, p ? p : &d, nullptr);
 }
 
 void rt_default_temporal_params(rt_temporal_params* p) {
@@ -1081,13 +1091,13 @@ void rt_default_temporal_params(rt_temporal_params* p) {
 int rt_temporal_rgba8(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y) {
     rt_temporal_params d;
     if (!p) rt_default_temporal_params(&d);
-    return present(c, "rt_temporal_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, p ? p : &d, dn);
+    return present(c, "rt_temporal_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, p ? p : &d, dn, nullptr);
 }
 
 int rt_read_temporal(rt_ctx* c, const rt_temporal_params* p, const rt_denoise_params* dn, float* host_rgba) {
     rt_temporal_params d;
     if (!p) rt_default_temporal_params(&d);
-    return present(c, "rt_read_temporal", {nullptr, 0, 0, host_rgba}, p ? p : &d, dn);
+    return present(c, "rt_read_temporal", {nullptr, 0, 0, host_rgba}, p ? p : &d, dn, nullptr);
 }
 
 int rt_reset_temporal(rt_ctx* c) {

@@ -81,6 +81,8 @@ struct rt_ctx {
     DeviceArray<float4> d_prim_nt; DeviceArray<int> d_prim_id;
     bool prim_valid = false;
     DeviceArray<float4> d_denoise[2];             // ping-pong images of the denoiser (rt_denoise.cu), allocated on first use
+    DeviceArray<float4> d_gather;                 // member 0 of a group: the rank-order sum of every member's buffer (rt_group.cu),
+                                                  // allocated on first use
     // temporal resolve (rt_temporal.cu), allocated on first use, 88 B per pixel: history H and guides G as ping-pong pairs (half
     // tp_cur holds the last call's), the prior P
     DeviceArray<float4> d_tp_h[2], d_tp_nt[2]; DeviceArray<int> d_tp_id[2];
@@ -127,4 +129,22 @@ int prepare(rt_ctx* c);
 int enable_peer_access_to(rt_ctx* c, const void* ptr, const char* what);   // no-op for the context's own device
 int resolve_fused_unchecked(rt_ctx* c, const void* const* accum_ptrs, int world, uint32_t total_samples, int first_pixel, int n_pixels,
                             void* dst, int flip_y);
+
+// Where a presented image goes: an ARGB8 host surface, or (argb NULL) the float (r, g, b, .) image of the filter or the temporal blend.
+struct PresentOut {
+    uint32_t* argb; int pitch_bytes; int flip_y;
+    float* rgba;
+};
+// What present() resolves: a sum image (width * height float4 on the context's device) holding `samples` samples per pixel; `full`:
+// it holds every sample of the image (not a shard's part), which the temporal history needs.
+struct PresentSrc {
+    const float4* sum; uint32_t samples; bool full;
+};
+// present()'s argument checks (output, temporal and filter parameters), with the messages of the single-context calls; *pow_log2:
+// log2 of the filter's normal power
+int check_present(rt_ctx* c, const char* fn, const PresentOut& out, bool full, const rt_temporal_params* tp, const rt_denoise_params* dn,
+                  int* pow_log2 = nullptr);
+// src NULL: the context's own accumulation buffer, {d_accum, samples, world == 1} after prepare() and the optional render
+int present(rt_ctx* c, const char* fn, const PresentOut& out, const rt_temporal_params* tp, const rt_denoise_params* dn,
+            const PresentSrc* src, const int* spp = nullptr);
 }

@@ -3,6 +3,8 @@
 // member's accumulation buffer over NVLink peer mappings and writing device 0's surface. Replaces what the reference does
 // with 16 worker threads and a spin gate (Raytracer.cpp:331-342, 374-384, 598-607): "spawn" = rt_create_multi, "frame" =
 // rt_group_render_spp (asynchronous launches on every device's stream), "join" = the event waits of rt_group_resolve_rgba8.
+// The denoised and temporal resolves run the same exchange with the reduce kernel instead, which gathers the unresolved sum on
+// device 0, and then present it there like a single context.
 // No torch, no NCCL, no IPC: in one process the peers' buffers are ordinary device pointers once peer access is enabled, and
 // the ordering between the devices' streams is expressed with CUDA events.
 #include <cuda_runtime.h>
@@ -16,7 +18,7 @@
 
 struct rt_group {
     std::vector<rt_ctx*> ctx;
-    std::vector<cudaEvent_t> ev_rendered, ev_resolved;    // per member, on its device
+    std::vector<cudaEvent_t> ev_rendered, ev_read;    // per member, on its device (exchange())
     std::string err;
 };
 
@@ -55,6 +57,88 @@ int for_members(rt_group* g, bool threads, F fn) {
     }
     for (int i = 0; i < n; ++i) if (rc[(size_t)i] < 0) return member_fail(g, i, rc[(size_t)i]);
     return rc.empty() ? RT_OK : rc[0];
+}
+
+// Every member's accumulation buffer (rank order) and the sum of their sample counts; the members must agree on the resolution.
+int collect(rt_group* g, const char* fn, const void** accum, uint32_t& total) {
+    const int w = g->ctx[0]->par.width, h = g->ctx[0]->par.height;
+    total = 0;
+    for (size_t i = 0; i < g->ctx.size(); ++i) {
+        rt_ctx* c = g->ctx[i];
+        const int rc = rtb_capi::prepare(c);
+        if (rc != RT_OK) return member_fail(g, (int)i, rc);
+        if (c->par.width != w || c->par.height != h) return gfail(g, RT_ERR_INVALID, std::string(fn) + ": members differ in resolution");
+        total += c->samples;
+        accum[i] = c->d_accum.get();
+    }
+    return RT_OK;
+}
+
+// The ordering between the members' streams around one exchange (the fused resolve, the reduce):
+//   1. every member records "rendered": its samples are in its buffer;
+//   2. each member waits for every other member's "rendered" and runs launch(i, first, count) over its slice of the pixels,
+//      [n_px * i / n, n_px * (i + 1) / n);
+//   3. it records "read": its slice is written and it has read every buffer;
+//   4. every member waits for every "read": nobody touches its buffer again (next reset / render) before all have read it, and
+//      whatever member 0 enqueues next sees the whole result.
+// launch returns RT_OK or the group's error code (it sets g->err).
+template <typename F>
+int exchange(rt_group* g, F launch) {
+    const int n = (int)g->ctx.size();
+    for (int i = 0; i < n; ++i) {
+        RTG_CUDA(g, cudaSetDevice(g->ctx[(size_t)i]->device));
+        RTG_CUDA(g, cudaEventRecord(g->ev_rendered[(size_t)i], g->ctx[(size_t)i]->stream));
+    }
+    const long long n_px = (long long)g->ctx[0]->par.width * g->ctx[0]->par.height;
+    for (int i = 0; i < n; ++i) {
+        rt_ctx* c = g->ctx[(size_t)i];
+        RTG_CUDA(g, cudaSetDevice(c->device));
+        for (int j = 0; j < n; ++j) if (j != i) RTG_CUDA(g, cudaStreamWaitEvent(c->stream, g->ev_rendered[(size_t)j], 0));
+        const int first = (int)(n_px * i / n), count = (int)(n_px * (i + 1) / n) - first;
+        const int rc = launch(i, first, count);
+        if (rc != RT_OK) return rc;
+        RTG_CUDA(g, cudaSetDevice(c->device));
+        RTG_CUDA(g, cudaEventRecord(g->ev_read[(size_t)i], c->stream));
+    }
+    for (int i = 0; i < n; ++i) {
+        rt_ctx* c = g->ctx[(size_t)i];
+        RTG_CUDA(g, cudaSetDevice(c->device));
+        for (int j = 0; j < n; ++j) if (j != i) RTG_CUDA(g, cudaStreamWaitEvent(c->stream, g->ev_read[(size_t)j], 0));
+    }
+    return RT_OK;
+}
+
+// The group's denoised and temporal resolves: the rank-order sum of every member's buffer is gathered into member 0's d_gather
+// (k_reduce_fused, each member storing its slice over NVLink), and member 0 presents it as the whole image's samples through the
+// single-context path, with its own primary-hit guides, history, pose, accumulation epoch and radiance key (every setter is broadcast,
+// so they are the group's). Checks everything before the first launch.
+int group_present(rt_group* g, const char* fn, const rtb_capi::PresentOut& out, const rt_temporal_params* tp, const rt_denoise_params* dn) {
+    if (!g) return RT_ERR_INVALID;
+    const int n = (int)g->ctx.size();
+    rt_ctx* c0 = g->ctx[0];
+    int rc = rtb_capi::check_present(c0, fn, out, true, tp, dn);
+    if (rc != RT_OK) return member_fail(g, 0, rc);
+    const void* accum[RT_MAX_PEERS] = {};
+    uint32_t total = 0;
+    if ((rc = collect(g, fn, accum, total)) != RT_OK) return rc;
+    const size_t px = (size_t)c0->par.width * c0->par.height;
+    RTG_CUDA(g, cudaSetDevice(c0->device));
+    if (c0->d_gather.capacity() < px) {
+        RTG_CUDA(g, cudaStreamSynchronize(c0->stream));
+        RTG_CUDA(g, c0->d_gather.reserve(px));
+    }
+    float4* sum = c0->d_gather.get();
+    PeerPtrs pp;
+    memset(&pp, 0, sizeof pp);
+    for (int r = 0; r < n; ++r) pp.p[r] = (const float4*)accum[r];
+    rc = exchange(g, [&](int i, int first, int count) -> int {
+        RTG_CUDA(g, launch_reduce_fused(pp, n, first, count, sum, g->ctx[(size_t)i]->stream));   // peer access was enabled at creation
+        return RT_OK;
+    });
+    if (rc != RT_OK) return rc;
+    const rtb_capi::PresentSrc src = {sum, total, true};
+    rc = rtb_capi::present(c0, fn, out, tp, dn, &src);
+    return rc < 0 ? member_fail(g, 0, rc) : rc;
 }
 
 }  // namespace
@@ -101,7 +185,7 @@ int rt_create_multi(int n_devices, const int* cuda_devices, rt_group** out) {
         cudaEvent_t a = nullptr, b = nullptr;
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&a, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b, cudaEventDisableTiming);
-        g->ev_rendered.push_back(a); g->ev_resolved.push_back(b);
+        g->ev_rendered.push_back(a); g->ev_read.push_back(b);
         if (e != cudaSuccess) return bail(RT_ERR_CUDA, std::string("rt_create_multi: ") + cudaGetErrorString(e));
     }
     *out = g;
@@ -117,7 +201,7 @@ int rt_group_destroy(rt_group* g) {
     for (size_t i = 0; i < g->ctx.size(); ++i) {
         cudaSetDevice(g->ctx[i]->device);
         if (i < g->ev_rendered.size() && g->ev_rendered[i]) cudaEventDestroy(g->ev_rendered[i]);
-        if (i < g->ev_resolved.size() && g->ev_resolved[i]) cudaEventDestroy(g->ev_resolved[i]);
+        if (i < g->ev_read.size() && g->ev_read[i]) cudaEventDestroy(g->ev_read[i]);
         rt_destroy(g->ctx[i]);
     }
     delete g;
@@ -177,42 +261,53 @@ int rt_group_resolve_rgba8(rt_group* g, uint32_t* host_out, int pitch_bytes, int
     if (!g) return RT_ERR_INVALID;
     const int n = (int)g->ctx.size();
     rt_ctx* c0 = g->ctx[0];
-    const int w = c0->par.width, h = c0->par.height;
+    const int w = c0->par.width;
     if (!host_out || pitch_bytes < w * 4) return gfail(g, RT_ERR_INVALID, "rt_group_resolve_rgba8: bad output buffer");
     if (n == 1) {
         const int rc = rt_resolve_rgba8(c0, host_out, pitch_bytes, flip_y);
         return rc < 0 ? member_fail(g, 0, rc) : rc;
     }
-    uint32_t total = 0;
     const void* accum[RT_MAX_PEERS] = {};
-    for (int i = 0; i < n; ++i) {
-        rt_ctx* c = g->ctx[(size_t)i];
-        const int rc = rtb_capi::prepare(c);
-        if (rc != RT_OK) return member_fail(g, i, rc);
-        if (c->par.width != w || c->par.height != h) return gfail(g, RT_ERR_INVALID, "rt_group_resolve_rgba8: members differ in resolution");
-        total += c->samples;
-        accum[i] = c->d_accum.get();
-        RTG_CUDA(g, cudaEventRecord(g->ev_rendered[(size_t)i], c->stream));          // "my samples are in my buffer"
-    }
-    const long long n_px = (long long)w * h;
-    for (int i = 0; i < n; ++i) {
-        rt_ctx* c = g->ctx[(size_t)i];
-        RTG_CUDA(g, cudaSetDevice(c->device));
-        for (int j = 0; j < n; ++j) if (j != i) RTG_CUDA(g, cudaStreamWaitEvent(c->stream, g->ev_rendered[(size_t)j], 0));
-        const int first = (int)(n_px * i / n), count = (int)(n_px * (i + 1) / n) - first;
-        const int rc = rtb_capi::resolve_fused_unchecked(c, accum, n, total, first, count, c0->d_argb.get(), flip_y);   // peer access was enabled at creation
-        if (rc != RT_OK) return member_fail(g, i, rc);
-        RTG_CUDA(g, cudaSetDevice(c->device));
-        RTG_CUDA(g, cudaEventRecord(g->ev_resolved[(size_t)i], c->stream));          // "my slice is written, I have read your buffers"
-    }
-    // nobody touches its buffer again (next reset / render) before every member has read it; member 0 then downloads
-    for (int i = 0; i < n; ++i) {
-        rt_ctx* c = g->ctx[(size_t)i];
-        RTG_CUDA(g, cudaSetDevice(c->device));
-        for (int j = 0; j < n; ++j) if (j != i) RTG_CUDA(g, cudaStreamWaitEvent(c->stream, g->ev_resolved[(size_t)j], 0));
-    }
-    const int rc = rt_read_surface(c0, host_out, pitch_bytes);
+    uint32_t total = 0;
+    int rc = collect(g, "rt_group_resolve_rgba8", accum, total);
+    if (rc != RT_OK) return rc;
+    rc = exchange(g, [&](int i, int first, int count) {
+        const int r = rtb_capi::resolve_fused_unchecked(g->ctx[(size_t)i], accum, n, total, first, count, c0->d_argb.get(), flip_y);   // peer access was enabled at creation
+        return r < 0 ? member_fail(g, i, r) : r;
+    });
+    if (rc != RT_OK) return rc;
+    rc = rt_read_surface(c0, host_out, pitch_bytes);
     return rc < 0 ? member_fail(g, 0, rc) : rc;
+}
+
+int rt_group_denoise_rgba8(rt_group* g, const rt_denoise_params* p, uint32_t* host_out, int pitch_bytes, int flip_y) {
+    rt_denoise_params d;
+    if (!p) rt_default_denoise_params(&d);
+    return group_present(g, "rt_group_denoise_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, nullptr, p ? p : &d);
+}
+
+int rt_group_read_denoised(rt_group* g, const rt_denoise_params* p, float* host_rgba) {
+    rt_denoise_params d;
+    if (!p) rt_default_denoise_params(&d);
+    return group_present(g, "rt_group_read_denoised", {nullptr, 0, 0, host_rgba}, nullptr, p ? p : &d);
+}
+
+// dn NULL: no filter
+int rt_group_temporal_rgba8(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y) {
+    rt_temporal_params d;
+    if (!tp) rt_default_temporal_params(&d);
+    return group_present(g, "rt_group_temporal_rgba8", {host_out, pitch_bytes, flip_y, nullptr}, tp ? tp : &d, dn);
+}
+
+int rt_group_read_temporal(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, float* host_rgba) {
+    rt_temporal_params d;
+    if (!tp) rt_default_temporal_params(&d);
+    return group_present(g, "rt_group_read_temporal", {nullptr, 0, 0, host_rgba}, tp ? tp : &d, dn);
+}
+
+int rt_group_reset_temporal(rt_group* g) {
+    if (!g) return RT_ERR_INVALID;
+    return rt_reset_temporal(g->ctx[0]);                       // the history lives on member 0
 }
 
 int rt_group_get_stats(rt_group* g, rt_stats* out) {

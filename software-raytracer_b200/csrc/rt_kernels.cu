@@ -794,6 +794,21 @@ __global__ void k_resolve_fused(PeerPtrs peers, int world, float count, int widt
     out[(size_t)x + (size_t)(flip_y ? height - 1 - y : y) * width] = resolve_pixel(sum, count);
 }
 
+// ---- fused multi-GPU reduce into one device's buffer (rt_group_denoise_rgba8 / rt_group_temporal_rgba8) ---------------------
+// k_resolve_fused without the resolve: the float4 sum, formed by the same rank-order loop (so resolve_pixel(out[p], total) gives
+// k_resolve_fused's bits), stored at pixel p of `out` (a peer store when it is another device's). 16 B read per rank, 16 B written.
+__global__ void k_reduce_fused(PeerPtrs peers, int world, int first, int n, float4* __restrict__ out) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int p = first + i;
+    float4 sum = peers.p[0][p];
+    for (int r = 1; r < world; ++r) {
+        const float4 v = peers.p[r][p];
+        sum.x += v.x; sum.y += v.y; sum.z += v.z;
+    }
+    out[p] = sum;
+}
+
 // ---- the same with the inter-rank ordering on the device (rt_exchange_resolve; one process per GPU) -------------------------
 // No collective library and no host synchronisation: ranks signal each other through flag words in device memory that the
 // peers have mapped (CUDA IPC over NVLink). Epochs only grow, so nothing is ever reset and a late reader cannot see a stale
@@ -1141,6 +1156,12 @@ cudaError_t launch_resolve_fused(const PeerPtrs& peers, int world, uint32_t samp
                                  int flip_y, uint32_t* out, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     k_resolve_fused<<<(n + 255) / 256, 256, 0, st>>>(peers, world, (float)samples, width, height, first, n, flip_y, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_reduce_fused(const PeerPtrs& peers, int world, int first, int n, float4* out, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    k_reduce_fused<<<(n + 255) / 256, 256, 0, st>>>(peers, world, first, n, out);
     return cudaGetLastError();
 }
 

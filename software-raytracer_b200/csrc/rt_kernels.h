@@ -76,6 +76,9 @@ cudaError_t launch_resolve(const float4* accum, uint32_t samples, int width, int
 
 cudaError_t launch_resolve_fused(const PeerPtrs& peers, int world, uint32_t samples, int width, int height, int first, int n,
                                  int flip_y, uint32_t* out, cudaStream_t st);
+// The sum of launch_resolve_fused, unresolved: pixels [first, first+n) of every rank's buffer added in rank order into out[first ..]
+// (whole-image buffer, y-up like the accumulation buffers).
+cudaError_t launch_reduce_fused(const PeerPtrs& peers, int world, int first, int n, float4* out, cudaStream_t st);
 
 // ---- denoised resolve (rt_denoise.cu; filter in rt_denoise.cuh) ----------------------------------------------------
 // Largest a-trous step whose pass stages its tile + apron in shared memory; larger steps read through L1 (measured: DESIGN.md 8).

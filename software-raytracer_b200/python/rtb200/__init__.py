@@ -87,6 +87,7 @@ EXPORTS = [
     "rt_group_render_spp", "rt_group_resolve_rgba8", "rt_group_get_stats",
     "rt_default_denoise_params", "rt_denoise_rgba8", "rt_read_denoised",
     "rt_default_temporal_params", "rt_temporal_rgba8", "rt_read_temporal", "rt_reset_temporal",
+    "rt_group_denoise_rgba8", "rt_group_read_denoised", "rt_group_temporal_rgba8", "rt_group_read_temporal", "rt_group_reset_temporal",
 ]
 
 
@@ -126,8 +127,12 @@ def load_library(path=None):
     lib.rt_group_last_error.restype = C.c_char_p
     lib.rt_group_last_error.argtypes = [C.c_void_p]
     lib.rt_create_multi.argtypes = [C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]
-    for name in ("rt_group_destroy", "rt_group_size", "rt_group_reset_accumulation"):
+    for name in ("rt_group_destroy", "rt_group_size", "rt_group_reset_accumulation", "rt_group_reset_temporal"):
         getattr(lib, name).argtypes = [C.c_void_p]
+    lib.rt_group_denoise_rgba8.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+    lib.rt_group_read_denoised.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.rt_group_temporal_rgba8.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+    lib.rt_group_read_temporal.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.rt_object_name.restype = C.c_char_p
     lib.rt_object_name.argtypes = [C.c_void_p, C.c_int]
     lib.rt_scene_name.restype = C.c_char_p
@@ -594,6 +599,40 @@ class TracerGroup:
             out = np.zeros((h, w), np.uint32)
         self._chk(self.lib.rt_group_resolve_rgba8(self.g, _p(out), out.strides[0], int(flip_y)))
         return out
+
+    def denoise_rgba8(self, params=None, flip_y=True, out=None):
+        """rt_group_denoise_rgba8: the group's frame with the a-trous filter in front (params None: the library's defaults)."""
+        w, h = self.params.width, self.params.height
+        if out is None:
+            out = np.zeros((h, w), np.uint32)
+        self._chk(self.lib.rt_group_denoise_rgba8(self.g, C.byref(params) if params is not None else None, _p(out), out.strides[0], int(flip_y)))
+        return out
+
+    def read_denoised(self, params=None):
+        """rt_group_read_denoised: the filtered mean radiance of the group's samples, (height, width, 4) float32 (r, g, b, 0), y-up."""
+        w, h = self.params.width, self.params.height
+        out = np.zeros((h, w, 4), np.float32)
+        self._chk(self.lib.rt_group_read_denoised(self.g, C.byref(params) if params is not None else None, _p(out)))
+        return out
+
+    def temporal_rgba8(self, tparams=None, dn=None, flip_y=True, out=None):
+        """rt_group_temporal_rgba8: the group's frame with the reprojected history blended in (dn None: no filter)."""
+        w, h = self.params.width, self.params.height
+        if out is None:
+            out = np.zeros((h, w), np.uint32)
+        self._chk(self.lib.rt_group_temporal_rgba8(self.g, C.byref(tparams) if tparams is not None else None, C.byref(dn) if dn is not None else None,
+                                                   _p(out), out.strides[0], int(flip_y)))
+        return out
+
+    def read_temporal(self, tparams=None, dn=None):
+        """rt_group_read_temporal: (height, width, 4) float32 (r, g, b, N_eff), y-up."""
+        w, h = self.params.width, self.params.height
+        out = np.zeros((h, w, 4), np.float32)
+        self._chk(self.lib.rt_group_read_temporal(self.g, C.byref(tparams) if tparams is not None else None, C.byref(dn) if dn is not None else None, _p(out)))
+        return out
+
+    def reset_temporal(self):
+        self._chk(self.lib.rt_group_reset_temporal(self.g))
 
     def stats(self):
         s = RtStats()
