@@ -296,6 +296,36 @@ int rt_read_temporal(rt_ctx* ctx, const rt_temporal_params* tp, const rt_denoise
 /* Forget the history: the next temporal call presents the plain (or filtered) mean. */
 int rt_reset_temporal(rt_ctx* ctx);
 
+/* Pixel filter: anti-aliased path renders. The reference shoots every sample through the pixel corner (GetRayDirection,
+ * Raytracer.cpp:106-122), so however many samples accumulate, edges stay stair-stepped. With a filter every path-mode sample
+ * traces its own primary ray, offset from the corner by a per-sample (jx, jy) drawn from Philox4x32-10 with counter (pixel, global
+ * sample index, 0, 1) and the context's key: RT_FILTER_BOX uniform on [-radius, radius)^2, RT_FILTER_TENT the separable tent of
+ * that radius. The footprint is centred on the corner, so the image does not shift against the unfiltered one. DESIGN.md 5 states
+ * the arithmetic exactly; a zero offset gives GetRayDirection's bits.
+ *   - rt_set_pixel_filter: RT_ERR_INVALID for an unknown type, a radius that is not finite or not in (0, 4], or nonzero reserved
+ *     words; nothing changes then. NULL = RT_FILTER_NONE, which is the reference's render, bit for bit.
+ *   - Changing the filter does not reset the accumulation (the host decides, as with rt_set_params); it changes the radiance key,
+ *     so a temporal history is dropped.
+ *   - With a filter, path-mode renders run the regeneration megakernel without primary-hit reuse: RT_PIPELINE_AUTO does not time
+ *     the wavefront or streaming pipelines, and RT_PIPELINE_WAVEFRONT / RT_PIPELINE_STREAM or RT_OPT_BVH_SCHED 1 render with the
+ *     megakernel too (rt_stats.pipeline reports RT_PIPELINE_REGEN). traced_segments == segments for such renders, plus the
+ *     primary-hit cache pass when the cache is traced as a guide.
+ *   - Preview mode and block-filled frames (rt_set_pixel_step > 1) ignore the filter: they are the reference's coarse interaction
+ *     frames. rt_pick, rt_read_aov, rt_read_ray_dirs and the primary-hit cache stay the unjittered corner rays, so the denoised,
+ *     temporal and group resolves work unchanged on an anti-aliased buffer, guided by the corner rays. */
+enum { RT_FILTER_NONE = 0, RT_FILTER_BOX = 1, RT_FILTER_TENT = 2 };
+typedef struct {
+    int32_t type;           /* RT_FILTER_* */
+    float radius;           /* half-width of the footprint in pixels, (0, 4] */
+    int32_t reserved[2];    /* 0 */
+} rt_pixel_filter;          /* 16 bytes */
+void rt_default_pixel_filter(rt_pixel_filter* f);                  /* RT_FILTER_NONE, radius 0.5 (the box's natural width) */
+int rt_set_pixel_filter(rt_ctx* ctx, const rt_pixel_filter* f);    /* NULL = none */
+int rt_get_pixel_filter(rt_ctx* ctx, rt_pixel_filter* out);
+/* The primary direction of global sample `sample` for every pixel (width*height*3 floats, y-up), from the same device function
+ * the render kernels use; with RT_FILTER_NONE rt_read_ray_dirs' corner rays. */
+int rt_read_sample_dirs(rt_ctx* ctx, uint32_t sample, float* dirs);
+
 /* Page-locked host memory for the surface handed to rt_resolve_rgba8 / rt_read_surface: the device-to-host copy
  * then runs as one DMA instead of being staged by the driver (1280x720 frame loop: 0.30 ms instead of 0.44 ms per
  * frame). Any host pointer works; this is only faster. */
@@ -430,6 +460,7 @@ int rt_group_read_denoised(rt_group* g, const rt_denoise_params* p, float* host_
 int rt_group_temporal_rgba8(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, uint32_t* host_out, int pitch_bytes, int flip_y);
 int rt_group_read_temporal(rt_group* g, const rt_temporal_params* tp, const rt_denoise_params* dn, float* host_rgba);
 int rt_group_reset_temporal(rt_group* g);
+int rt_group_set_pixel_filter(rt_group* g, const rt_pixel_filter* f);   /* rt_set_pixel_filter on every member */
 int rt_group_get_stats(rt_group* g, rt_stats* out);           /* sums over the members; last_render_ms = the slowest */
 
 #ifdef __cplusplus

@@ -776,6 +776,35 @@ int rt_reference_pixel_step(float screen_scale, float progressive_scaler) {
 
 int rt_reference_strip_columns(int width) { return (int)ceil(width / 16) + 1; }   // Raytracer.cpp:28,330 (integer division first)
 
+void rt_default_pixel_filter(rt_pixel_filter* f) {
+    if (!f) return;
+    memset(f, 0, sizeof *f);
+    f->type = RT_FILTER_NONE; f->radius = 0.5f;
+}
+
+int rt_set_pixel_filter(rt_ctx* c, const rt_pixel_filter* f) {
+    if (!c) return RT_ERR_INVALID;
+    rt_pixel_filter v;
+    rt_default_pixel_filter(&v);
+    if (f) {
+        if (f->type != RT_FILTER_NONE && f->type != RT_FILTER_BOX && f->type != RT_FILTER_TENT)
+            return fail(c, RT_ERR_INVALID, "rt_set_pixel_filter: type takes RT_FILTER_NONE / BOX / TENT");
+        if (!(std::isfinite(f->radius) && f->radius > 0.f && f->radius <= 4.f))
+            return fail(c, RT_ERR_INVALID, "rt_set_pixel_filter: radius must be finite and in (0, 4]");
+        if (f->reserved[0] != 0 || f->reserved[1] != 0) return fail(c, RT_ERR_INVALID, "rt_set_pixel_filter: reserved words must be 0");
+        v = *f;
+    }
+    if (memcmp(&v, &c->filter, sizeof v) != 0) ++c->radiance_key;   // the expected radiance of a pixel changes: a temporal history ends
+    c->filter = v;
+    return RT_OK;
+}
+
+int rt_get_pixel_filter(rt_ctx* c, rt_pixel_filter* out) {
+    if (!c || !out) return RT_ERR_INVALID;
+    *out = c->filter;
+    return RT_OK;
+}
+
 int rt_set_shard(rt_ctx* c, int rank, int world) {
     if (!c || world < 1 || rank < 0 || rank >= world) return fail(c, RT_ERR_INVALID, "rt_set_shard: bad rank/world");
     c->rank = rank; c->world = world;
@@ -816,7 +845,10 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
     AccelSel ac;
     if ((rc = make_accel(c, want_accel(c), camera_extent(c), ac)) != RT_OK) return rc;
     c->used_accel = accel_of(ac);
-    if (c->par.mode == RT_MODE_PATH && (rc = autotune_pipeline(c, ac, spp)) != RT_OK) return rc;
+    // a pixel filter applies to full-resolution path renders, which then run the megakernel's jittered forms (rt_set_pixel_filter)
+    const bool filtered = c->filter.type != RT_FILTER_NONE && c->par.mode == RT_MODE_PATH && c->pixel_step == 1;
+    const PixelFilter pf = {c->filter.type, c->filter.radius};
+    if (c->par.mode == RT_MODE_PATH && !filtered && (rc = autotune_pipeline(c, ac, spp)) != RT_OK) return rc;
     RT_CUDA(c, cudaEventRecord(c->ev0, c->stream));
     if (c->pixel_step > 1) {
         // SCREEN_SCALE / progressive resolution: one path per block, block-filled (Raytracer.cpp:233-248)
@@ -842,14 +874,15 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
         // this rank's slice of the global sample indices [next, next+spp)
         int mine = 0; uint32_t first = 0;
         rt_shard_range(spp, c->rank, c->world, c->next_sample, &first, &mine);
-        const int pipe = c->opt_pipeline != RT_PIPELINE_AUTO ? c->opt_pipeline : (c->tuned_pipeline > 0 && mine >= kWavefrontMinSpp ? c->tuned_pipeline : RT_PIPELINE_REGEN);
+        const int pipe = filtered ? RT_PIPELINE_REGEN
+                       : c->opt_pipeline != RT_PIPELINE_AUTO ? c->opt_pipeline : (c->tuned_pipeline > 0 && mine >= kWavefrontMinSpp ? c->tuned_pipeline : RT_PIPELINE_REGEN);
         // the streaming kernel walks the binary BVH only; for other back ends RT_PIPELINE_STREAM runs the bounce-round kernels
         const bool streaming = pipe == RT_PIPELINE_STREAM && ac.kind == kAccelBvh && !ac.bvh.wnodes && c->opt_bvh_sched == 0;
         bool wavefront = (pipe == RT_PIPELINE_WAVEFRONT || pipe == RT_PIPELINE_STREAM) &&
                          (streaming || c->par.max_bounces <= 60);   // bounce rounds: one queue counter per round; deeper paths use the megakernel
-        const bool scheduled = !wavefront && ac.kind == kAccelBvh && c->opt_bvh_sched && c->view.n_tri == 0;   // experimental kernel, re-traces primaries
+        const bool scheduled = !wavefront && !filtered && ac.kind == kAccelBvh && c->opt_bvh_sched && c->view.n_tri == 0;   // experimental kernel, re-traces primaries
         PrimCache pc;
-        if (c->opt_primary_reuse && !scheduled && mine > 0 && (rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
+        if (c->opt_primary_reuse && !scheduled && !filtered && mine > 0 && (rc = ensure_prim_cache(c, ac)) != RT_OK) return rc;
         const PrimCache* prim = prim_cache_arg(c, pc);
         if (wavefront) {
             if (!c->wf) c->wf = wavefront_create();
@@ -872,7 +905,7 @@ static int render_samples(rt_ctx* c, int spp, FrameTarget* frame) {
             if (frame) frame->samples_after = c->samples + (uint32_t)mine;
             RT_CUDA(c, launch_render_regen(c->view, ac, c->frame, c->d_accum.get(), first, mine, prim, c->d_counters.get(), c->stream, c->opt_pool_tiles,
                                            c->opt_flat_coop == 2 ? (c->opt_accel == RT_ACCEL_AUTO ? c->tuned_flat_coop != 0 : c->view.n_box == 0) : c->opt_flat_coop != 0,
-                                           c->opt_trav_stats != 0, c->world == 1 && mine > 0 ? frame : nullptr));
+                                           c->opt_trav_stats != 0, c->world == 1 && mine > 0 ? frame : nullptr, filtered ? &pf : nullptr));
         }
         if (!wavefront) c->used_pipeline = RT_PIPELINE_REGEN;
         c->next_sample += (uint32_t)spp;
@@ -1168,6 +1201,20 @@ int rt_read_ray_dirs(rt_ctx* c, float* dirs) {
     if (e == cudaSuccess) e = cudaMemcpyAsync(dirs, d.get(), px * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
     if (e != cudaSuccess) return cuda_fail(c, e, "rt_read_ray_dirs");
+    return RT_OK;
+}
+
+int rt_read_sample_dirs(rt_ctx* c, uint32_t sample, float* dirs) {
+    int rc = prepare(c);
+    if (rc != RT_OK) return rc;
+    if (!dirs) return fail(c, RT_ERR_INVALID, "rt_read_sample_dirs: NULL output");
+    const size_t px = (size_t)c->par.width * c->par.height;
+    DeviceArray<float> d;
+    cudaError_t e = d.reserve(px * 3);
+    if (e == cudaSuccess) e = launch_sample_dirs(c->frame, PixelFilter{c->filter.type, c->filter.radius}, sample, d.get(), c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dirs, d.get(), px * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) return cuda_fail(c, e, "rt_read_sample_dirs");
     return RT_OK;
 }
 

@@ -104,6 +104,7 @@ struct rt_ctx {
     uint64_t paths = 0, total_paths = 0, total_segments_base = 0;
     int rank = 0, world = 1;
     int pixel_step = 1, strip_columns = 0;   // block-filled frames (rt_set_pixel_step)
+    rt_pixel_filter filter = {RT_FILTER_NONE, 0.5f, {0, 0}};   // rt_set_pixel_filter
     int opt_pipeline = RT_PIPELINE_AUTO, opt_accel = RT_ACCEL_AUTO, opt_bvh_threshold = 512;
     int opt_bvh_sched = 0, opt_bvh_wait_k = 20, opt_bvh_leaf = 4, opt_primary_reuse = 1;
     int opt_trav_stats = 0;            // RT_OPT_TRAVERSAL_STATS

@@ -237,6 +237,11 @@ int rt_group_set_params(rt_group* g, const rt_params* p) {
     return for_members(g, false, [&](int i) { return rt_set_params(g->ctx[(size_t)i], p); });
 }
 
+int rt_group_set_pixel_filter(rt_group* g, const rt_pixel_filter* f) {
+    if (!g) return RT_ERR_INVALID;
+    return for_members(g, false, [&](int i) { return rt_set_pixel_filter(g->ctx[(size_t)i], f); });
+}
+
 int rt_group_set_option(rt_group* g, int option, int value) {
     if (!g) return RT_ERR_INVALID;
     return for_members(g, false, [&](int i) { return rt_set_option(g->ctx[(size_t)i], option, value); });

@@ -10,6 +10,7 @@
 #include <mutex>
 
 #include "rt_device.cuh"
+#include "rt_filter.cuh"
 #include "rt_resolve.cuh"
 #include "rt_trace.cuh"
 
@@ -47,6 +48,15 @@ __global__ void k_ray_dirs(FrameView fr, float* __restrict__ out) {
     float3 d = ray_dir(fr, px, py);
     size_t p = (size_t)px + (size_t)py * fr.width;
     out[3 * p] = d.x; out[3 * p + 1] = d.y; out[3 * p + 2] = d.z;
+}
+
+// rt_read_sample_dirs: the primary direction of global sample `sample` of every pixel, as the jittered render kernels draw it
+__global__ void k_sample_dirs(FrameView fr, PixelFilter pf, uint32_t sample, float* __restrict__ out) {
+    int px = blockIdx.x * blockDim.x + threadIdx.x, py = blockIdx.y;
+    if (px >= fr.width) return;
+    const uint32_t pixel = (uint32_t)px + (uint32_t)py * (uint32_t)fr.width;
+    float3 d = filtered_ray_dir(fr, pf, px, py, pixel, sample);
+    out[3 * (size_t)pixel] = d.x; out[3 * (size_t)pixel + 1] = d.y; out[3 * (size_t)pixel + 2] = d.z;
 }
 
 template <int MODE, bool COUNT = false>
@@ -216,10 +226,14 @@ __global__ void k_philox(uint4 ctr, uint2 key, uint4* out) { *out = philox4x32_1
 // across the closest-hit query, which brings the kernel to 72 registers = 7 CTAs per SM. The stash costs 1.5 % at equal occupancy and
 // the seventh CTA gives 4 %: Scene1 1080p 1024 spp 108.2 -> 105.5 ms; a 640x480 launch (2400 CTAs: 2.3 instead of 2.7 waves, the last
 // as long and emptier) loses 4 %, so the launcher takes this form for large grids only (profiles/r4u_ab_stash.txt). Same bits.
-template <int MODE, bool REUSE, bool COUNT = false, bool STASH = false>
-__global__ void __launch_bounds__(kThreads, STASH ? RTB_REGEN_STASH_BLOCKS : RTB_REGEN_MIN_BLOCKS) k_render_regen(SceneView sc, BvhView bv, FlatView fl, FrameView fr, float4* __restrict__ accum,
-                                                            uint32_t s_begin, int n_samples, PrimCache prim,
-                                                            unsigned long long* __restrict__ seg_counter) {
+//
+// JITTER (a pixel filter, rt_filter.cuh; never with REUSE): every sample starts from its own primary direction, filtered_ray_dir() of its
+// global sample index, instead of the pixel's corner ray d0 - the non-reuse loop with a different d0. k_render_regen_aa below.
+template <int MODE, bool REUSE, bool COUNT, bool STASH, bool JITTER>
+__device__ __forceinline__ void render_regen(const SceneView& sc, const BvhView& bv, const FlatView& fl, const FrameView& fr, float4* __restrict__ accum,
+                                             uint32_t s_begin, int n_samples, const PrimCache& prim, unsigned long long* __restrict__ seg_counter,
+                                             const PixelFilter& pf) {
+    static_assert(!(JITTER && REUSE), "a jittered primary ray is not the cached one");
     extern __shared__ float4 smem[];
     const TraceCtx tc = setup_trace<MODE>(sc, bv, fl, smem);
     int px, py;
@@ -227,9 +241,9 @@ __global__ void __launch_bounds__(kThreads, STASH ? RTB_REGEN_STASH_BLOCKS : RTB
     const uint32_t pixel = inside ? (uint32_t)px + (uint32_t)py * (uint32_t)fr.width : 0u;
     if (!inside) n_samples = 0;
 
-    const float3 d0 = ray_dir(fr, px, py);
+    const float3 d0 = JITTER ? f3(0.f, 0.f, 0.f) : ray_dir(fr, px, py);
     float3 acc = f3(0.f, 0.f, 0.f);
-    float3 o = fr.cam_pos, d = d0;
+    float3 o = fr.cam_pos, d = JITTER ? filtered_ray_dir(fr, pf, px, py, pixel, s_begin) : d0;
     float3 T = f3(0.f, 0.f, 0.f), L = f3(0.f, 0.f, 0.f);
     int s = 0, depth = 0;
     unsigned int segs = 0, traced = 0;
@@ -280,7 +294,7 @@ __global__ void __launch_bounds__(kThreads, STASH ? RTB_REGEN_STASH_BLOCKS : RTB
                         ++segs; scatter = true;
                     }
                 } else {
-                    d = d0;
+                    d = JITTER ? filtered_ray_dir(fr, pf, px, py, pixel, s_begin + (uint32_t)s) : d0;
                     if (REUSE && s < n_samples) { h = h0; ++segs; scatter = true; }   // next sample starts from the cached primary hit
                 }
             }
@@ -306,6 +320,19 @@ __global__ void __launch_bounds__(kThreads, STASH ? RTB_REGEN_STASH_BLOCKS : RTB
         atomicAdd(seg_counter + 2, (unsigned long long)total_tr); atomicAdd(seg_counter + 3, (unsigned long long)total_tr);
     }
     if (COUNT) flush_trav_count(cnt, traced, seg_counter);
+}
+template <int MODE, bool REUSE, bool COUNT = false, bool STASH = false>
+__global__ void __launch_bounds__(kThreads, STASH ? RTB_REGEN_STASH_BLOCKS : RTB_REGEN_MIN_BLOCKS) k_render_regen(SceneView sc, BvhView bv, FlatView fl, FrameView fr, float4* __restrict__ accum,
+                                                            uint32_t s_begin, int n_samples, PrimCache prim,
+                                                            unsigned long long* __restrict__ seg_counter) {
+    render_regen<MODE, REUSE, COUNT, STASH, false>(sc, bv, fl, fr, accum, s_begin, n_samples, prim, seg_counter, PixelFilter{kFilterNone, 0.f});
+}
+// the same loop with a pixel filter: one jittered primary ray per sample (no primary-hit reuse)
+template <int MODE, bool COUNT = false>
+__global__ void __launch_bounds__(kThreads, RTB_REGEN_MIN_BLOCKS) k_render_regen_aa(SceneView sc, BvhView bv, FlatView fl, FrameView fr, float4* __restrict__ accum,
+                                                                                    uint32_t s_begin, int n_samples,
+                                                                                    unsigned long long* __restrict__ seg_counter, PixelFilter pf) {
+    render_regen<MODE, false, COUNT, false, true>(sc, bv, fl, fr, accum, s_begin, n_samples, PrimCache{nullptr, nullptr}, seg_counter, pf);
 }
 
 // ---- resolve: sum/count -> Reinhard -> truncating ARGB8 pack (Raytracer.cpp:73-75): resolve_pixel() in rt_resolve.cuh ----------
@@ -361,144 +388,164 @@ static __device__ __noinline__ void pool_chunk_out(const float4* accum, uint32_t
         }
     }
 }
+// The pixel-pool loop as the body of k_render_pool (JITTER false) and k_render_pool_aa (JITTER true: every sample of a pixel starts from
+// its own filtered_ray_dir(), rt_filter.cuh, instead of the pixel's d0; no primary-hit reuse). A macro rather than a device function: inlined
+// from a device function, the loop of the existing kernels came out with a different register allocation (the same result, other SASS).
+// Expects the kernel parameters below and `pf` in scope.
+#define RTB_RENDER_POOL_BODY(JITTER)                                                                                                                                                                                \
+    extern __shared__ float4 smem[];                                                                                                                                                                                \
+    const TraceCtx tc = setup_trace<MODE>(sc, bv, fl, smem);                                                                                                                                                        \
+    constexpr unsigned FULL = 0xffffffffu;                                                                                                                                                                          \
+    const int lane = threadIdx.x & 31;                                                                                                                                                                              \
+    const int tiles_x = (fr.width + kPoolTW - 1) / kPoolTW, tiles_y = (fr.height + kPoolTH - 1) / kPoolTH;                                                                                                          \
+    const unsigned int n_tiles = (unsigned int)tiles_x * (unsigned int)tiles_y;                                                                                                                                     \
+    /* frame output (FRAME: its own instantiation, the bookkeeping costs registers; requires pool_tiles <= 2): see FrameOut */                                                                                      \
+    constexpr bool fuse = FRAME;                                                                                                                                                                                    \
+    unsigned int* const chunk_tile = reinterpret_cast<unsigned int*>(reinterpret_cast<unsigned char*>(smem) + fo.smem_off) + (threadIdx.x >> 5) * kPoolSlots;                                                       \
+    unsigned long long left8 = 0ull;                          /* pixels not yet finished of the chunks in flight, byte (seq % kPoolSlots) */                                                                        \
+    int seq_cur = -1, my_seq = 0;                             /* chunks are numbered per warp in claim order */                                                                                                     \
+    /* a lane can finish two pixels in one pass: the one it was tracing, and a fresh one whose primary ray misses (or a chunk slot */                                                                               \
+    /* outside the image): the chunk numbers of both, -1 = none */                                                                                                                                                  \
+    int fin_a = -1, fin_b = -1;                                                                                                                                                                                     \
+    uint32_t pixel = 0;                                       /* the lane's current pixel */                                                                                                                        \
+    /* end of a pass: the finished pixels leave their chunks' counts; a chunk that reaches zero is resolved and sent (ONE call site) */                                                                             \
+    auto retire = [&]() {                                                                                                                                                                                           \
+_Pragma("unroll 1")                                                                                                                                                                                                    \
+        for (int e = 0; e < 2; ++e) {                                                                                                                                                                               \
+            const int mine = e ? fin_b : fin_a;                                                                                                                                                                     \
+            unsigned m_fin = __ballot_sync(FULL, mine >= 0);                                                                                                                                                        \
+            while (m_fin) {                                                                                                                                                                                         \
+                const int sq = __shfl_sync(FULL, mine, __ffs((int)m_fin) - 1);                                                                                                                                      \
+                const unsigned same = __ballot_sync(FULL, mine == sq);                                                                                                                                              \
+                m_fin &= ~same;                                                                                                                                                                                     \
+                const int sh = 8 * (sq & (kPoolSlots - 1));                                                                                                                                                         \
+                left8 -= (unsigned long long)__popc(same) << sh;                                                                                                                                                    \
+                if (((left8 >> sh) & 0xffull) == 0ull) {                                                                                                                                                            \
+                    __syncwarp();                            /* the chunk's sums were written by lanes of this warp */                                                                                              \
+                    pool_chunk_out(accum, fo.out, fo.out2, fo.count, fo.flip_y, fr.width, fr.height, tiles_x, n_tiles, pool_tiles, chunk_tile[sq & (kPoolSlots - 1)], lane);                                        \
+                }                                                                                                                                                                                                   \
+            }                                                                                                                                                                                                       \
+        }                                                                                                                                                                                                           \
+        fin_a = -1; fin_b = -1;                                                                                                                                                                                     \
+    };                                                                                                                                                                                                              \
+    /* the warp's current chunk of `pool_tiles` tiles, claimed from the launch's cursor; the NEXT chunk is requested as soon as */                                                                                  \
+    /* the current one is half handed out, so the atomic's round trip overlaps the tracing (its result is first read when needed) */                                                                                \
+    unsigned int tile0 = 0, claimed = 0;                                                    /* warp-uniform */                                                                                                      \
+    int next = 0, total = 0;                                                                                                                                                                                        \
+    bool have_claim = false, drained = false;                                                                                                                                                                       \
+    bool busy = false;                                                                                                                                                                                              \
+    float3 d0 = f3(0.f, 0.f, 1.f), acc = f3(0.f, 0.f, 0.f), o = fr.cam_pos, d = d0;                                                                                                                                 \
+    float3 T = f3(0.f, 0.f, 0.f), L = f3(0.f, 0.f, 0.f);                                                                                                                                                            \
+    int s = 0, depth = 0;                                                                                                                                                                                           \
+    unsigned int segs = 0, traced = 0;                                                                                                                                                                              \
+    Hit h0;                                                                                                                                                                                                         \
+    h0.id = -1; h0.t = 0.f; h0.n = f3(0.f, 0.f, 0.f); h0.p = f3(0.f, 0.f, 0.f);                                                                                                                                     \
+                                                                                                                                                                                                                    \
+    /* One iteration: closest hit for the lanes that hold a ray -> end-of-path handling -> idle lanes (also those that finished a pixel */                                                                          \
+    /* just now) take the next pixels of the chunk -> ONE scatter block for continuing paths, restarted samples and fresh pixels. */                                                                                \
+    /* (The first version scattered fresh pixels inside the pick-up: a second copy of the scatter code that ran in almost every */                                                                                  \
+    /* iteration for the handful of lanes that had just taken a pixel.) */                                                                                                                                          \
+    for (;;) {                                                                                                                                                                                                      \
+        Hit h = trace_all<MODE>(sc, tc, o, d, busy);                                                                                                                                                                \
+        bool scat = false;                                                                                                                                                                                          \
+        if (busy) {                                                                                                                                                                                                 \
+            ++segs; ++traced;                                                                                                                                                                                       \
+            float3 c;                                                                                                                                                                                               \
+            if (path_ends(sc, fr, h, d, T, L, depth, c)) {                                                                                                                                                          \
+                acc.x += c.x; acc.y += c.y; acc.z += c.z;                                                                                                                                                           \
+                ++s; depth = 0; o = fr.cam_pos; d = d0;     /* no reuse: the next iteration traces the primary ray again */                                                                                         \
+                if (JITTER && s < n_samples) d = filtered_ray_dir(fr, pf, (int)(pixel % (uint32_t)fr.width), (int)(pixel / (uint32_t)fr.width), pixel, s_begin + (uint32_t)s);                                      \
+                if (s >= n_samples) {                                                                                                                                                                               \
+                    float4 a = accum[pixel];                                                                                                                                                                        \
+                    a.x += acc.x; a.y += acc.y; a.z += acc.z;                                                                                                                                                       \
+                    accum[pixel] = a;                                                                                                                                                                               \
+                    if (fuse) fin_a = my_seq;                                                                                                                                                                       \
+                    busy = false;                                                                                                                                                                                   \
+                } else if (REUSE) { h = h0; ++segs; scat = true; }     /* next sample from the cached primary hit */                                                                                                \
+            } else scat = true;                                                                                                                                                                                     \
+        }                                                                                                                                                                                                           \
+        const unsigned m_need = __ballot_sync(FULL, !busy);                                                                                                                                                         \
+        if (!have_claim && !drained && 2 * next >= total) {  /* ask for the next chunk early */                                                                                                                     \
+            if (lane == 0) claimed = atomicAdd(tile_cursor, (unsigned int)pool_tiles);                                                                                                                              \
+            have_claim = true;                                                                                                                                                                                      \
+        }                                                                                                                                                                                                           \
+        /* (frame output: the chunk kPoolSlots claims back must be complete before its bookkeeping slot is used again - else wait a pass. */                                                                        \
+        /* With 4 slots that happened often enough - one deep path under 31 lanes racing through sky chunks - to cost 15 % of the kernel.) */                                                                       \
+        if (m_need != 0u && next >= total && have_claim && !(fuse && ((left8 >> (8 * ((seq_cur + 1) & (kPoolSlots - 1)))) & 0xffull) != 0ull)) {   /* the current chunk is handed out: switch to the claimed one */ \
+            tile0 = __shfl_sync(FULL, claimed, 0);                                                                                                                                                                  \
+            have_claim = false;                                                                                                                                                                                     \
+            if (tile0 >= n_tiles) { drained = true; total = 0; }                                                                                                                                                    \
+            else { const unsigned int rem = n_tiles - tile0; total = (int)(rem < (unsigned int)pool_tiles ? rem : (unsigned int)pool_tiles) * 32; }                                                                 \
+            next = 0;                                                                                                                                                                                               \
+            if (fuse && total > 0) {                                                                                                                                                                                \
+                ++seq_cur;                                                                                                                                                                                          \
+                left8 += (unsigned long long)total << (8 * (seq_cur & (kPoolSlots - 1)));                                                                                                                           \
+                if (lane == 0) chunk_tile[seq_cur & (kPoolSlots - 1)] = tile0;                                                                                                                                      \
+            }                                                                                                                                                                                                       \
+        }                                                                                                                                                                                                           \
+        if (m_need != 0u && next < total) {                                                                                                                                                                         \
+            const int idx = next + __popc(m_need & ((1u << lane) - 1u));                                                                                                                                            \
+            next += __popc(m_need);                                                                                                                                                                                 \
+            if (!busy && idx < total) {                                                                                                                                                                             \
+                const unsigned int tile = tile0 + (unsigned int)(idx >> 5);                                                                                                                                         \
+                const int px = (int)(tile % (unsigned int)tiles_x) * kPoolTW + (idx % kPoolTW), py = (int)(tile / (unsigned int)tiles_x) * kPoolTH + ((idx & 31) / kPoolTW);                                        \
+                if (fuse) { my_seq = seq_cur; if (!(px < fr.width && py < fr.height)) fin_b = my_seq; }   /* nothing to trace for this slot of the chunk */                                                         \
+                if (px < fr.width && py < fr.height) {                                                                                                                                                              \
+                    pixel = (uint32_t)px + (uint32_t)py * (uint32_t)fr.width;                                                                                                                                       \
+                    d0 = JITTER ? filtered_ray_dir(fr, pf, px, py, pixel, s_begin) : ray_dir(fr, px, py);                                                                                                           \
+                    acc = f3(0.f, 0.f, 0.f); o = fr.cam_pos; d = d0; s = 0; depth = 0;                                                                                                                              \
+                    busy = true;                                                                                                                                                                                    \
+                    if (REUSE) {                                                                                                                                                                                    \
+                        h0 = cached_primary(prim, pixel, o, d);                                                                                                                                                     \
+                        float3 c;                                                                                                                                                                                   \
+                        if (primary_ends(sc, fr, h0, c)) {                                                                                                                                                          \
+                            /* the primary ray misses (or max_bounces == 0): every sample of the pixel has the value c */                                                                                           \
+                            for (; s < n_samples; ++s) { acc.x += c.x; acc.y += c.y; acc.z += c.z; }                                                                                                                \
+                            segs += (unsigned int)n_samples;                                                                                                                                                        \
+                            float4 a = accum[pixel];                                                                                                                                                                \
+                            a.x += acc.x; a.y += acc.y; a.z += acc.z;                                                                                                                                               \
+                            accum[pixel] = a;                                                                                                                                                                       \
+                            if (fuse) fin_b = my_seq;                                                                                                                                                               \
+                            busy = false;                    /* takes another pixel in the next pass */                                                                                                             \
+                        } else { h = h0; ++segs; scat = true; }                                                                                                                                                     \
+                    }                                                                                                                                                                                               \
+                }                                                                                                                                                                                                   \
+            }                                                                                                                                                                                                       \
+        }                                                                                                                                                                                                           \
+        if (fuse) retire();                                                                                                                                                                                         \
+        if (scat) scatter_segment(sc, fr, h, pixel, s_begin + (uint32_t)s, o, d, T, L, depth);                                                                                                                      \
+        if (!__any_sync(FULL, busy) && drained) break;      /* not drained: the next pass switches to the claimed chunk */                                                                                          \
+    }                                                                                                                                                                                                               \
+                                                                                                                                                                                                                    \
+    unsigned int total_s = segs, total_tr = traced;                                                                                                                                                                 \
+_Pragma("unroll")                                                                                                                                                                                                   \
+    for (int off = 16; off > 0; off >>= 1) {                                                                                                                                                                        \
+        total_s += __shfl_down_sync(FULL, total_s, off);                                                                                                                                                            \
+        total_tr += __shfl_down_sync(FULL, total_tr, off);                                                                                                                                                          \
+    }                                                                                                                                                                                                               \
+    if (lane == 0 && total_s) {                                                                                                                                                                                     \
+        atomicAdd(seg_counter, (unsigned long long)total_s); atomicAdd(seg_counter + 1, (unsigned long long)total_s);                                                                                               \
+        atomicAdd(seg_counter + 2, (unsigned long long)total_tr); atomicAdd(seg_counter + 3, (unsigned long long)total_tr);                                                                                         \
+    }                                                                                                                                                                                                               \
+
 template <int MODE, bool REUSE, bool FRAME>
 __global__ void __launch_bounds__(kThreads, RTB_REGEN_MIN_BLOCKS) k_render_pool(SceneView sc, BvhView bv, FlatView fl, FrameView fr, float4* __restrict__ accum,
                                                            uint32_t s_begin, int n_samples, int pool_tiles, PrimCache prim,
                                                            unsigned int* __restrict__ tile_cursor, unsigned long long* __restrict__ seg_counter, FrameOut fo) {
-    extern __shared__ float4 smem[];
-    const TraceCtx tc = setup_trace<MODE>(sc, bv, fl, smem);
-    constexpr unsigned FULL = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const int tiles_x = (fr.width + kPoolTW - 1) / kPoolTW, tiles_y = (fr.height + kPoolTH - 1) / kPoolTH;
-    const unsigned int n_tiles = (unsigned int)tiles_x * (unsigned int)tiles_y;
-    // frame output (FRAME: its own instantiation, the bookkeeping costs registers; requires pool_tiles <= 2): see FrameOut
-    constexpr bool fuse = FRAME;
-    unsigned int* const chunk_tile = reinterpret_cast<unsigned int*>(reinterpret_cast<unsigned char*>(smem) + fo.smem_off) + (threadIdx.x >> 5) * kPoolSlots;
-    unsigned long long left8 = 0ull;                          // pixels not yet finished of the chunks in flight, byte (seq % kPoolSlots)
-    int seq_cur = -1, my_seq = 0;                             // chunks are numbered per warp in claim order
-    // a lane can finish two pixels in one pass: the one it was tracing, and a fresh one whose primary ray misses (or a chunk slot
-    // outside the image): the chunk numbers of both, -1 = none
-    int fin_a = -1, fin_b = -1;
-    uint32_t pixel = 0;                                       // the lane's current pixel
-    // end of a pass: the finished pixels leave their chunks' counts; a chunk that reaches zero is resolved and sent (ONE call site)
-    auto retire = [&]() {
-#pragma unroll 1
-        for (int e = 0; e < 2; ++e) {
-            const int mine = e ? fin_b : fin_a;
-            unsigned m_fin = __ballot_sync(FULL, mine >= 0);
-            while (m_fin) {
-                const int sq = __shfl_sync(FULL, mine, __ffs((int)m_fin) - 1);
-                const unsigned same = __ballot_sync(FULL, mine == sq);
-                m_fin &= ~same;
-                const int sh = 8 * (sq & (kPoolSlots - 1));
-                left8 -= (unsigned long long)__popc(same) << sh;
-                if (((left8 >> sh) & 0xffull) == 0ull) {
-                    __syncwarp();                            // the chunk's sums were written by lanes of this warp
-                    pool_chunk_out(accum, fo.out, fo.out2, fo.count, fo.flip_y, fr.width, fr.height, tiles_x, n_tiles, pool_tiles, chunk_tile[sq & (kPoolSlots - 1)], lane);
-                }
-            }
-        }
-        fin_a = -1; fin_b = -1;
-    };
-    // the warp's current chunk of `pool_tiles` tiles, claimed from the launch's cursor; the NEXT chunk is requested as soon as
-    // the current one is half handed out, so the atomic's round trip overlaps the tracing (its result is first read when needed)
-    unsigned int tile0 = 0, claimed = 0;                                                    // warp-uniform
-    int next = 0, total = 0;
-    bool have_claim = false, drained = false;
-    bool busy = false;
-    float3 d0 = f3(0.f, 0.f, 1.f), acc = f3(0.f, 0.f, 0.f), o = fr.cam_pos, d = d0;
-    float3 T = f3(0.f, 0.f, 0.f), L = f3(0.f, 0.f, 0.f);
-    int s = 0, depth = 0;
-    unsigned int segs = 0, traced = 0;
-    Hit h0;
-    h0.id = -1; h0.t = 0.f; h0.n = f3(0.f, 0.f, 0.f); h0.p = f3(0.f, 0.f, 0.f);
-
-    // One iteration: closest hit for the lanes that hold a ray -> end-of-path handling -> idle lanes (also those that finished a pixel
-    // just now) take the next pixels of the chunk -> ONE scatter block for continuing paths, restarted samples and fresh pixels.
-    // (The first version scattered fresh pixels inside the pick-up: a second copy of the scatter code that ran in almost every
-    // iteration for the handful of lanes that had just taken a pixel.)
-    for (;;) {
-        Hit h = trace_all<MODE>(sc, tc, o, d, busy);
-        bool scat = false;
-        if (busy) {
-            ++segs; ++traced;
-            float3 c;
-            if (path_ends(sc, fr, h, d, T, L, depth, c)) {
-                acc.x += c.x; acc.y += c.y; acc.z += c.z;
-                ++s; depth = 0; o = fr.cam_pos; d = d0;     // no reuse: the next iteration traces the primary ray again
-                if (s >= n_samples) {
-                    float4 a = accum[pixel];
-                    a.x += acc.x; a.y += acc.y; a.z += acc.z;
-                    accum[pixel] = a;
-                    if (fuse) fin_a = my_seq;
-                    busy = false;
-                } else if (REUSE) { h = h0; ++segs; scat = true; }     // next sample from the cached primary hit
-            } else scat = true;
-        }
-        const unsigned m_need = __ballot_sync(FULL, !busy);
-        if (!have_claim && !drained && 2 * next >= total) {  // ask for the next chunk early
-            if (lane == 0) claimed = atomicAdd(tile_cursor, (unsigned int)pool_tiles);
-            have_claim = true;
-        }
-        // (frame output: the chunk kPoolSlots claims back must be complete before its bookkeeping slot is used again - else wait a pass.
-        // With 4 slots that happened often enough - one deep path under 31 lanes racing through sky chunks - to cost 15 % of the kernel.)
-        if (m_need != 0u && next >= total && have_claim && !(fuse && ((left8 >> (8 * ((seq_cur + 1) & (kPoolSlots - 1)))) & 0xffull) != 0ull)) {   // the current chunk is handed out: switch to the claimed one
-            tile0 = __shfl_sync(FULL, claimed, 0);
-            have_claim = false;
-            if (tile0 >= n_tiles) { drained = true; total = 0; }
-            else { const unsigned int rem = n_tiles - tile0; total = (int)(rem < (unsigned int)pool_tiles ? rem : (unsigned int)pool_tiles) * 32; }
-            next = 0;
-            if (fuse && total > 0) {
-                ++seq_cur;
-                left8 += (unsigned long long)total << (8 * (seq_cur & (kPoolSlots - 1)));
-                if (lane == 0) chunk_tile[seq_cur & (kPoolSlots - 1)] = tile0;
-            }
-        }
-        if (m_need != 0u && next < total) {
-            const int idx = next + __popc(m_need & ((1u << lane) - 1u));
-            next += __popc(m_need);
-            if (!busy && idx < total) {
-                const unsigned int tile = tile0 + (unsigned int)(idx >> 5);
-                const int px = (int)(tile % (unsigned int)tiles_x) * kPoolTW + (idx % kPoolTW), py = (int)(tile / (unsigned int)tiles_x) * kPoolTH + ((idx & 31) / kPoolTW);
-                if (fuse) { my_seq = seq_cur; if (!(px < fr.width && py < fr.height)) fin_b = my_seq; }   // nothing to trace for this slot of the chunk
-                if (px < fr.width && py < fr.height) {
-                    pixel = (uint32_t)px + (uint32_t)py * (uint32_t)fr.width;
-                    d0 = ray_dir(fr, px, py);
-                    acc = f3(0.f, 0.f, 0.f); o = fr.cam_pos; d = d0; s = 0; depth = 0;
-                    busy = true;
-                    if (REUSE) {
-                        h0 = cached_primary(prim, pixel, o, d);
-                        float3 c;
-                        if (primary_ends(sc, fr, h0, c)) {
-                            // the primary ray misses (or max_bounces == 0): every sample of the pixel has the value c
-                            for (; s < n_samples; ++s) { acc.x += c.x; acc.y += c.y; acc.z += c.z; }
-                            segs += (unsigned int)n_samples;
-                            float4 a = accum[pixel];
-                            a.x += acc.x; a.y += acc.y; a.z += acc.z;
-                            accum[pixel] = a;
-                            if (fuse) fin_b = my_seq;
-                            busy = false;                    // takes another pixel in the next pass
-                        } else { h = h0; ++segs; scat = true; }
-                    }
-                }
-            }
-        }
-        if (fuse) retire();
-        if (scat) scatter_segment(sc, fr, h, pixel, s_begin + (uint32_t)s, o, d, T, L, depth);
-        if (!__any_sync(FULL, busy) && drained) break;      // not drained: the next pass switches to the claimed chunk
-    }
-
-    unsigned int total_s = segs, total_tr = traced;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        total_s += __shfl_down_sync(FULL, total_s, off);
-        total_tr += __shfl_down_sync(FULL, total_tr, off);
-    }
-    if (lane == 0 && total_s) {
-        atomicAdd(seg_counter, (unsigned long long)total_s); atomicAdd(seg_counter + 1, (unsigned long long)total_s);
-        atomicAdd(seg_counter + 2, (unsigned long long)total_tr); atomicAdd(seg_counter + 3, (unsigned long long)total_tr);
-    }
+    const PixelFilter pf = {kFilterNone, 0.f};
+    RTB_RENDER_POOL_BODY(false)
 }
+// the same with a pixel filter: one jittered primary ray per sample (no primary-hit reuse)
+template <int MODE, bool FRAME>
+__global__ void __launch_bounds__(kThreads, RTB_REGEN_MIN_BLOCKS) k_render_pool_aa(SceneView sc, BvhView bv, FlatView fl, FrameView fr, float4* __restrict__ accum,
+                                                              uint32_t s_begin, int n_samples, int pool_tiles,
+                                                              unsigned int* __restrict__ tile_cursor, unsigned long long* __restrict__ seg_counter, FrameOut fo,
+                                                              PixelFilter pf) {
+    constexpr bool REUSE = false;
+    const PrimCache prim = {nullptr, nullptr};
+    RTB_RENDER_POOL_BODY(true)
+}
+#undef RTB_RENDER_POOL_BODY
 
 // ---- BVH render kernel with warp-level phase scheduling ---------------------------------------
 // Same lane-owns-a-pixel / regeneration scheme as k_render_regen, but the BVH traversal is an
@@ -927,6 +974,12 @@ static cudaError_t ensure_smem_optin() {
     if ((e = optin(k_render_regen<2, false, true>)) != cudaSuccess) return e;
     if ((e = optin(k_render_regen<3, false, true>)) != cudaSuccess) return e;
     if ((e = optin(k_render_regen<5, true, false, true>)) != cudaSuccess) return e;      // the 7-CTA form (STASH)
+    // the pixel filter's forms
+    RTB_OPTIN2(k_render_pool_aa)
+    if ((e = optin(k_render_regen_aa<0>)) != cudaSuccess) return e; if ((e = optin(k_render_regen_aa<1>)) != cudaSuccess) return e;
+    if ((e = optin(k_render_regen_aa<2>)) != cudaSuccess) return e; if ((e = optin(k_render_regen_aa<3>)) != cudaSuccess) return e;
+    if ((e = optin(k_render_regen_aa<4>)) != cudaSuccess) return e; if ((e = optin(k_render_regen_aa<5>)) != cudaSuccess) return e;
+    if ((e = optin(k_render_regen_aa<2, true>)) != cudaSuccess) return e; if ((e = optin(k_render_regen_aa<3, true>)) != cudaSuccess) return e;
 #undef RTB_OPTIN
 #undef RTB_OPTIN2
 #undef RTB_OPTIN3
@@ -963,6 +1016,11 @@ cudaError_t launch_primary_aov(const SceneView& sc, const AccelSel& ac, const Fr
 
 cudaError_t launch_ray_dirs(const FrameView& fr, float* out, cudaStream_t st) {
     k_ray_dirs<<<dim3((fr.width + 127) / 128, fr.height), 128, 0, st>>>(fr, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sample_dirs(const FrameView& fr, PixelFilter pf, uint32_t sample, float* out, cudaStream_t st) {
+    k_sample_dirs<<<dim3((fr.width + 127) / 128, fr.height), 128, 0, st>>>(fr, pf, sample, out);
     return cudaGetLastError();
 }
 
@@ -1038,8 +1096,9 @@ constexpr long long kStashMinWarpTiles = 40000;
 
 cudaError_t launch_render_regen(const SceneView& sc, const AccelSel& ac, const FrameView& fr, float4* accum,
                                 uint32_t s_begin, int n_samples, const PrimCache* prim_cache, unsigned long long* seg_counter, cudaStream_t st, int pool_override, bool flat_coop,
-                                bool count_traversal, FrameTarget* frame) {
+                                bool count_traversal, FrameTarget* frame, const PixelFilter* filter) {
     if (n_samples <= 0) return cudaSuccess;
+    if (filter) prim_cache = nullptr;                         // every sample traces its own jittered primary ray
     const bool reuse_primary = prim_cache != nullptr;
     PrimCache prim;
     prim.nt = prim_cache ? prim_cache->nt : nullptr; prim.id = prim_cache ? prim_cache->id : nullptr;
@@ -1080,7 +1139,9 @@ cudaError_t launch_render_regen(const SceneView& sc, const AccelSel& ac, const F
             frame->fused = true;
         }
 #define RTB_POOL_CASE(M) case M: \
-            if (fo.out) { if (reuse_primary) k_render_pool<M, true, true><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, prim, cursor, seg_counter, fo); \
+            if (filter) { if (fo.out) k_render_pool_aa<M, true><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, cursor, seg_counter, fo, *filter); \
+                          else k_render_pool_aa<M, false><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, cursor, seg_counter, fo, *filter); } \
+            else if (fo.out) { if (reuse_primary) k_render_pool<M, true, true><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, prim, cursor, seg_counter, fo); \
                           else k_render_pool<M, false, true><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, prim, cursor, seg_counter, fo); } \
             else { if (reuse_primary) k_render_pool<M, true, false><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, prim, cursor, seg_counter, fo); \
                    else k_render_pool<M, false, false><<<(unsigned int)blocks, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, pool_tiles, prim, cursor, seg_counter, fo); } \
@@ -1091,7 +1152,9 @@ cudaError_t launch_render_regen(const SceneView& sc, const AccelSel& ac, const F
     }
     if (count_traversal && (mode == 2 || mode == 3) && !ac.bvh.wnodes) {
         const dim3 grid = tile_grid(fr.width, fr.height);
-        if (mode == 2 && reuse_primary) k_render_regen<2, true, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
+        if (filter && mode == 2) k_render_regen_aa<2, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, seg_counter, *filter);
+        else if (filter) k_render_regen_aa<3, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, seg_counter, *filter);
+        else if (mode == 2 && reuse_primary) k_render_regen<2, true, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
         else if (mode == 2) k_render_regen<2, false, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
         else if (reuse_primary) k_render_regen<3, true, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
         else k_render_regen<3, false, true><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
@@ -1100,6 +1163,13 @@ cudaError_t launch_render_regen(const SceneView& sc, const AccelSel& ac, const F
     // large grids of the pooled flat traversal with the primary-hit cache (the headline configuration): the 7-CTA form (k_render_regen STASH)
     static const bool no_stash = [] { const char* v = getenv("RTB200_REGEN_STASH"); return v && v[0] == '0'; }();    // A/B
     static const long long stash_min = [] { const char* v = getenv("RTB200_STASH_MIN_TILES"); return v ? atoll(v) : kStashMinWarpTiles; }();   // A/B
+    if (filter) {
+        const dim3 grid = tile_grid(fr.width, fr.height);
+#define RTB_AA_CASE(M) case M: k_render_regen_aa<M><<<grid, kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, seg_counter, *filter); break;
+        switch (mode) { RTB_AA_CASE(0) RTB_AA_CASE(1) RTB_AA_CASE(2) RTB_AA_CASE(3) RTB_AA_CASE(4) default: RTB_AA_CASE(5) }
+#undef RTB_AA_CASE
+        return cudaGetLastError();
+    }
     if (mode == 5 && reuse_primary && !no_stash && n_tiles_all >= stash_min) {
         k_render_regen<5, true, false, true><<<tile_grid(fr.width, fr.height), kThreads, sb, st>>>(sc, ac.bvh, ac.flat, fr, accum, s_begin, n_samples, prim, seg_counter);
         return cudaGetLastError();

@@ -4,6 +4,7 @@
 #include <stdint.h>
 
 #include "rt_device.cuh"
+#include "rt_filter.cuh"
 #include "rt_temporal.cuh"
 
 namespace rtb {
@@ -35,6 +36,8 @@ struct PrimCache { const float4* nt; const int* id; };
 cudaError_t launch_primary_aov(const SceneView& sc, const AccelSel& ac, const FrameView& fr, int* id, float* t,
                                float* n, float* p, cudaStream_t st);
 cudaError_t launch_ray_dirs(const FrameView& fr, float* out, cudaStream_t st);
+// filtered_ray_dir() (rt_filter.cuh) of global sample `sample` for every pixel: width * height * 3 floats
+cudaError_t launch_sample_dirs(const FrameView& fr, PixelFilter pf, uint32_t sample, float* out, cudaStream_t st);
 cudaError_t launch_trace_rays(const SceneView& sc, const AccelSel& ac, const float* org, const float* dir, int n,
                               int* id, float* t, float* nrm, float* pt, cudaStream_t st,
                               unsigned long long* counters = nullptr);   // non-NULL + binary BVH: the counting instantiation (counters[8..12])
@@ -63,7 +66,8 @@ cudaError_t launch_render_regen(const SceneView& sc, const AccelSel& ac, const F
                                 int pool_override = 0,    // 0: automatic; 1: always one pixel per lane; n >= 2: pool of n tiles per warp
                                 bool flat_coop = true,    // flat accelerator: warp-cooperative levels 2/3 (rt_trace.cuh)
                                 bool count_traversal = false,    // binary-BVH back ends: count node visits / primitive tests into seg_counter[8..12]
-                                FrameTarget* frame = nullptr);
+                                FrameTarget* frame = nullptr,
+                                const PixelFilter* filter = nullptr);   // non-NULL: the jittered forms, one primary ray per sample (prim_cache ignored)
 cudaError_t launch_render_bvh(const SceneView& sc, const AccelSel& ac, const FrameView& fr, float4* accum, uint32_t s_begin,
                               int n_samples, unsigned long long* seg_counter, int wait_k, cudaStream_t st);
 cudaError_t launch_render_preview(const SceneView& sc, const AccelSel& ac, const FrameView& fr, float4* accum,

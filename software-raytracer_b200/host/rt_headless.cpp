@@ -10,6 +10,7 @@
 // filter (rt_denoise_rgba8; single GPU only).
 // --temporal CAP: frames are presented through the temporal resolve (rt_temporal_rgba8, history cap CAP, --denoise K as its filter;
 // single GPU only). --orbit DEG: the camera turns DEG degrees about its up axis before every --interactive frame (a fly-through).
+// --filter none|box|tent, --filter-radius R: anti-aliased path frames through the pixel filter (rt_set_pixel_filter; with --gpus too).
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -38,6 +39,8 @@ int main(int argc, char** argv) {
     bool preview = false;
     float scale = 1.0f;
     double orbit = 0.0;
+    rt_pixel_filter filter;
+    rt_default_pixel_filter(&filter);
     for (int i = 1; i < argc; ++i) {
         auto arg = [&](const char* n) { return !strcmp(argv[i], n) && i + 1 < argc; };
         if (arg("--scene")) scene_path = argv[++i];
@@ -52,6 +55,14 @@ int main(int argc, char** argv) {
         else if (arg("--denoise")) denoise = atoi(argv[++i]);
         else if (arg("--temporal")) temporal = atoi(argv[++i]);
         else if (arg("--orbit")) orbit = atof(argv[++i]);
+        else if (arg("--filter")) {
+            const char* v = argv[++i];
+            if (!strcmp(v, "none")) filter.type = RT_FILTER_NONE;
+            else if (!strcmp(v, "box")) filter.type = RT_FILTER_BOX;
+            else if (!strcmp(v, "tent")) filter.type = RT_FILTER_TENT;
+            else { fprintf(stderr, "rt_headless: --filter takes none, box or tent\n"); return 2; }
+        }
+        else if (arg("--filter-radius")) filter.radius = (float)atof(argv[++i]);
         else if (!strcmp(argv[i], "--preview")) preview = true;
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
     }
@@ -61,6 +72,7 @@ int main(int argc, char** argv) {
         fprintf(stderr, "rt_headless: --denoise is not supported with --gpus > 1 (a member's buffer holds only its shard of the samples)\n");
         return 2;
     }
+    if (!(filter.radius > 0.f && filter.radius <= 4.f)) { fprintf(stderr, "rt_headless: --filter-radius takes (0, 4] pixels\n"); return 2; }
     if (temporal < 0 || temporal > 4096) { fprintf(stderr, "rt_headless: --temporal takes a history cap of 0 .. 4096\n"); return 2; }
     if (gpus > 1 && temporal > 0) {
         fprintf(stderr, "rt_headless: --temporal is not supported with --gpus > 1 (a member's buffer holds only its shard of the samples)\n");
@@ -76,7 +88,8 @@ int main(int argc, char** argv) {
         rt_params par; rt_default_params(&par);
         par.width = w; par.height = h; par.max_bounces = bounces; par.mode = RT_MODE_PATH;
         rt_camera cam; rt_default_camera(&cam);
-        if (rt_group_set_params(g, &par) != RT_OK || rt_group_set_camera(g, &cam) != RT_OK || rt_group_reset_accumulation(g) != RT_OK) return die("setup");
+        if (rt_group_set_params(g, &par) != RT_OK || rt_group_set_camera(g, &cam) != RT_OK || rt_group_set_pixel_filter(g, &filter) != RT_OK ||
+            rt_group_reset_accumulation(g) != RT_OK) return die("setup");
         Pinned surface((size_t)w * h);
         using clk = std::chrono::steady_clock;
         if (rt_group_render_spp(g, spp) != RT_OK || rt_group_resolve_rgba8(g, surface.data(), w * 4, 1) != RT_OK) return die("warm-up frame");   // builds, tunes
@@ -107,6 +120,7 @@ int main(int argc, char** argv) {
         rt.SIMPLEDRAW = preview; rt.MAXBOUNCES = bounces; rt.TARGETFRAMES = 1 << 30; rt.SCREEN_SCALE = scale;
         rt.DENOISE_PASSES = denoise;
         rt.TEMPORAL_HISTORY = temporal;
+        rt.PIXEL_FILTER = filter.type; rt.PIXEL_FILTER_RADIUS = filter.radius;
         const float orbit_rad = (float)(orbit * M_PI / 180.0);
         Pinned surface((size_t)w * h);                          // interactive frames are streamed into it by the render kernel itself (rt_render_frame)
         using clk = std::chrono::steady_clock;

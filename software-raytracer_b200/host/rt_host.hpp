@@ -119,6 +119,7 @@ class Raytracer {
     rt_ctx* ctx = nullptr;
     rt_params par;
     bool doSetFrame = true;
+    int appliedFilter = RT_FILTER_NONE; float appliedRadius = 0.5f;
     static void check(int rc, rt_ctx* c) { if (rc < 0) throw std::runtime_error(rt_last_error(c)); }
 public:
     int FOV = 55, MAXBOUNCES = 2, TARGETFRAMES = 4096, ACCUMULATIONFRAMES = 1;     // Raytracer.cpp:31-34
@@ -127,6 +128,8 @@ public:
     int DENOISE_PASSES = 0;                         // > 0: frames are presented through the a-trous filter (rt_denoise_rgba8), 0: plain resolve
     int TEMPORAL_HISTORY = 0;                       // > 0: frames are presented through the temporal resolve (rt_temporal_rgba8) with this
                                                     // history cap (and DENOISE_PASSES as its filter), 0: off
+    int PIXEL_FILTER = RT_FILTER_NONE;              // RT_FILTER_*: anti-aliased path frames (rt_set_pixel_filter); a change restarts the accumulation
+    float PIXEL_FILTER_RADIUS = 0.5f;               // the filter's half-width in pixels, (0, 4]
     Transform camera;                                                               // :295-297
 
     Raytracer(int width = 1280, int height = 720, int device = 0) {                 // :26-27
@@ -222,6 +225,14 @@ private:
         check(rt_set_params(ctx, &par), ctx);
         rt_camera cam = camera.ToCamera(FOV);
         check(rt_set_camera(ctx, &cam), ctx);
+        if (PIXEL_FILTER != appliedFilter || PIXEL_FILTER_RADIUS != appliedRadius) {   // like a bounce change: the accumulation restarts
+            rt_pixel_filter f;
+            rt_default_pixel_filter(&f);
+            f.type = PIXEL_FILTER; f.radius = PIXEL_FILTER_RADIUS;
+            check(rt_set_pixel_filter(ctx, &f), ctx);
+            appliedFilter = PIXEL_FILTER; appliedRadius = PIXEL_FILTER_RADIUS;
+            doSetFrame = true;
+        }
         bool setFrame;
         // :576-581; the 1/4-scale first frame only shows something quickly, which the reprojected history does with TEMPORAL_HISTORY > 0
         if (doSetFrame) { setFrame = true; ACCUMULATIONFRAMES = 1; progressiveResolutionScaler = TEMPORAL_HISTORY > 0 ? 1.0f : 1.0f / 4.0f; doSetFrame = false; }

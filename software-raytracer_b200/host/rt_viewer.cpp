@@ -185,6 +185,9 @@ int main(int argc, char** argv) {
                 if (rt.SCREEN_SCALE != scaleBefore) rt.Invalidate();      // block size changes: mixing would blur (the reference keeps accumulating)
                 ImGui::SliderInt("Denoise passes", &rt.DENOISE_PASSES, 0, 8);  // presentation only: the accumulation goes on
                 ImGui::SliderInt("Temporal history", &rt.TEMPORAL_HISTORY, 0, 256);   // 0: off; > 0: the image survives camera moves
+                // 0 none, 1 box, 2 tent (RT_FILTER_*): anti-aliased path frames at render scale 1 (block-filled frames ignore it)
+                ImGui::SliderInt("Pixel filter", &rt.PIXEL_FILTER, RT_FILTER_NONE, RT_FILTER_TENT);
+                ImGui::SliderFloat("Filter radius", &rt.PIXEL_FILTER_RADIUS, 0.25f, 2.0f);
             }
             ImGui::Text("Application average %.3f \nms/frame (%.1f FPS)", 1000.0f / io.Framerate, io.Framerate);
             ImGui::End();

@@ -24,6 +24,7 @@ RT_OPT_BVH_QUANT = 15
 RT_MAX_PEERS = 16
 RT_PIPELINE_AUTO, RT_PIPELINE_REGEN, RT_PIPELINE_WAVEFRONT, RT_PIPELINE_STREAM = 0, 1, 2, 3
 RT_ACCEL_AUTO, RT_ACCEL_BRUTE, RT_ACCEL_BVH, RT_ACCEL_FLAT = 0, 1, 2, 3
+RT_FILTER_NONE, RT_FILTER_BOX, RT_FILTER_TENT = 0, 1, 2
 
 
 class RtObject(C.Structure):
@@ -60,6 +61,10 @@ class RtTemporalParams(C.Structure):
     _fields_ = [("max_history", C.c_int32), ("tau_depth", C.c_float), ("tau_normal", C.c_float), ("reserved", C.c_int32)]
 
 
+class RtPixelFilter(C.Structure):
+    _fields_ = [("type", C.c_int32), ("radius", C.c_float), ("reserved", C.c_int32 * 2)]
+
+
 class RtTraversalStats(C.Structure):
     _fields_ = [("queries", C.c_uint64), ("node_visits", C.c_uint64), ("prim_tests", C.c_uint64),
                 ("sphere_tests", C.c_uint64), ("cube_tests", C.c_uint64), ("tri_tests", C.c_uint64),
@@ -88,6 +93,7 @@ EXPORTS = [
     "rt_default_denoise_params", "rt_denoise_rgba8", "rt_read_denoised",
     "rt_default_temporal_params", "rt_temporal_rgba8", "rt_read_temporal", "rt_reset_temporal",
     "rt_group_denoise_rgba8", "rt_group_read_denoised", "rt_group_temporal_rgba8", "rt_group_read_temporal", "rt_group_reset_temporal",
+    "rt_default_pixel_filter", "rt_set_pixel_filter", "rt_get_pixel_filter", "rt_read_sample_dirs", "rt_group_set_pixel_filter",
 ]
 
 
@@ -119,7 +125,7 @@ def load_library(path=None):
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name in ("rt_host_alloc", "rt_host_free", "rt_last_error", "rt_accum_device_ptr", "rt_argb_device_ptr", "rt_create", "rt_default_params", "rt_default_camera",
-                    "rt_default_denoise_params", "rt_default_temporal_params", "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
+                    "rt_default_denoise_params", "rt_default_temporal_params", "rt_default_pixel_filter", "rt_rotate_camera", "rt_abi_version", "rt_object_name", "rt_scene_name", "rt_group_ctx", "rt_group_last_error"):
             continue
         fn.restype = C.c_int
     lib.rt_group_ctx.restype = C.c_void_p
@@ -145,6 +151,9 @@ def load_library(path=None):
     lib.rt_default_camera.restype = None
     lib.rt_default_denoise_params.restype = None
     lib.rt_default_temporal_params.restype = None
+    lib.rt_default_pixel_filter.restype = None
+    lib.rt_read_sample_dirs.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+    lib.rt_group_set_pixel_filter.argtypes = [C.c_void_p, C.c_void_p]
     lib.rt_rotate_camera.restype = None
     if path is None:
         _lib = lib
@@ -179,6 +188,22 @@ def default_temporal_params(**kw):
     for k, v in kw.items():
         setattr(p, k, v)
     return p
+
+
+def default_pixel_filter(**kw):
+    """rt_default_pixel_filter (RT_FILTER_NONE, radius 0.5), with any field overridden by keyword (type, radius)."""
+    f = RtPixelFilter()
+    load_library().rt_default_pixel_filter(C.byref(f))
+    for k, v in kw.items():
+        setattr(f, k, v)
+    return f
+
+
+def _filter_arg(f, radius):
+    """set_pixel_filter's argument: an RtPixelFilter, None (no filter) or an RT_FILTER_* type with `radius` (None: 0.5)."""
+    if f is None or isinstance(f, RtPixelFilter):
+        return f
+    return default_pixel_filter(type=int(f), **({} if radius is None else {"radius": radius}))
 
 
 def default_camera(fov=55):
@@ -341,6 +366,16 @@ class PathTracer:
     def set_shard(self, rank, world):
         return self._chk(self.lib.rt_set_shard(self.h, rank, world))
 
+    def set_pixel_filter(self, f=None, radius=None):
+        """rt_set_pixel_filter: f an RtPixelFilter, an RT_FILTER_* type (with `radius`, default 0.5) or None (no filter)."""
+        f = _filter_arg(f, radius)
+        return self._chk(self.lib.rt_set_pixel_filter(self.h, C.byref(f) if f is not None else None))
+
+    def pixel_filter(self):
+        f = RtPixelFilter()
+        self._chk(self.lib.rt_get_pixel_filter(self.h, C.byref(f)))
+        return f
+
     # hot path
     def reset_accumulation(self):
         return self._chk(self.lib.rt_reset_accumulation(self.h))
@@ -433,6 +468,13 @@ class PathTracer:
         w, h = self.params.width, self.params.height
         out = np.zeros((h, w, 3), np.float32)
         self._chk(self.lib.rt_read_ray_dirs(self.h, _p(out)))
+        return out
+
+    def read_sample_dirs(self, sample):
+        """rt_read_sample_dirs: the primary direction of global sample `sample` of every pixel, (height, width, 3) float32, y-up."""
+        w, h = self.params.width, self.params.height
+        out = np.zeros((h, w, 3), np.float32)
+        self._chk(self.lib.rt_read_sample_dirs(self.h, C.c_uint32(sample), _p(out)))
         return out
 
     def trace_rays(self, origin, direction):
@@ -589,6 +631,17 @@ class TracerGroup:
 
     def reset_accumulation(self):
         return self._chk(self.lib.rt_group_reset_accumulation(self.g))
+
+    def set_pixel_filter(self, f=None, radius=None):
+        """rt_group_set_pixel_filter: PathTracer.set_pixel_filter on every member."""
+        f = _filter_arg(f, radius)
+        return self._chk(self.lib.rt_group_set_pixel_filter(self.g, C.byref(f) if f is not None else None))
+
+    def pixel_filter(self):
+        return self.members[0].pixel_filter()
+
+    def read_sample_dirs(self, sample):
+        return self.members[0].read_sample_dirs(sample)
 
     def render_spp(self, spp):
         return self._chk(self.lib.rt_group_render_spp(self.g, spp))
