@@ -252,8 +252,8 @@ int rt_render_frame(rt_ctx* ctx, int spp, uint32_t* host_out, int pitch_bytes, i
 typedef struct {
     int32_t passes;         /* 0..8; 0 = the plain resolve, bit for bit */
     int32_t normal_power;   /* P: 1, 2, 4, .. 256 */
-    float sigma_color;      /* sigma_c: tolerance on Reinhard luminance at 1 spp */
-    float sigma_depth;      /* sigma_z: relative depth tolerance per pixel of step */
+    float sigma_color;      /* sigma_c: tolerance on Reinhard luminance at 1 spp; 2^-16 .. FLT_MAX */
+    float sigma_depth;      /* sigma_z: relative depth tolerance per pixel of step; 2^-16 .. FLT_MAX */
 } rt_denoise_params;        /* 16 bytes */
 void rt_default_denoise_params(rt_denoise_params* p);
 /* rt_resolve_rgba8 with the filter in front. NULL params = defaults. Synchronises. */

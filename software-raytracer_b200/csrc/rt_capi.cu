@@ -937,8 +937,9 @@ static int check_denoise_params(rt_ctx* c, const char* fn, const rt_denoise_para
     while (pow_log2 < 9 && (1 << pow_log2) != p.normal_power) ++pow_log2;
     if (p.passes < 0 || p.passes > kDenoiseMaxPasses) return fail(c, RT_ERR_INVALID, std::string(fn) + ": passes must be 0 .. 8");
     if (pow_log2 > 8) return fail(c, RT_ERR_INVALID, std::string(fn) + ": normal_power must be a power of two in 1 .. 256");
-    if (!(p.sigma_color > 0.f && p.sigma_color <= FLT_MAX) || !(p.sigma_depth > 0.f && p.sigma_depth <= FLT_MAX))
-        return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and positive");
+    // below kDenoiseSigmaMin the centre tap's weight, and with it every hit pixel, would be NaN (rt_denoise.cuh)
+    if (!(p.sigma_color >= kDenoiseSigmaMin && p.sigma_color <= FLT_MAX) || !(p.sigma_depth >= kDenoiseSigmaMin && p.sigma_depth <= FLT_MAX))
+        return fail(c, RT_ERR_INVALID, std::string(fn) + ": sigma_color and sigma_depth must be finite and at least 2^-16");
     return RT_OK;
 }
 

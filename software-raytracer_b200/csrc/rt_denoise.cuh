@@ -14,6 +14,12 @@ namespace rtb {
 
 constexpr int kDenoiseMaxPasses = 8;
 
+// Smallest sigma_color / sigma_depth the C-ABI accepts. With sigma_c >= 2^-16, sigma_c^2 >= 2^-32 is a normal float and
+// kc <= 4^7 (N + 4096) 2^32 < 2^79 stays finite for every pass, sample count and N_eff (tp_kc), so the centre tap's
+// dl^2 kc = 0 * kc is 0, never 0 * inf = NaN; with sigma_z >= 2^-16, dz >= 2^-16 1e-3 is a normal float, so |t_p - t_p| / dz is
+// 0, never 0 / 0. (A huge sigma_c gives sigma_c^2 = inf and kc = 0, which is harmless.)
+constexpr float kDenoiseSigmaMin = 0x1p-16f;
+
 // Reinhard-mapped luminance of a mean radiance (Rec. 709 weights)
 __host__ __device__ __forceinline__ float dn_luma(float r, float g, float b) {
     const float Y = 0.2126f * r + 0.7152f * g + 0.0722f * b;
